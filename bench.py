@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path's headline measurement (BASELINE.json: MDE/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- synthetic textured pairs
 1920x1080 with a known disparity field, window 9x9, 64 shifts (SURVEY 8d generator,
@@ -22,6 +22,9 @@ working set is far larger than L2.
 host core, each on its own slab of the same workload).
 Multi-GPU (torchrun): whole pairs are sharded over ranks, no collective on the data
 path (weak scaling: every rank runs `--pairs` pairs per step).
+
+--dump-outputs DIR writes rank 0's `best` and `web` of the last timed step as DIR/best.npy and
+DIR/web.npy (float32), so that two builds can be compared output for output on the same inputs.
 """
 import argparse
 import json
@@ -297,6 +300,22 @@ def _golden():
     return json.load(open(os.path.join(ROOT, "tests", "golden", "golden.json")))
 
 
+DUMP_ELEMENTS = 1 << 22  # per output: 16 MB of float32
+
+
+def dump_outputs(path, outputs):
+    """Write every device tensor of `outputs` as path/<name>.npy in float32 (the values are small integers, exact in
+    float32).  An output of more than DUMP_ELEMENTS elements is written as a fixed sample of them: sorted flat
+    indices drawn from seed 0, the same in every run with the same arguments."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in outputs.items():
+        if t.numel() > DUMP_ELEMENTS:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_ELEMENTS))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def time_batches(env, ctx, stream, run, steps):
     """steps calls of run() on the context's stream, device-timed, max over ranks -> ms per step."""
     torch = env.torch
@@ -505,6 +524,8 @@ def run_b200_arm(a, rank, world, local_rank):
               "golden": "tests/golden/golden.json synth/c2s/<seed>/wrap: CRC32 of web produced by the unmodified stereo.c"}
 
     # ---- the timed region: K steps, device-timed on the launching stream, max over ranks
+    if a.dump_outputs:  # so that what is dumped cannot be left over from the warm-up steps
+        best.fill_(-1), web.fill_(-1)
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     env.barrier()
@@ -518,6 +539,8 @@ def run_b200_arm(a, rank, world, local_rank):
     ms = env.rmax(ev0.elapsed_time(ev1))
     launches = a.steps * ctx.last_launches()  # per batch call: one pack + one main launch per group of pairs
     clocks = sampler.stop(tw0, tw1) if sampler else None
+    if a.dump_outputs and rank == 0:  # before the legs below write the same buffers again
+        dump_outputs(a.dump_outputs, {"best": best, "web": web})
     mde_step = B * W * H * D
     value = world * mde_step * a.steps / (ms * 1e-3) / 1e6
     us_pair_tp = ms * 1e3 / a.steps / B
@@ -710,7 +733,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-overlap", action="store_true", help="one sm_match_wta_dev call per pair (pack not overlapped)")
     ap.add_argument("--no-extra", action="store_true", help="skip the config4_pairs / config3_bands legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write best.npy and web.npy of the last timed step (float32; above %d elements a fixed "
+                         "seeded sample of them) into DIR" % DUMP_ELEMENTS)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm keeps no outputs)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -5,7 +5,8 @@ diffs every file of ser/ against par/ and of sergh/ against pargh/ (96 PPMs per 
 Here par/ and pargh/ come from debug/stereopar and debug/stereopar-ghost (host/driver.c over
 the C ABI); ser/ and sergh/ come from the reference's own serial programs when oracle/_ref
 holds them (built by `make -C oracle refserial`), and in any case from the CPU oracle's
-arrays written with a Python restatement of the reference's PPM writer.
+arrays written with a Python restatement of the reference's PPM writer, whose CRC32s are
+stored in tests/golden/ref_cases.json for fixtures 1-3.
 """
 import os
 import shutil
@@ -15,8 +16,8 @@ import numpy as np
 import pytest
 
 import oracle
-from test_host import _ppm_text
-from util import IMGS, ROOT, THRESHOLD, load_pair
+import ref_cases
+from util import IMGS, ROOT, THRESHOLD
 
 pytestmark = pytest.mark.gpu
 
@@ -49,29 +50,22 @@ def test_96_files_each(workdir):
 
 @pytest.mark.parametrize("variant,sub", [(0, "par"), (1, "pargh")])
 def test_ppms_equal_oracle_arrays(orc, workdir, variant, sub):
-    a, b = load_pair("1-240x135")
-    e1, e2 = orc.edges(a, THRESHOLD, variant), orc.edges(b, THRESHOLD, variant)
-    best, web = orc.match_wta(e1, e2, 30, 21, variant)
-    expect = {"edges-1.ppm": _ppm_text(e1, True), "edges-2.ppm": _ppm_text(e2, True),
-              "score_best-0.ppm": _ppm_text(best, False), "web-1.ppm": _ppm_text(web, False),
-              "web-2.ppm": _ppm_text(orc.fill_web_holes(web, 32), False)}
-    rc, out = orc.draw_contour_map(web, 10)
-    assert rc == 0
-    expect["output-0.ppm"] = _ppm_text(out, True)
-    for i in range(30):
-        m, sa, s = orc.shift_planes(e1, e2, 21, i, variant)
-        expect["matches-%d.ppm" % i] = _ppm_text(m, True)
-        expect["score_all-%d.ppm" % i] = _ppm_text(sa, False)
-        expect["scores-%d.ppm" % i] = _ppm_text(s, False)
+    expect = ref_cases.driver_ppms(orc, "1-240x135", variant)
     for name in NAMES:
         assert open(workdir / sub / name).read() == expect[name], name
 
 
+def _stored_reference_files(fixture):
+    return {sub: ref_cases.stored()["driver/%s/%s" % (fixture, v)] for sub, v in (("par", "wrap"), ("pargh", "ghost"))}
+
+
 def test_diff_sh_against_the_reference_serial_programs(workdir):
+    for sub, want in _stored_reference_files("1-240x135").items():
+        assert ref_cases.file_crcs(workdir / sub) == want, sub
     ser = os.path.join(ROOT, "oracle", "_ref", "debug", "stereomatch")
     sergh = os.path.join(ROOT, "oracle", "_ref", "debug", "stereomatch-ghost")
     if not (os.path.exists(ser) and os.path.exists(sergh)):
-        pytest.skip("oracle/_ref/debug not built (make -C oracle refserial needs /root/reference)")
+        return  # the live comparison needs the reference's serial programs built into oracle/_ref/debug
     for exe in (ser, sergh):
         r = subprocess.run([exe, "a.png", "b.png"], cwd=workdir, capture_output=True, text=True)
         assert r.returncode == 0, r.stderr
@@ -82,6 +76,21 @@ def test_diff_sh_against_the_reference_serial_programs(workdir):
                 problems.append("problem with image %s (%s - %s)" % (name, x, y))
     assert len(os.listdir(workdir / "ser")) == 96
     assert not problems, problems
+
+
+@pytest.mark.parametrize("fixture", ["2-480x270", "3-960x540"])
+def test_diff_sh_larger_fixtures_against_stored_reference_files(tmp_path, fixture):
+    """The test/diff.sh loop on fixtures 2 and 3 (fixture 1: the tests above): every file of par/ and pargh/,
+    written by debug/stereopar and debug/stereopar-ghost, against the stored CRC32s of ser/ and sergh/."""
+    for f in ("a.png", "b.png"):
+        shutil.copy(os.path.join(IMGS, fixture, f), tmp_path / f)
+    for sub, want in _stored_reference_files(fixture).items():
+        (tmp_path / sub).mkdir()
+        exe = os.path.join(ROOT, "debug", "stereopar" if sub == "par" else "stereopar-ghost")
+        r = subprocess.run([exe, "a.png", "b.png"], cwd=tmp_path, capture_output=True, text=True)
+        assert r.returncode == 0, (sub, r.stderr)
+        assert ref_cases.file_crcs(tmp_path / sub) == want, (fixture, sub)
+    shutil.rmtree(tmp_path, ignore_errors=True)
 
 
 @pytest.mark.parametrize("fixture", ["1-240x135", "2-480x270", "3-960x540"])

@@ -2,14 +2,16 @@
 
  * against tests/golden/golden.json -- CRC32s produced by the UNMODIFIED reference
    (tests/golden/make_golden.py; the fixture rows equal SURVEY.md 8c's table);
- * against the reference itself (oracle/_ref, built by oracle/Makefile) when it is
-   present -- it is in the build container and travels to the GPU box prebuilt;
+ * on the cases compared with the reference itself: against the CRCs stored for them in
+   tests/golden/ref_cases.json (tests/ref_cases.py) always, and array for array against
+   oracle/_ref (built by oracle/Makefile) when it is present;
  * the fast (separable) box sums against the literal sw*sw tap loop.
 """
 import numpy as np
 import pytest
 
 import oracle
+import ref_cases
 from util import FIXTURES, THRESHOLD, load_pair, vname
 
 SURVEY_WEB = {  # SURVEY.md 8(c), the `web` column
@@ -107,8 +109,9 @@ def test_fast_box_equals_direct(orc, sw, variant):
 @pytest.mark.parametrize("variant", [oracle.WRAP, oracle.GHOST])
 def test_oracle_equals_reference_build(orc, variant):
     """Array-for-array against the reference's own functions (edges, planes, best, web)."""
+    assert ref_cases.build_case(orc, variant) == ref_cases.stored()["build/" + vname(variant)]
     if not oracle.ref_available(variant, 30):
-        pytest.skip("oracle/_ref not built (make -C oracle ref needs /root/reference)")
+        return  # the live comparison needs the reference built into oracle/_ref
     a, b = load_pair("1-240x135")
     ref = oracle.RefLib(variant, 30)
     e1r, e2r = ref.edges(a, THRESHOLD), ref.edges(b, THRESHOLD)
@@ -130,10 +133,11 @@ def test_oracle_equals_reference_build(orc, variant):
 
 @pytest.mark.parametrize("variant", [oracle.WRAP, oracle.GHOST])
 def test_oracle_equals_reference_other_shift_counts(orc, variant):
-    for D in (16, 64, 128):
+    assert ref_cases.shift_counts_case(orc, variant) == ref_cases.stored()["shift_counts/" + vname(variant)]
+    for D in ref_cases.SHIFT_COUNTS:
         if not oracle.ref_available(variant, D):
-            pytest.skip("oracle/_ref not built")
-        left, right, _ = orc.synth_pair(5 + D, 200, 64, D)
+            continue  # the live comparison needs the reference built into oracle/_ref
+        left, right = ref_cases.shift_counts_pair(orc, D)
         e1, e2 = orc.edges(left, THRESHOLD, variant), orc.edges(right, THRESHOLD, variant)
         ref = oracle.RefLib(variant, D)
         assert np.array_equal(ref.edges(left, THRESHOLD), e1)
@@ -183,17 +187,15 @@ def test_fill_web_holes_equals_reference(orc):
     """Holes (zeros) at row ends: the reference's unwrapped IDX(x+-1, y) makes the last pixel of a row a neighbour
     of the first pixel of the next (stereo.c:237-243).  Holes stay away from the first and last rows, where the
     reference reads outside the array; an even number of passes, so that it returns (and does not free) our buffer."""
+    assert ref_cases.fill_holes_case(orc) == ref_cases.stored()["fill_web_holes"]
     if not oracle.ref_available(oracle.WRAP, 30):
-        pytest.skip("oracle/_ref not built")
+        return  # the live comparison needs the reference built into oracle/_ref
     import ctypes as C
-    rng = np.random.default_rng(5)
-    w, h = 37, 23
-    web = rng.integers(1, 31, size=(h, w), dtype=np.int32)
-    for (y, x) in [(5, w - 1), (7, 0), (9, w - 1), (10, 0), (12, 18), (12, 19), (13, 18)]:
-        web[y, x] = 0
+    web = ref_cases.holes_web()
+    h, w = web.shape
     L = oracle.RefLib(oracle.WRAP, 30).L
     L.fill_web_holes.restype = C.c_void_p
-    for times in (2, 6, 32):
+    for times in ref_cases.HOLE_PASSES:
         ref = np.ascontiguousarray(web.copy())
         p = L.fill_web_holes(ref.ctypes.data_as(C.c_void_p), w, h, times)
         assert p == ref.ctypes.data
@@ -204,13 +206,11 @@ def test_fill_web_holes_equals_reference(orc):
 def test_oracle_equals_reference_wide_windows(orc, variant):
     """Windows beyond the reference default (23..63): the GPU tests use the oracle as checker there too, so the
     oracle is pinned to the reference's own functions for them (small frames: the reference does sw*sw taps)."""
-    for (w, h, D, sw) in [(120, 60, 30, 23), (90, 90, 64, 27), (200, 64, 30, 31), (96, 70, 30, 33), (80, 64, 16, 63),
-                          (150, 45, 64, 45)]:
+    assert ref_cases.wide_windows_case(orc, variant) == ref_cases.stored()["wide_windows/" + vname(variant)]
+    for (w, h, D, sw) in ref_cases.WIDE_WINDOWS:
         if not oracle.ref_available(variant, D):
-            pytest.skip("oracle/_ref not built")
-        rng = np.random.default_rng(w + sw)
-        le = (rng.random((h, w)) < 0.4).astype(np.uint8)
-        re = np.roll(le, 5, axis=1) ^ (rng.random((h, w)) < 0.03).astype(np.uint8)
+            continue  # the live comparison needs the reference built into oracle/_ref
+        le, re = ref_cases.wide_windows_maps(w, h, sw)
         br, wr = oracle.RefLib(variant, D).match_wta(le, re, sw)
         bo, wo = orc.match_wta(le, re, D, sw, variant)
         assert np.array_equal(bo, br) and np.array_equal(wo, wr), (w, h, D, sw)
