@@ -88,10 +88,28 @@ typedef enum sm_info {
     SM_INFO_WARPS_PER_SM = 1,     /* resident warps per SM of the kernel instantiation this geometry uses */
     SM_INFO_PAIRS_PER_LAUNCH = 2, /* pairs the batch entries put into one launch (0 before the first batch call) */
     SM_INFO_TMEM_COLUMNS = 3,     /* tensor-memory columns one CTA allocates for the vertical-window ring */
-    SM_INFO_EDGE_THRESHOLDS = 4   /* 1: the edge detector's current decision table is exactly a threshold table
+    SM_INFO_EDGE_THRESHOLDS = 4,  /* 1: the edge detector's current decision table is exactly a threshold table
                                      (symmetric and monotone, checked bit by bit on the device) and the fast
                                      detector uses it; 0: it falls back to the bit table; -1: no table built yet */
+    SM_INFO_KERNEL_SHAPE = 5,     /* the kernel the most recent hot-path launch on this context ran, as an
+                                     sm_shape code (0 before any launch).  A batch call launches once per group of
+                                     pairs: the code is that of its last group */
+    SM_INFO_ROW_RUNS = 6          /* row runs per strip of that launch (its grid.y, after rounding the runs to whole
+                                     blocks of rows); 0 before any launch and for the direct kernel */
 } sm_info;
+
+/* SM_INFO_KERNEL_SHAPE codes.  A bit-sliced launch reports SM_SHAPE_BITSLICE | half | the flags of its
+ * instantiation, the direct kernel SM_SHAPE_DIRECT. */
+typedef enum sm_shape {
+    SM_SHAPE_HALF = 0xF,        /* mask: window half, square_width / 2 (0..15) */
+    SM_SHAPE_TWO_WORDS = 0x10,  /* two 32-bit words per lane (64 shifts per pass, or two pixels with C2) */
+    SM_SHAPE_SEG8 = 0x20,       /* 8-pixel walker segments (8-row blocks); 16-pixel segments otherwise */
+    SM_SHAPE_C2 = 0x40,         /* column pairs: the two words of a lane are two pixels, 32 shifts or fewer */
+    SM_SHAPE_HP = 0x80,         /* half-word pairs: each word serves two pixels, 16 shifts or fewer */
+    SM_SHAPE_MULTI = 0x100,     /* more than 64 shifts: successive 64-shift chunks merged in place */
+    SM_SHAPE_BITSLICE = 0x200,  /* set in every bit-sliced code */
+    SM_SHAPE_DIRECT = 0x400     /* the direct kernel (SM_KERNEL_DIRECT) */
+} sm_shape;
 
 /* ---- library-level -------------------------------------------------------- */
 

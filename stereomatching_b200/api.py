@@ -18,6 +18,10 @@ WRAP, GHOST = 0, 1
 KERNEL_AUTO, KERNEL_DIRECT, KERNEL_BITSLICE = 0, 1, 2
 OPT_EDGES_FP64, OPT_PIPE_GROUP, OPT_ROW_RUNS = 1, 2, 3
 INFO_WARPS_PER_SM, INFO_PAIRS_PER_LAUNCH, INFO_TMEM_COLUMNS, INFO_EDGE_THRESHOLDS = 1, 2, 3, 4
+INFO_KERNEL_SHAPE, INFO_ROW_RUNS = 5, 6
+# INFO_KERNEL_SHAPE codes (enum sm_shape): bit-sliced = SHAPE_BITSLICE | half | flags, direct = SHAPE_DIRECT
+(SHAPE_HALF, SHAPE_TWO_WORDS, SHAPE_SEG8, SHAPE_C2, SHAPE_HP, SHAPE_MULTI, SHAPE_BITSLICE,
+ SHAPE_DIRECT) = 0xF, 0x10, 0x20, 0x40, 0x80, 0x100, 0x200, 0x400
 (EDGES1, EDGES2, MATCH, SCORE_ALL, SCORE, BEST, WEB, WEB_FILLED, OUTPUT) = range(9)
 _PLANE_DTYPE = {EDGES1: np.uint8, EDGES2: np.uint8, MATCH: np.uint8, SCORE_ALL: np.int32,
                 SCORE: np.int32, BEST: np.int32, WEB: np.int32, WEB_FILLED: np.int32,

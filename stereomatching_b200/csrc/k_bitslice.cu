@@ -849,7 +849,7 @@ k_bitslice(BitsliceArgs a)
 }
 
 template <int HALF, int NW, int SEG, bool C2, bool HP>
-int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode)
+int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec)
 {
     using C = WS<HALF, NW, SEG>;
     if (mode == MODE_TMEM_COLUMNS) return C::TCOLS;
@@ -957,6 +957,11 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode)
         kern<<<grid, 32 * C::WPC, C::SMEM_REQ, s>>>(a);
     }
     SM_CUDA(cudaGetLastError());
+    if (rec) {
+        rec->shape = SM_SHAPE_BITSLICE | HALF | (NW == 2 ? SM_SHAPE_TWO_WORDS : 0) | (SEG == 8 ? SM_SHAPE_SEG8 : 0) |
+                     (C2 ? SM_SHAPE_C2 : 0) | (HP ? SM_SHAPE_HP : 0) | (multi ? SM_SHAPE_MULTI : 0);
+        rec->row_runs = (int)grid.y;
+    }
     return 1;
 }
 
@@ -1006,7 +1011,7 @@ static Shape pick_shape(const HotArgs &h, int num_sms)
     return sh;
 }
 
-static int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode)
+static int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec = nullptr)
 {
     if (mode == MODE_PREPARE && h.npairs == 1) {
         // a context launches one pair at a time AND batches: prepare the batch flavour too if it is another kernel
@@ -1022,7 +1027,7 @@ static int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode)
     const int half = h.g.half;
 #define SM_SHAPE(HF, NW_, SEG_, C2_, HP_) \
     if (half == HF && sh.nw == NW_ && sh.seg == SEG_ && sh.c2 == C2_ && sh.hp == HP_) \
-        return launch_one<HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode);
+        return launch_one<HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec);
 #define SM_HALVES(M, ...) \
     M(0, __VA_ARGS__) M(1, __VA_ARGS__) M(2, __VA_ARGS__) M(3, __VA_ARGS__) M(4, __VA_ARGS__) M(5, __VA_ARGS__) \
     M(6, __VA_ARGS__) M(7, __VA_ARGS__) M(8, __VA_ARGS__) M(9, __VA_ARGS__) M(10, __VA_ARGS__) M(11, __VA_ARGS__) \
@@ -1049,7 +1054,10 @@ static int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode)
 // walk of 16 + 2*15 steps fits the walker's 96-bit window; wider windows take the direct kernel.
 bool bitslice_supports(int half, int D) { return half >= 0 && half <= 15 && D >= 1 && D <= 512; }
 
-int launch_bitslice(const HotArgs &h, int num_sms, cudaStream_t s) { return dispatch(h, num_sms, s, MODE_LAUNCH); }
+int launch_bitslice(const HotArgs &h, int num_sms, cudaStream_t s, LaunchRecord *rec)
+{
+    return dispatch(h, num_sms, s, MODE_LAUNCH, rec);
+}
 
 // How many pairs of a batch to put into one launch.  Every warp pays 2*half warm-up rows per
 // run, so runs should be as long as the frame allows: pairs are added to the launch until one

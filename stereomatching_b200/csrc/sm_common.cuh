@@ -85,12 +85,19 @@ struct HotArgs {
     int blocks_per_sm = 0;
 };
 
+// What a hot-path launch ran (SM_INFO_KERNEL_SHAPE, SM_INFO_ROW_RUNS): filled in by the launcher from the
+// values it launched with.
+struct LaunchRecord {
+    int shape = 0;     // sm_shape code
+    int row_runs = 0;  // grid.y
+};
+
 // launchers (each returns the number of kernels launched, or a negative sm_status)
 int launch_pack(const uint8_t *e1, const uint8_t *e2, int FH, int row0, int variant,
                 const PackedGeom &g, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
                 int npairs = 1, size_t edge_stride = 0, size_t plane_stride = 0);
 int launch_direct(const HotArgs &a, cudaStream_t s);
-int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s);
+int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);
 bool bitslice_supports(int half, int D);
 int prepare_bitslice(const HotArgs &a, int num_sms);
 int bitslice_tmem_columns(const HotArgs &a);

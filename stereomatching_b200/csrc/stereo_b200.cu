@@ -52,6 +52,7 @@ struct sm_ctx {
     int last_launches = 0;
     int tuned_segs = 0;  // SM_OPT_ROW_RUNS: row runs per strip of a one-pair launch (0: the kernel's cost model)
     int occ = 0;         // resident warps per SM of the bit-sliced kernel of this geometry (prepare_bitslice)
+    LaunchRecord last_launch;  // the most recent hot-path launch (SM_INFO_KERNEL_SHAPE, SM_INFO_ROW_RUNS)
 
     // frame-sized device arrays (a band context touches only the rows it needs)
     uint8_t *img_u8[2] = {nullptr, nullptr};
@@ -230,9 +231,17 @@ int launch_main(sm_ctx *c, const HotArgs &a, cudaStream_t st)
             set_error("bit-sliced kernel does not cover square_width %d / num_shifts %d", c->sw, c->D);
             return SM_ERR_ARG;
         }
-        return launch_bitslice(a, c->num_sms, st);
+        LaunchRecord rec;
+        const int rc = launch_bitslice(a, c->num_sms, st, &rec);
+        if (rc >= 0) c->last_launch = rec;
+        return rc;
     }
-    return launch_direct(a, st);
+    const int rc = launch_direct(a, st);
+    if (rc >= 0) {
+        c->last_launch.shape = SM_SHAPE_DIRECT;
+        c->last_launch.row_runs = 0;
+    }
+    return rc;
 }
 
 int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, int32_t *best, int32_t *web)
@@ -287,8 +296,9 @@ void profile_free(sm_ctx *c)
 
 extern "C" const char *sm_last_error(void) { return g_err; }
 
-// 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out
-extern "C" int sm_version(void) { return (1 << 16) | 2; }
+// 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out;
+// 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS
+extern "C" int sm_version(void) { return (1 << 16) | 3; }
 
 extern "C" int sm_device_count(void)
 {
@@ -521,6 +531,8 @@ extern "C" int sm_get_info(sm_ctx *c, int what)
     case SM_INFO_WARPS_PER_SM: return c->occ;
     case SM_INFO_PAIRS_PER_LAUNCH: return c->batch_group_cap;
     case SM_INFO_TMEM_COLUMNS: return bitslice_supports(c->half, c->D) ? bitslice_tmem_columns(hot_args(c, c->best, c->web)) : 0;
+    case SM_INFO_KERNEL_SHAPE: return c->last_launch.shape;
+    case SM_INFO_ROW_RUNS: return c->last_launch.row_runs;
     case SM_INFO_EDGE_THRESHOLDS: {
         if (!c->edge_lut || c->lut_threshold < 0.0) return -1;
         uint32_t flag = 0;

@@ -52,6 +52,20 @@ def test_version_and_error_string():
     assert isinstance(L.sm_last_error(), bytes)
 
 
+def test_info_items_and_shape_codes_match_the_header():
+    """ABI 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS and the sm_shape code bits, as the binding spells them."""
+    assert smb.lib().sm_version() == (1 << 16) | 3
+    text = open(os.path.join(ROOT, "include", "stereo_b200.h")).read()
+    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+    values = {k: int(v, 0) for k, v in re.findall(r"\b(SM_(?:INFO|SHAPE)_[A-Z0-9_]+)\s*=\s*(0x[0-9A-Fa-f]+|\d+)", text)}
+    for name, value in values.items():
+        assert getattr(smb.api, name[3:]) == value, name
+    assert "SM_INFO_KERNEL_SHAPE" in values and "SM_INFO_ROW_RUNS" in values and "SM_SHAPE_DIRECT" in values
+    # the flag bits do not overlap each other or the window half
+    bits = [v for k, v in values.items() if k.startswith("SM_SHAPE_")]
+    assert sum(bits) == 0x7FF and len(bits) == 8
+
+
 def test_band_rows_partition():
     for h in (1, 7, 135, 1080, 2160):
         for n in (1, 2, 3, 4, 8):
