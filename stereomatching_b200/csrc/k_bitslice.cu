@@ -50,9 +50,11 @@
 // A run's first 2*half rows only fill the vertical window: a short block and then whole blocks that add
 // into the sums and the ring and nothing else, in front of the whole, branch-free steady blocks.
 //
-// The ALU pipe binds this kernel (LOP3), so what is not bit-plane logic is kept off it: the selects of the
-// winner-take-all are predicated multiply-adds, store addresses are one widening multiply-add on a per-lane
-// base (FMA pipe), ring slots advance by compare-and-subtract (uniform datapath).
+// The ALU pipe binds this kernel (LOP3), so what is not bit-plane logic is kept off it: the walker's complement and
+// the selects of the winner-take-all are predicated multiply-adds, the winning lane's index is a multiply-add on
+// shift amounts, store addresses are one widening multiply-add on a per-lane base (FMA pipe), ring slots advance by
+// compare-and-subtract (uniform datapath).  The bit-plane logic itself is written one LOP3 per term
+// (tools/sass_budget.py counts what ptxas made of it).
 //
 // Launching.  Several pairs per launch (grid z) run in the throughput shape: runs of about 32
 // windows, several waves deep.  One pair per launch takes the number of row runs a small cost
@@ -209,6 +211,15 @@ __device__ __forceinline__ void tm_pin(uint32_t (&v)[EC])
 __device__ __forceinline__ void tm_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tm_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+// x, y, z -> the 3-input function whose truth table is LUT (x = 0xF0, y = 0xCC, z = 0xAA): one LOP3
+template <int LUT>
+__device__ __forceinline__ uint32_t lop3(uint32_t x, uint32_t y, uint32_t z)
+{
+    uint32_t r;
+    asm("lop3.b32 %0, %1, %2, %3, %4;" : "=r"(r) : "r"(x), "r"(y), "r"(z), "n"(LUT));
+    return r;
+}
+
 // V (PV planes) += H (KH planes), ripple carry; the sum always fits PV planes.
 template <int PV, int KH>
 __device__ __forceinline__ void planes_add(uint32_t (&V)[PV], const uint32_t (&H)[5])
@@ -250,27 +261,48 @@ __device__ __forceinline__ void planes_sub(uint32_t (&V)[PV], const uint32_t (&H
 }
 
 // V += Hn - Ho in one ripple: d = Hn - Ho as KH planes plus a sign plane, then V += sext(d).
-// 2*KH + 2*PV - 1 ops instead of 2 * (2*PV - 1).
-template <int PV, int KH>
+// 2*KH + 2*PV - 1 LOP3 instead of 2 * (2*PV - 1).  AS_WRITTEN: one LOP3 per term (left to the compiler, the terms
+// are re-associated into about 23 instead of 21 per plane pair at window 9).  The kernels with several 64-shift
+// chunks (MULTI) keep the compiler's form: at their 128 registers the explicit one makes them spill.
+template <int PV, int KH, bool AS_WRITTEN>
 __device__ __forceinline__ void planes_addsub(uint32_t (&V)[PV], const uint32_t (&Hn)[5], const uint32_t (&Ho)[5])
 {
-    uint32_t d[KH];
-    uint32_t b = ~Hn[0] & Ho[0];
-    d[0] = Hn[0] ^ Ho[0];
+    if constexpr (AS_WRITTEN) {
+        // plane k of d is added as soon as it is known (fewer live registers than all of d first)
+        const uint32_t d0 = lop3<0x3C>(Hn[0], Ho[0], Ho[0]);  // Hn ^ Ho
+        uint32_t b = lop3<0x0C>(Hn[0], Ho[0], Ho[0]);         // borrow: ~Hn & Ho
+        uint32_t c = lop3<0xC0>(V[0], d0, d0);                // carry: V & d
+        V[0] = lop3<0x3C>(V[0], d0, d0);
 #pragma unroll
-    for (int k = 1; k < KH; k++) {
-        d[k] = Hn[k] ^ Ho[k] ^ b;
-        b = (~Hn[k] & (Ho[k] | b)) | (Ho[k] & b);
-    }
-    const uint32_t sgn = b;  // lanes where Hn < Ho: d is negative, its upper planes are all ones
-    uint32_t c = V[0] & d[0];
-    V[0] ^= d[0];
+        for (int k = 1; k < PV; k++) {
+            uint32_t x = b;  // k >= KH: lanes where Hn < Ho, d is negative and its upper planes are all ones
+            if (k < KH) {
+                x = lop3<0x96>(Hn[k], Ho[k], b);
+                b = lop3<0x8E>(Hn[k], Ho[k], b);  // borrow: majority of ~Hn, Ho, b
+            }
+            const uint32_t sum = lop3<0x96>(V[k], x, c);
+            if (k + 1 < PV) c = lop3<0xE8>(V[k], x, c);  // carry: majority
+            V[k] = sum;
+        }
+    } else {
+        uint32_t d[KH];
+        uint32_t b = ~Hn[0] & Ho[0];
+        d[0] = Hn[0] ^ Ho[0];
 #pragma unroll
-    for (int k = 1; k < PV; k++) {
-        const uint32_t x = k < KH ? d[k] : sgn;
-        uint32_t sum = V[k] ^ x ^ c;
-        c = (V[k] & x) | (c & (V[k] ^ x));
-        V[k] = sum;
+        for (int k = 1; k < KH; k++) {
+            d[k] = Hn[k] ^ Ho[k] ^ b;
+            b = (~Hn[k] & (Ho[k] | b)) | (Ho[k] & b);
+        }
+        const uint32_t sgn = b;  // lanes where Hn < Ho: d is negative, its upper planes are all ones
+        uint32_t c = V[0] & d[0];
+        V[0] ^= d[0];
+#pragma unroll
+        for (int k = 1; k < PV; k++) {
+            const uint32_t x = k < KH ? d[k] : sgn;
+            uint32_t sum = V[k] ^ x ^ c;
+            c = (V[k] & x) | (c & (V[k] ^ x));
+            V[k] = sum;
+        }
     }
 }
 
@@ -291,14 +323,6 @@ __device__ __forceinline__ void load_walk_raw(WalkRaw &o, const HotArgs &h, int 
     for (int k = 0; k < 4; k++) o.r[k] = __ldg(pq + k);
 #pragma unroll
     for (int k = 0; k < 3; k++) o.a[k] = __ldg(pa + k), o.b[k] = __ldg(pb + k);
-}
-
-template <int LUT>
-__device__ __forceinline__ uint32_t lop3(uint32_t x, uint32_t y, uint32_t z)
-{
-    uint32_t r;
-    asm("lop3.b32 %0, %1, %2, %3, %4;" : "=r"(r) : "r"(x), "r"(y), "r"(z), "n"(LUT));
-    return r;
 }
 
 // Sum of N one-bit words as bit planes, by carry-save adders: plane K is the parity of the N
@@ -329,7 +353,7 @@ __device__ __forceinline__ void csa_planes(const uint32_t (&a)[N], uint32_t (&P)
 // instead of 2*HALF counter steps; from then on one word enters and one leaves per step.
 template <int HALF, int NW, int SEG, bool VALID_ALL, bool HP>
 __device__ __forceinline__ void walk(const uint32_t (&q)[3], const uint32_t (&lw)[2], const uint32_t (&vw)[2],
-                                     uint4 *hq, uint32_t *h5, uint32_t *mq)
+                                     uint32_t ones, uint4 *hq, uint32_t *h5, uint32_t *mq)
 {
     using C = WS<HALF, NW, SEG>;
     constexpr int N = C::N, KH = C::KH, STEPS = C::STEPS;
@@ -349,7 +373,10 @@ __device__ __forceinline__ void walk(const uint32_t (&q)[3], const uint32_t (&lw
             mm ^= halves(nl, t);                      // per half: L(u) ? R : ~R
             if (!VALID_ALL) mm &= halves(vw, t);      // per half: taps outside the image count nothing
         } else {
-            if (!(lw[t >> 5] & (1u << (t & 31)))) mm = ~mm;               // L(u) ? R : ~R
+            // L(u) ? R : ~R, the complement as a predicated multiply-add (~x == x * 0xFFFFFFFF + 0xFFFFFFFF) on the
+            // FMA pipe.  `ones` is 0xFFFFFFFF that ptxas cannot see, or it turns the multiply-add into an IADD3.
+            asm("{ .reg .pred p; setp.eq.u32 p, %1, 0; @p mad.lo.u32 %0, %0, %2, %2; }"
+                : "+r"(mm) : "r"(lw[t >> 5] & (1u << (t & 31))), "r"(ones));
             if (!VALID_ALL && !(vw[t >> 5] & (1u << (t & 31)))) mm = 0u;  // taps outside the image count nothing
         }
         if (t >= HALF && t < HALF + SEG) mq[(t - HALF) * NW] = mm;    // centre word of pixel ws*SEG + t - HALF
@@ -365,12 +392,13 @@ __device__ __forceinline__ void walk(const uint32_t (&q)[3], const uint32_t (&lw
     for (int t = 2 * HALF; t < STEPS; t++) {
         const uint32_t mm = m[t] = match_word(t);
         const uint32_t mout = t >= N ? m[t - N] : 0u;
-        // up/down counter: +1 where mm & ~mout, -1 where mout & ~mm
-        uint32_t c = (mm ^ mout) & (P[0] ^ mout);
-        P[0] ^= mm ^ mout;
+        // up/down counter: +1 where mm & ~mout, -1 where mout & ~mm; one LOP3 per term, as written (left to the
+        // compiler, the terms are re-associated into more instructions)
+        uint32_t c = lop3<0x24>(mm, mout, P[0]);  // (mm ^ mout) & (P[0] ^ mout)
+        P[0] = lop3<0x96>(P[0], mm, mout);
 #pragma unroll
         for (int k = 1; k < KH; k++) {
-            uint32_t cn = c & (P[k] ^ mout);
+            const uint32_t cn = lop3<0x60>(c, P[k], mout);  // c & (P[k] ^ mout)
             P[k] ^= c;
             c = cn;
         }
@@ -383,17 +411,23 @@ __device__ __forceinline__ void walk(const uint32_t (&q)[3], const uint32_t (&lw
 // their bit-serial chains (AND -> test -> select, PV times) gives the scheduler NR_ chains
 // to overlap.  The selects are predicated multiply-adds on purpose: ptxas puts them on the
 // FMA pipe, which is otherwise idle, instead of the ALU pipe that carries all the LOP3 work.
-template <int NR_, int NW, int PV>
+//
+// AS_WRITTEN (all but the MULTI kernels, which would spill at their 128 registers): the first plane's select and
+// the winning lane's index are kept off the ALU pipe too (below); otherwise ptxas makes the former three SELs per
+// row and the latter two FLO, a LOP3, a max and an add.
+template <int NR_, int NW, int PV, bool AS_WRITTEN>
 __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint32_t (&M)[NR_][NW],
-                                    const uint32_t (&valid)[NW], int one, int (&best)[NR_], int (&idx)[NR_])
+                                    const uint32_t (&valid)[NW], int one, int base, int (&best)[NR_], int (&web)[NR_])
 {
     uint32_t cand[NR_][NW];
 #pragma unroll
     for (int k = 0; k < NR_; k++) {
         best[k] = 0;
+        if (!AS_WRITTEN) {
 #pragma unroll
-        for (int w = 0; w < NW; w++)  // register copy via the FMA pipe: the first plane then is a predicated move like the others
-            asm("mad.lo.u32 %0, %1, %2, 0;" : "=r"(cand[k][w]) : "r"(valid[w]), "r"(one));
+            for (int w = 0; w < NW; w++)
+                asm("mad.lo.u32 %0, %1, %2, 0;" : "=r"(cand[k][w]) : "r"(valid[w]), "r"(one));
+        }
     }
 #pragma unroll
     for (int p = PV - 1; p >= 0; p--) {
@@ -402,7 +436,27 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
             // t = cand & V_p & M with the "any lane left" test folded into the same LOP3s: the
             // predicate output of one feeds the next (lop3.or d|p), so a plane costs NW ALU
             // instructions instead of NW + 1 (a separate OR-and-test)
-            if (NW == 2) {
+            if (AS_WRITTEN && p == PV - 1) {
+                // first plane, cand = valid: cand = q ? t : valid.  Without a lane left t is 0, so that is t, plus
+                // valid where !q: a predicated multiply-add on t's own register.  (A copy of valid overwritten where
+                // q is what ptxas turns into a SEL on the ALU pipe.)
+                if (NW == 2) {
+                    asm("{ .reg .pred q0, q;\n\t"
+                        "lop3.or.b32 %0|q0, %3, %4, %5, 0x80, 0;\n\t"
+                        "lop3.or.b32 %1|q, %6, %7, %8, 0x80, q0;\n\t"
+                        "@!q mad.lo.u32 %0, %3, %9, %0;\n\t@!q mad.lo.u32 %1, %6, %9, %1;\n\t"
+                        "@q mad.lo.s32 %2, %9, %10, %2; }"
+                        : "=r"(cand[k][0]), "=r"(cand[k][NW - 1]), "+r"(best[k])
+                        : "r"(valid[0]), "r"(V[k][0][p]), "r"(M[k][0]), "r"(valid[NW - 1]), "r"(V[k][NW - 1][p]),
+                          "r"(M[k][NW - 1]), "r"(one), "r"(1 << p));
+                } else {
+                    asm("{ .reg .pred q;\n\t"
+                        "lop3.or.b32 %0|q, %2, %3, %4, 0x80, 0;\n\t"
+                        "@!q mad.lo.u32 %0, %2, %5, %0;\n\t@q mad.lo.s32 %1, %5, %6, %1; }"
+                        : "=r"(cand[k][0]), "+r"(best[k])
+                        : "r"(valid[0]), "r"(V[k][0][p]), "r"(M[k][0]), "r"(one), "r"(1 << p));
+                }
+            } else if (NW == 2) {
                 asm("{ .reg .pred q0, q; .reg .b32 t0, t1;\n\t"
                     "lop3.or.b32 t0|q0, %0, %3, %4, 0x80, 0;\n\t"
                     "lop3.or.b32 t1|q, %1, %5, %6, 0x80, q0;\n\t"
@@ -420,11 +474,25 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
     }
 #pragma unroll
     for (int k = 0; k < NR_; k++) {
-        // highest surviving lane; a later word holds higher shifts.  The bit index of an empty
-        // word is -1, and -1 ^ 32 stays negative, so one signed max picks the right word
-        // (word 0 is never empty: it starts as valid[0] != 0 and is only replaced by non-zero t)
-        idx[k] = 31 - __clz(cand[k][0]);
-        if (NW == 2) idx[k] = max(idx[k], (31 - __clz(cand[k][NW - 1])) ^ 32);
+        // web = base + the highest surviving lane; a later word holds higher shifts.  m = 32 * NW - 1 - lane, from
+        // the shift amounts (31 - highest bit) of the words: with two words, that of word 1 if it has a lane, else
+        // 32 + that of word 0, which is one unsigned min, since an empty word's shift amount is 0xFFFFFFFF (and if
+        // word 0 is empty, word 1 is not: 0xFFFFFFFF + 32 wraps to 31, not below word 1's).  base + 32 * NW - 1 - m
+        // is a multiply-add by -one: the FMA pipe.
+        if (!AS_WRITTEN) {
+            // the bit index of an empty word is -1, and -1 ^ 32 stays negative, so one signed max picks the word
+            int idx = 31 - __clz(cand[k][0]);
+            if (NW == 2) idx = max(idx, (31 - __clz(cand[k][NW - 1])) ^ 32);
+            web[k] = base + idx;
+            continue;
+        }
+        uint32_t m, m1;
+        asm("bfind.shiftamt.u32 %0, %1;" : "=r"(m) : "r"(cand[k][0]));
+        if (NW == 2) {
+            asm("bfind.shiftamt.u32 %0, %1;" : "=r"(m1) : "r"(cand[k][NW - 1]));
+            m = min(m1, m + 32u);
+        }
+        asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(web[k]) : "r"(m), "r"(-one), "r"(base + 32 * NW - 1));
     }
 }
 
@@ -577,10 +645,9 @@ k_bitslice(BitsliceArgs a)
         const int row_bytes = 4 * g.W;
         int32_t *const lane_best = a.h.best + ximg, *const lane_web = a.h.web + ximg;
 
-        // store a finished row (best, idx) and advance the output pointers.  MULTI: a later chunk holds higher
+        // store a finished row (best, web) and advance the output pointers.  MULTI: a later chunk holds higher
         // shifts, so it wins ties against what the earlier chunks left in `best` (prev)
-        auto put = [&](int best, int idx, int prev) {
-            const int web = 32 * wg0 + idx + 1;
+        auto put = [&](int best, int web, int prev) {
             bool st = store_ok;
             if (MULTI && chunk != 0) st = st && best >= prev;
             store_if<0>(lane_best, orow, row_bytes, best, st);
@@ -594,24 +661,24 @@ k_bitslice(BitsliceArgs a)
             return v;
         };
         // C2: the two pixels of a lane (columns ximg and ximg + 32) of one finished row
-        auto put2 = [&](int best0, int idx0, int best1, int idx1) {
+        auto put2 = [&](int best0, int web0, int best1, int web1) {
             store_if<0>(lane_best, orow, row_bytes, best0, store_ok);
-            store_if<0>(lane_web, orow, row_bytes, idx0 + 1, store_ok);
+            store_if<0>(lane_web, orow, row_bytes, web0, store_ok);
             store_if<TW>(lane_best, orow, row_bytes, best1, store_ok2);
-            store_if<TW>(lane_web, orow, row_bytes, idx1 + 1, store_ok2);
+            store_if<TW>(lane_web, orow, row_bytes, web1, store_ok2);
             orow++;
         };
         // HP: the 2 * NW pixels of a lane of one finished row: word w covers columns ximg + w * WCOLS and that + 16
-        auto put_hp = [&](const int *bl, const int *il, const int *bh, const int *ih) {
+        auto put_hp = [&](const int *bl, const int *wl, const int *bh, const int *wh) {
             store_if<0>(lane_best, orow, row_bytes, bl[0], ximg < g.W);
-            store_if<0>(lane_web, orow, row_bytes, il[0] + 1, ximg < g.W);
+            store_if<0>(lane_web, orow, row_bytes, wl[0], ximg < g.W);
             store_if<16>(lane_best, orow, row_bytes, bh[0], ximg + 16 < g.W);
-            store_if<16>(lane_web, orow, row_bytes, ih[0] - 16 + 1, ximg + 16 < g.W);
+            store_if<16>(lane_web, orow, row_bytes, wh[0], ximg + 16 < g.W);
             if constexpr (NW == 2) {
                 store_if<WCOLS>(lane_best, orow, row_bytes, bl[NW - 1], ximg + WCOLS < g.W);
-                store_if<WCOLS>(lane_web, orow, row_bytes, il[NW - 1] + 1, ximg + WCOLS < g.W);
+                store_if<WCOLS>(lane_web, orow, row_bytes, wl[NW - 1], ximg + WCOLS < g.W);
                 store_if<WCOLS + 16>(lane_best, orow, row_bytes, bh[NW - 1], ximg + WCOLS + 16 < g.W);
-                store_if<WCOLS + 16>(lane_web, orow, row_bytes, ih[NW - 1] - 16 + 1, ximg + WCOLS + 16 < g.W);
+                store_if<WCOLS + 16>(lane_web, orow, row_bytes, wh[NW - 1], ximg + WCOLS + 16 < g.W);
             }
             orow++;
         };
@@ -632,16 +699,17 @@ k_bitslice(BitsliceArgs a)
                         for (int p = 0; p < PV; p++) V1[k * NW + w][0][p] = Vs[k][w][p];
                     }
                 const uint32_t vl1[1] = {valid_lo}, vh1[1] = {valid_hi};
-                int bl[NCH], il[NCH], bh[NCH], ih[NCH];
-                wta<NCH, 1, PV>(V1, M1, vl1, one, bl, il);
-                wta<NCH, 1, PV>(V1, M1, vh1, one, bh, ih);
+                // the upper half's lanes are 16..31 of the word: web = lane - 16 + 1
+                int bl[NCH], wl[NCH], bh[NCH], wh[NCH];
+                wta<NCH, 1, PV, !MULTI>(V1, M1, vl1, one, 1, bl, wl);
+                wta<NCH, 1, PV, !MULTI>(V1, M1, vh1, one, 1 - 16, bh, wh);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put_hp(bl + k * NW, il + k * NW, bh + k * NW, ih + k * NW);
+                for (int k = 0; k < G_; k++) put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW);
             } else if constexpr (!C2) {
-                int best[G_], idx[G_];
-                wta<G_, NW, PV>(Vs, Ms, valid, one, best, idx);
+                int best[G_], web[G_];
+                wta<G_, NW, PV, !MULTI>(Vs, Ms, valid, one, 32 * wg0 + 1, best, web);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put(best[k], idx[k], prev[k]);
+                for (int k = 0; k < G_; k++) put(best[k], web[k], prev[k]);
             } else {
                 uint32_t V1[2 * G_][1][PV], M1[2 * G_][1];
 #pragma unroll
@@ -653,10 +721,10 @@ k_bitslice(BitsliceArgs a)
                         for (int p = 0; p < PV; p++) V1[2 * k + w][0][p] = Vs[k][w][p];
                     }
                 const uint32_t valid1[1] = {valid[0]};
-                int best[2 * G_], idx[2 * G_];
-                wta<2 * G_, 1, PV>(V1, M1, valid1, one, best, idx);
+                int best[2 * G_], web[2 * G_];
+                wta<2 * G_, 1, PV, !MULTI>(V1, M1, valid1, one, 1, best, web);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put2(best[2 * k], idx[2 * k], best[2 * k + 1], idx[2 * k + 1]);
+                for (int k = 0; k < G_; k++) put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1]);
             }
         };
         auto load_m = [&](int mslot_c, uint32_t (&M)[NW]) {
@@ -688,9 +756,9 @@ k_bitslice(BitsliceArgs a)
                 const unsigned long long vl = (((unsigned long long)vw[1]) << 32) | vw[0];
                 const bool all_valid = (~vl & ((1ull << (STEPS + (HP ? 16 : 0))) - 1ull)) == 0ull;
                 if (__all_sync(0xFFFFFFFFu, all_valid || !active)) {
-                    if (active) walk<HALF, NW, SEG, true, HP>(q, lw, vw, hq, h5, mq);
+                    if (active) walk<HALF, NW, SEG, true, HP>(q, lw, vw, -one, hq, h5, mq);
                 } else {
-                    if (active) walk<HALF, NW, SEG, false, HP>(q, lw, vw, hq, h5, mq);
+                    if (active) walk<HALF, NW, SEG, false, HP>(q, lw, vw, -one, hq, h5, mq);
                 }
             }
             __syncwarp();
@@ -787,7 +855,7 @@ k_bitslice(BitsliceArgs a)
                         tm_store<EC>(tring + ts[k] * EC, en);  // the entering row takes the leaving row's place
 #pragma unroll
                         for (int w = 0; w < NW; w++) {
-                            planes_addsub<PV, KH>(V[w], hn[w], ho[w]);
+                            planes_addsub<PV, KH, !MULTI>(V[w], hn[w], ho[w]);
 #pragma unroll
                             for (int p = 0; p < PV; p++) Vs[k][w][p] = V[w][p];
                         }
