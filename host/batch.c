@@ -6,13 +6,14 @@
  * reference has no batch program; this one exists to exercise the multi-GPU entry of the C ABI
  * (sm_multi_*, include/stereo_b200.h) without Python.
  *
- *   stereobatch WIDTH HEIGHT NUM_SHIFTS SQUARE_WIDTH N_PAIRS [wrap|ghost] [u8|i32] [n_gpus]
+ *   stereobatch WIDTH HEIGHT NUM_SHIFTS SQUARE_WIDTH N_PAIRS [wrap|ghost] [u8|u16|i32] [n_gpus]
  *
  * Input: the synthetic textured pairs of SURVEY 8(d) (seed 1234 + 2k for pair k), threshold 0.15.
  * Output line (stdout):
  *   gpus = G, pairs = N, elapsed = S, pairs_per_s = P, mde_per_s = M, web_crc32 = XXXXXXXX
  * `elapsed` covers H2D, edges, hot path and D2H of all pairs (second of two runs); the CRC is zlib's
- * over the web array as returned (i32 little endian, or u8).
+ * over the web array as returned (i32 or u16 little endian, or u8).  u16 runs sm_multi_run_batch16, whose hot
+ * kernel writes the 16-bit web itself.
  */
 #include <stdint.h>
 #include <stdio.h>
@@ -72,12 +73,14 @@ static double now(void)
 int main(int argc, char **argv)
 {
     if (argc < 6) {
-        fprintf(stderr, "usage: %s width height num_shifts square_width n_pairs [wrap|ghost] [u8|i32] [n_gpus]\n", argv[0]);
+        fprintf(stderr, "usage: %s width height num_shifts square_width n_pairs [wrap|ghost] [u8|u16|i32] [n_gpus]\n",
+                argv[0]);
         return 1;
     }
     const int w = atoi(argv[1]), h = atoi(argv[2]), d = atoi(argv[3]), sw = atoi(argv[4]), n = atoi(argv[5]);
     const int variant = (argc > 6 && strcmp(argv[6], "ghost") == 0) ? SM_GHOST : SM_WRAP;
-    const int u8 = argc > 7 && strcmp(argv[7], "u8") == 0;
+    const int u8 = argc > 7 && strcmp(argv[7], "u8") == 0, u16 = argc > 7 && strcmp(argv[7], "u16") == 0;
+    const size_t elem = u8 ? 1 : (u16 ? 2 : 4); /* bytes per web element */
     int ngpu = sm_device_count();
     if (ngpu < 1) {
         fprintf(stderr, "error: no CUDA device: %s\n", sm_last_error());
@@ -93,19 +96,24 @@ int main(int argc, char **argv)
     void *web;
     CHECK(sm_host_alloc((void **)&first, npix * n));
     CHECK(sm_host_alloc((void **)&second, npix * n));
-    CHECK(sm_host_alloc(&web, npix * n * (u8 ? 1 : 4)));
+    CHECK(sm_host_alloc(&web, npix * n * elem));
     for (int k = 0; k < n; k++) synth_pair(1234 + 2 * (uint64_t)k, w, h, d, first + npix * k, second + npix * k);
 
     int devices[64];
     for (int g = 0; g < ngpu && g < 64; g++) devices[g] = g;
     sm_multi *m;
     CHECK(sm_multi_create(&m, devices, ngpu, w, h, d, sw, variant));
-    CHECK(sm_multi_run_batch(m, n, first, second, 0.15, web, u8, NULL)); /* first run: buffers, kernels */
-    double t1 = now();
-    CHECK(sm_multi_run_batch(m, n, first, second, 0.15, web, u8, NULL));
+    double t1 = 0.0;
+    for (int run = 0; run < 2; run++) { /* first run: buffers, kernels */
+        t1 = now();
+        if (u16)
+            CHECK(sm_multi_run_batch16(m, n, first, second, 0.15, (uint16_t *)web, NULL));
+        else
+            CHECK(sm_multi_run_batch(m, n, first, second, 0.15, web, u8, NULL));
+    }
     double t2 = now();
     unsigned long crc = crc32(0L, Z_NULL, 0);
-    const size_t bytes = npix * n * (u8 ? 1 : 4);
+    const size_t bytes = npix * n * elem;
     for (size_t off = 0; off < bytes; off += (size_t)1 << 30) {
         size_t len = bytes - off < ((size_t)1 << 30) ? bytes - off : ((size_t)1 << 30);
         crc = crc32(crc, (const unsigned char *)web + off, (unsigned)len);

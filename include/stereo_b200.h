@@ -115,7 +115,9 @@ typedef enum sm_shape {
 
 /* Message of the last failure on this thread ("" if none). */
 const char *sm_last_error(void);
-/* ABI version: (major << 16) | minor. */
+/* ABI version: (major << 16) | minor.  The 16-bit result entries (sm_match_wta_dev_batch16, sm_run_batch16,
+ * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16) are additions to 1.3 that leave every other entry as it
+ * was; clients detect them by symbol. */
 int sm_version(void);
 /* Number of CUDA devices visible, or a negative sm_status. */
 int sm_device_count(void);
@@ -201,6 +203,14 @@ int sm_match_wta_dev_batch(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edge
                            const uint8_t *d_second_edges, size_t edge_stride, int32_t *d_best,
                            int32_t *d_web, size_t out_stride);
 
+/* The same with 16-bit results, stored by the hot kernel itself (2 B per pixel and array instead of 4): web is in
+ * 1..num_shifts <= 512 and best at most (2*(square_width/2)+1)^2 <= 3969, so both are exact.  d_best may be NULL:
+ * then of the caller's memory only d_web is written (best goes to a scratch array of the context's).  Checks, streams, pairs per launch, the kernel chosen (SM_INFO_KERNEL_SHAPE) and
+ * sm_elapsed_ms / sm_last_launches are those of sm_match_wta_dev_batch; n_pairs == 1 is the one-pair launch of
+ * sm_match_wta. */
+int sm_match_wta_dev_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edges, const uint8_t *d_second_edges,
+                             size_t edge_stride, uint16_t *d_best, uint16_t *d_web, size_t out_stride);
+
 /* Device time of the last sm_match_wta* call on this context, CUDA events on the
  * context's stream (the reference brackets the whole algorithm() with
  * CLOCK_MONOTONIC instead, stereo.cu:308,334-335).  Waits for the call to finish. */
@@ -243,6 +253,8 @@ int sm_download(sm_ctx *ctx, int which, int shift, void *host);
 
 /* web as u8 (valid when num_shifts <= 255): a quarter of the D2H bytes. */
 int sm_download_web_u8(sm_ctx *ctx, uint8_t *host);
+/* web as u16 (any num_shifts): half the D2H bytes. */
+int sm_download_web_u16(sm_ctx *ctx, uint16_t *host);
 
 /* ---- whole pairs, batched (SURVEY 8e, config 4; 8f n4) ------------------------ */
 
@@ -256,6 +268,10 @@ int sm_download_web_u8(sm_ctx *ctx, uint8_t *host);
  * context per device (pair k -> device k mod n), no cross-device traffic. */
 int sm_run_batch(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second,
                  double threshold, void *web_out, int web_u8, int32_t *best_out);
+/* The same with 16-bit web and best for any num_shifts: the hot kernel writes them directly (no int32 array, no
+ * narrowing launch) and each comes back as one copy per group at 2 B per pixel.  best_out may be NULL. */
+int sm_run_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                   uint16_t *web_out, uint16_t *best_out);
 
 /* The same over several GPUs of one box (SURVEY 8e, BASELINE config 4: whole pairs sharded across the
  * GPUs, inputs scattered from the host, no cross-device traffic): one context and one host thread per
@@ -265,6 +281,9 @@ int sm_multi_create(sm_multi **out, const int *devices, int n_devices, int width
                     int num_shifts, int square_width, int variant);
 int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
                        double threshold, void *web_out, int web_u8, int32_t *best_out);
+/* The same through sm_run_batch16 (best_out may be NULL). */
+int sm_multi_run_batch16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                         uint16_t *web_out, uint16_t *best_out);
 int sm_multi_device_count(const sm_multi *m);
 int sm_multi_destroy(sm_multi *m);
 
@@ -277,6 +296,10 @@ int sm_bands_create(sm_bands **out, const int *devices, int n_devices, int width
                     int num_shifts, int square_width, int variant);
 int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                  int32_t *web_out, int32_t *best_out);
+/* The same with 16-bit web / best (best_out may be NULL): each band's hot kernel writes its rows as u16 and only
+ * those rows are copied back. */
+int sm_bands_run16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                   uint16_t *web_out, uint16_t *best_out);
 int sm_bands_destroy(sm_bands *b);
 
 /* ---- geometry helpers (host-side, no GPU) --------------------------------------- */

@@ -33,12 +33,13 @@ SYMBOLS = [
     "sm_last_error", "sm_version", "sm_device_count", "sm_host_alloc", "sm_host_free",
     "sm_create", "sm_create_band", "sm_destroy", "sm_set_stream", "sm_set_kernel",
     "sm_synchronize", "sm_upload_f64", "sm_upload_u8", "sm_edges", "sm_set_edges",
-    "sm_match_wta", "sm_match_wta_dev", "sm_match_wta_dev_batch", "sm_elapsed_ms", "sm_last_launches",
+    "sm_match_wta", "sm_match_wta_dev", "sm_match_wta_dev_batch", "sm_match_wta_dev_batch16",
+    "sm_elapsed_ms", "sm_last_launches",
     "sm_profile_begin", "sm_profile_read", "sm_set_option", "sm_get_info",
     "sm_fill_web_holes", "sm_set_web", "sm_draw_contour_map", "sm_download", "sm_download_web_u8",
-    "sm_run_batch", "sm_band_rows",
-    "sm_multi_create", "sm_multi_run_batch", "sm_multi_device_count", "sm_multi_destroy",
-    "sm_bands_create", "sm_bands_run", "sm_bands_destroy",
+    "sm_download_web_u16", "sm_run_batch", "sm_run_batch16", "sm_band_rows",
+    "sm_multi_create", "sm_multi_run_batch", "sm_multi_run_batch16", "sm_multi_device_count", "sm_multi_destroy",
+    "sm_bands_create", "sm_bands_run", "sm_bands_run16", "sm_bands_destroy",
 ]
 
 
@@ -77,6 +78,7 @@ def lib() -> C.CDLL:
         L.sm_match_wta.argtypes = [vp]
         L.sm_match_wta_dev.argtypes = [vp, vp, vp, vp, vp]
         L.sm_match_wta_dev_batch.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
+        L.sm_match_wta_dev_batch16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
         L.sm_elapsed_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.sm_last_launches.argtypes = [vp]
         L.sm_profile_begin.argtypes = [vp, i]
@@ -86,14 +88,18 @@ def lib() -> C.CDLL:
         L.sm_draw_contour_map.argtypes = [vp, i, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.sm_download.argtypes = [vp, i, i, vp]
         L.sm_download_web_u8.argtypes = [vp, vp]
+        L.sm_download_web_u16.argtypes = [vp, vp]
         L.sm_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
+        L.sm_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_band_rows.argtypes = [i, i, i, C.POINTER(i), C.POINTER(i)]
         L.sm_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_multi_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
+        L.sm_multi_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_multi_device_count.argtypes = [vp]
         L.sm_multi_destroy.argtypes = [vp]
         L.sm_bands_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_bands_run.argtypes = [vp, vp, vp, d, vp, vp]
+        L.sm_bands_run16.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_destroy.argtypes = [vp]
         _lib = L
     return _lib
@@ -227,6 +233,12 @@ class StereoContext:
         _check(lib().sm_match_wta_dev_batch(self._c, n_pairs, C.c_void_p(d_first_edges), C.c_void_p(d_second_edges),
                                             edge_stride, C.c_void_p(d_best), C.c_void_p(d_web), out_stride))
 
+    def match_wta_dev_batch16(self, n_pairs: int, d_first_edges: int, d_second_edges: int, edge_stride: int,
+                              d_best, d_web: int, out_stride: int):
+        """match_wta_dev_batch with uint16 outputs written by the hot kernel; d_best may be None (web only)."""
+        _check(lib().sm_match_wta_dev_batch16(self._c, n_pairs, C.c_void_p(d_first_edges), C.c_void_p(d_second_edges),
+                                              edge_stride, C.c_void_p(d_best or None), C.c_void_p(d_web), out_stride))
+
     def elapsed_ms(self) -> float:
         ms = C.c_float()
         _check(lib().sm_elapsed_ms(self._c, C.byref(ms)))
@@ -271,24 +283,46 @@ class StereoContext:
         _check(lib().sm_download_web_u8(self._c, _ptr(out)))
         return out
 
-    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None):
-        """first/second: (n, H, W) u8.  Returns web (n, H, W) [and best]."""
+    def download_web_u16(self, out=None):
+        if out is None:
+            out = np.zeros((self.H, self.W), np.uint16)
+        assert out.dtype == np.uint16 and out.shape == (self.H, self.W) and out.flags.c_contiguous
+        _check(lib().sm_download_web_u16(self._c, _ptr(out)))
+        return out
+
+    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False):
+        """first/second: (n, H, W) u8.  Returns web (n, H, W) [and best]: int32, web as uint8 with web_u8, or (web16)
+        both as uint16, written by the hot kernel itself."""
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
-        if web_out is None:
-            web_out = np.zeros((n, self.H, self.W), np.uint8 if web_u8 else np.int32)
-        best = np.zeros((n, self.H, self.W), np.int32) if want_best else None
-        _check(lib().sm_run_batch(self._c, n, _ptr(first), _ptr(second), threshold, _ptr(web_out),
-                                  int(web_u8), _ptr(best) if want_best else None))
-        return (web_out, best) if want_best else web_out
+        return _run_batch(self._c, lib().sm_run_batch, lib().sm_run_batch16, first, second, threshold, web_u8,
+                          want_best, web_out, web16)
 
     # -- convenience: the reference's whole step 2 on host edge maps -----------
     def match_wta_host(self, first_edges, second_edges):
         self.set_edges(first_edges, second_edges)
         self.match_wta()
         return self.download(BEST), self.download(WEB)
+
+
+def _run_batch(handle, run, run16, first, second, threshold, web_u8, want_best, web_out, web16):
+    """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16)."""
+    if web16 and web_u8:
+        raise ValueError("web16 and web_u8 exclude each other")
+    n, H, W = first.shape
+    dt = np.uint16 if web16 else (np.uint8 if web_u8 else np.int32)
+    if web_out is None:
+        web_out = np.zeros((n, H, W), dt)
+    assert web_out.dtype == dt and web_out.shape == (n, H, W) and web_out.flags.c_contiguous
+    best = np.zeros((n, H, W), np.uint16 if web16 else np.int32) if want_best else None
+    if web16:
+        _check(run16(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None))
+    else:
+        _check(run(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), int(web_u8),
+                   _ptr(best) if want_best else None))
+    return (web_out, best) if want_best else web_out
 
 
 class MultiGpuBatch:
@@ -302,17 +336,13 @@ class MultiGpuBatch:
         _check(lib().sm_multi_create(C.byref(self._m), arr, len(devices), width, height, num_shifts, square_width,
                                      variant))
 
-    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None):
+    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False):
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
-        if web_out is None:
-            web_out = np.zeros((n, self.H, self.W), np.uint8 if web_u8 else np.int32)
-        best = np.zeros((n, self.H, self.W), np.int32) if want_best else None
-        _check(lib().sm_multi_run_batch(self._m, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), int(web_u8),
-                                        _ptr(best) if want_best else None))
-        return (web_out, best) if want_best else web_out
+        return _run_batch(self._m, lib().sm_multi_run_batch, lib().sm_multi_run_batch16, first, second, threshold,
+                          web_u8, want_best, web_out, web16)
 
     def close(self):
         if self._m:
@@ -336,14 +366,16 @@ class MultiGpuBands:
         _check(lib().sm_bands_create(C.byref(self._b), arr, len(devices), width, height, num_shifts, square_width,
                                      variant))
 
-    def run(self, first, second, threshold=0.15, want_best=False):
+    def run(self, first, second, threshold=0.15, want_best=False, web16=False):
+        """web [and best] of one pair: int32, or uint16 with web16."""
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         assert first.shape == second.shape == (self.H, self.W)
-        web = np.zeros((self.H, self.W), np.int32)
-        best = np.zeros((self.H, self.W), np.int32) if want_best else None
-        _check(lib().sm_bands_run(self._b, _ptr(first), _ptr(second), threshold, _ptr(web),
-                                  _ptr(best) if want_best else None))
+        dt = np.uint16 if web16 else np.int32
+        web = np.zeros((self.H, self.W), dt)
+        best = np.zeros((self.H, self.W), dt) if want_best else None
+        run = lib().sm_bands_run16 if web16 else lib().sm_bands_run
+        _check(run(self._b, _ptr(first), _ptr(second), threshold, _ptr(web), _ptr(best) if want_best else None))
         return (web, best) if want_best else web
 
     def close(self):

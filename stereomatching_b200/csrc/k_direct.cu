@@ -41,7 +41,9 @@ __device__ __forceinline__ void window(const HotArgs &a, int x, int j, int i, in
     }
 }
 
-__global__ void __launch_bounds__(256) k_direct(HotArgs a)
+// best / web of pixel x of band row j, stored as T; best may be NULL (16-bit outputs: web only)
+template <typename T>
+__device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *web_out)
 {
     int x = blockIdx.x * blockDim.x + threadIdx.x;
     int j = blockIdx.y * blockDim.y + threadIdx.y;
@@ -57,15 +59,29 @@ __global__ void __launch_bounds__(256) k_direct(HotArgs a)
         }
     }
     size_t p = (size_t)(a.row0 + j) * a.g.W + x;
-    a.best[p] = best;
-    a.web[p] = web;
+    if (sizeof(T) == 4 || best_out) best_out[p] = (T)best;  // (the int32 kernel always has a best)
+    web_out[p] = (T)web;
 }
 
-int launch_direct(const HotArgs &a, cudaStream_t s)
+__global__ void __launch_bounds__(256) k_direct(HotArgs a)
+{
+    direct_pixel(a, static_cast<int32_t *>(a.best), static_cast<int32_t *>(a.web));
+}
+
+// the 16-bit twin (a.best may be NULL)
+__global__ void __launch_bounds__(256) k_direct16(HotArgs a)
+{
+    direct_pixel(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web));
+}
+
+int launch_direct(const HotArgs &a, cudaStream_t s, bool out16)
 {
     dim3 block(32, 8);
     dim3 grid((a.g.W + block.x - 1) / block.x, (a.g.BH + block.y - 1) / block.y);
-    k_direct<<<grid, block, 0, s>>>(a);
+    if (out16)
+        k_direct16<<<grid, block, 0, s>>>(a);
+    else
+        k_direct<<<grid, block, 0, s>>>(a);
     SM_CUDA(cudaGetLastError());
     return 1;
 }
@@ -100,6 +116,7 @@ int launch_planes(const HotArgs &a, int shift, uint8_t *match, int32_t *score_al
 void warm_direct()
 {
     warm_kernel(k_direct);
+    warm_kernel(k_direct16);
     warm_kernel(k_planes);
 }
 

@@ -134,27 +134,41 @@ int launch_contour(const int32_t *web, size_t n, const int32_t *d_minmax_slot, i
     return 1;
 }
 
+// four elements per thread: one 16-byte load, one 4- (uint8_t) or 8-byte (uint16_t) store
+template <typename T> struct Narrow4;
+template <> struct Narrow4<uint8_t> {
+    using V = uchar4;
+};
+template <> struct Narrow4<uint16_t> {
+    using V = ushort4;
+};
+
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_i32_to_u8(const int32_t *__restrict__ src, uint8_t *__restrict__ dst, size_t n)
+k_narrow(const int32_t *__restrict__ src, T *__restrict__ dst, size_t n)
 {
+    using V = typename Narrow4<T>::V;
     size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i + 3 < n) {
         int4 v = *reinterpret_cast<const int4 *>(src + i);
-        uchar4 o = make_uchar4((unsigned char)v.x, (unsigned char)v.y, (unsigned char)v.z,
-                               (unsigned char)v.w);
-        *reinterpret_cast<uchar4 *>(dst + i) = o;
+        V o;
+        o.x = (T)v.x, o.y = (T)v.y, o.z = (T)v.z, o.w = (T)v.w;
+        *reinterpret_cast<V *>(dst + i) = o;
     } else {
-        for (; i < n; i++) dst[i] = (uint8_t)src[i];
+        for (; i < n; i++) dst[i] = (T)src[i];
     }
 }
 
-int launch_i32_to_u8(const int32_t *src, uint8_t *dst, size_t n, cudaStream_t s)
+template <typename T>
+int launch_narrow(const int32_t *src, T *dst, size_t n, cudaStream_t s)
 {
     size_t q = (n + 3) / 4;
-    k_i32_to_u8<<<(unsigned)((q + 255) / 256), 256, 0, s>>>(src, dst, n);
+    k_narrow<T><<<(unsigned)((q + 255) / 256), 256, 0, s>>>(src, dst, n);
     SM_CUDA(cudaGetLastError());
     return 1;
 }
+template int launch_narrow<uint8_t>(const int32_t *, uint8_t *, size_t, cudaStream_t);
+template int launch_narrow<uint16_t>(const int32_t *, uint16_t *, size_t, cudaStream_t);
 
 void warm_step3()
 {
@@ -162,7 +176,8 @@ void warm_step3()
     warm_kernel(k_minmax_arm);
     warm_kernel(k_minmax);
     warm_kernel(k_contour);
-    warm_kernel(k_i32_to_u8);
+    warm_kernel(k_narrow<uint8_t>);
+    warm_kernel(k_narrow<uint16_t>);
 }
 
 }  // namespace smb

@@ -69,7 +69,9 @@ inline int packed_words_per_row(int W, int half, int D)
 struct HotArgs {
     PackedGeom g;
     const uint32_t *LA, *LB, *RB;  // [ER][WPR]
-    int32_t *best, *web;           // frame arrays [FH][W]; band row j -> frame row row0 + j
+    // frame arrays [FH][W] of int32_t, or of uint16_t for the 16-bit kernels (the same argument layout for both
+    // families); band row j -> frame row row0 + j.  The 16-bit direct kernel takes a NULL best (web only)
+    void *best, *web;
     int row0;
     // several independent pairs in one launch (blockIdx.z): pair p's planes are plane_stride
     // words further, its outputs out_stride elements further
@@ -96,10 +98,12 @@ struct LaunchRecord {
 int launch_pack(const uint8_t *e1, const uint8_t *e2, int FH, int row0, int variant,
                 const PackedGeom &g, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
                 int npairs = 1, size_t edge_stride = 0, size_t plane_stride = 0);
-int launch_direct(const HotArgs &a, cudaStream_t s);
+int launch_direct(const HotArgs &a, cudaStream_t s, bool out16 = false);  // out16: the 16-bit twin
 int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);
+int launch_bitslice16(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);  // uint16_t outputs
 bool bitslice_supports(int half, int D);
 int prepare_bitslice(const HotArgs &a, int num_sms);
+int prepare_bitslice16(const HotArgs &a, int num_sms);
 int bitslice_tmem_columns(const HotArgs &a);
 int bitslice_pairs_per_launch(const HotArgs &a, int num_sms, int max_pairs);
 // force the (lazily loaded) kernels of each translation unit into the context
@@ -135,6 +139,8 @@ int launch_minmax_arm(int32_t *d_minmax, cudaStream_t s);
 int launch_minmax(const int32_t *a, size_t n, int32_t *d_minmax, int cur, cudaStream_t s);
 int launch_contour(const int32_t *web, size_t n, const int32_t *d_minmax_slot, int lines, uint8_t *out,
                    cudaStream_t s);
-int launch_i32_to_u8(const int32_t *src, uint8_t *dst, size_t n, cudaStream_t s);
+// int32 -> T (uint8_t or uint16_t), element-wise truncation: the caller guarantees that the values fit
+template <typename T>
+int launch_narrow(const int32_t *src, T *dst, size_t n, cudaStream_t s);
 
 }  // namespace smb

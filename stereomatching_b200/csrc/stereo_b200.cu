@@ -67,6 +67,9 @@ struct sm_ctx {
     int pipe_group_opt = 0;        // SM_OPT_PIPE_GROUP: pairs per sm_run_batch stage (0: by frame size)
     int32_t *best = nullptr, *web = nullptr;
     bool have_web = false;
+    // frame-sized 16-bit arrays: sm_bands_run16's results, sm_download_web_u16's narrowed web
+    uint16_t *best16 = nullptr, *web16 = nullptr;
+    bool prepared16 = false;  // the 16-bit bit-sliced kernels of this geometry are loaded (prepare_bitslice16)
     int32_t *web2 = nullptr, *tmp = nullptr;  // step 3 ping-pong
     const int32_t *web_filled = nullptr;      // result of fill_web_holes (may alias web)
     bool have_web2 = false;
@@ -90,6 +93,11 @@ struct sm_ctx {
              *pRB[NPB] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_packed[NPB] = {nullptr, nullptr, nullptr}, ev_used[NPB] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr;
+    // the best of 16-bit batches without a caller's best (the bit-sliced kernel always stores it): one scratch per
+    // plane set, batch_group_cap frames each (ev_used[b] orders its reuse like that of the plane set)
+    // (with the caller's pair stride, out_stride: pbest16_elems elements each)
+    uint16_t *pBest16[NPB] = {nullptr, nullptr, nullptr};
+    size_t pbest16_elems = 0;
     // scratch for on-demand debug planes / u8 web
     uint8_t *scratch_u8 = nullptr;
     int32_t *scratch_i32 = nullptr;
@@ -106,6 +114,8 @@ struct sm_ctx {
         int32_t *web[NPIPE] = {nullptr, nullptr, nullptr};    // [group][npix]
         int32_t *best[NPIPE] = {nullptr, nullptr, nullptr};   // [group][npix]
         uint8_t *web8[NPIPE] = {nullptr, nullptr, nullptr};   // [group][npix], only for the u8 result
+        // the 16-bit results, written by the hot path itself ([group][npix]; best16 only when the caller wants best)
+        uint16_t *web16[NPIPE] = {nullptr, nullptr, nullptr}, *best16[NPIPE] = {nullptr, nullptr, nullptr};
         cudaEvent_t ev_up[NPIPE] = {nullptr, nullptr, nullptr}, ev_comp[NPIPE] = {nullptr, nullptr, nullptr},
                     ev_down[NPIPE] = {nullptr, nullptr, nullptr};
     } pipe;
@@ -207,36 +217,63 @@ int copy_band_d2h(sm_ctx *c, T *host, const T *dev)
     return SM_OK;
 }
 
-HotArgs hot_args(sm_ctx *c, int32_t *best, int32_t *web)
+// Where a hot-path call writes best / web: int32 arrays, or (web16 set) 16-bit ones, best16 possibly NULL.
+struct Outputs {
+    int32_t *best = nullptr, *web = nullptr;
+    uint16_t *best16 = nullptr, *web16 = nullptr;
+    // pair k of a batch: every array k * stride elements further
+    Outputs pair(size_t k, size_t stride) const
+    {
+        auto at = [&](auto *p) { return p ? p + k * stride : p; };
+        return {at(best), at(web), at(best16), at(web16)};
+    }
+};
+
+HotArgs hot_args(sm_ctx *c, const Outputs &o)
 {
     HotArgs a;
     a.g = c->g;
     a.LA = c->LA;
     a.LB = c->LB;
     a.RB = c->RB;
-    a.best = best;
-    a.web = web;
+    a.best = o.web16 ? (void *)o.best16 : (void *)o.best;
+    a.web = o.web16 ? (void *)o.web16 : (void *)o.web;
     a.row0 = c->row0;
     a.force_segs = c->tuned_segs;
     a.blocks_per_sm = c->occ;
     return a;
 }
 
-int launch_main(sm_ctx *c, const HotArgs &a, cudaStream_t st)
+int hot_kernel(const sm_ctx *c)
 {
-    int k = c->kernel;
-    if (k == SM_KERNEL_AUTO) k = bitslice_supports(c->half, c->D) ? SM_KERNEL_BITSLICE : SM_KERNEL_DIRECT;
+    return c->kernel == SM_KERNEL_AUTO ? (bitslice_supports(c->half, c->D) ? SM_KERNEL_BITSLICE : SM_KERNEL_DIRECT)
+                                       : c->kernel;
+}
+
+// The bit-sliced kernel always stores best (it merges 64-shift chunks through it, and a per-store predicate would cost
+// its 16-bit family registers): a 16-bit call without a best of the caller's gives it a scratch array.
+bool stores_best(const sm_ctx *c) { return hot_kernel(c) == SM_KERNEL_BITSLICE; }
+
+// The main kernel: of the 16-bit family with out16, else of the int32 one.
+int launch_main(sm_ctx *c, const HotArgs &a, bool out16, cudaStream_t st)
+{
+    const int k = hot_kernel(c);
     if (k == SM_KERNEL_BITSLICE) {
         if (!bitslice_supports(c->half, c->D)) {
             set_error("bit-sliced kernel does not cover square_width %d / num_shifts %d", c->sw, c->D);
             return SM_ERR_ARG;
         }
+        if (out16 && !c->prepared16) {  // (sm_create prepared the int32 family)
+            const int rc = prepare_bitslice16(hot_args(c, Outputs{}), c->num_sms);
+            if (rc < 0) return rc;
+            c->prepared16 = true;
+        }
         LaunchRecord rec;
-        const int rc = launch_bitslice(a, c->num_sms, st, &rec);
+        const int rc = out16 ? launch_bitslice16(a, c->num_sms, st, &rec) : launch_bitslice(a, c->num_sms, st, &rec);
         if (rc >= 0) c->last_launch = rec;
         return rc;
     }
-    const int rc = launch_direct(a, st);
+    const int rc = launch_direct(a, st, out16);
     if (rc >= 0) {
         c->last_launch.shape = SM_SHAPE_DIRECT;
         c->last_launch.row_runs = 0;
@@ -244,7 +281,7 @@ int launch_main(sm_ctx *c, const HotArgs &a, cudaStream_t st)
     return rc;
 }
 
-int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, int32_t *best, int32_t *web)
+int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, const Outputs &out)
 {
     int launches = 0, rc;
     cudaEvent_t *pe = (c->prof_ev && c->prof_n < c->prof_cap) ? c->prof_ev + 3 * c->prof_n : nullptr;
@@ -258,7 +295,7 @@ int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, int32_t *best, int3
         launches += rc;
     }
     if (pe) SM_CUDA(cudaEventRecord(pe[1], c->stream));
-    HotArgs a = hot_args(c, best, web);
+    HotArgs a = hot_args(c, out);
 #ifdef SMB_DEV
     static const bool no_pdl = getenv("SMB_NO_PDL") && atoi(getenv("SMB_NO_PDL"));  // experiment hook, development build only
 #else
@@ -268,7 +305,7 @@ int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, int32_t *best, int3
     // per-kernel profile put an event in between: the main kernel may start as its programmatic dependent.
     // (It waits for every earlier grid of the stream to complete before it reads anything, whatever that grid is.)
     a.after_pack = pe == nullptr && !no_pdl;
-    rc = launch_main(c, a, c->stream);
+    rc = launch_main(c, a, out.web16 != nullptr, c->stream);
     if (rc < 0) return rc;
     launches += rc;
     SM_CUDA(cudaEventRecord(c->ev1, c->stream));
@@ -297,7 +334,7 @@ void profile_free(sm_ctx *c)
 extern "C" const char *sm_last_error(void) { return g_err; }
 
 // 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out;
-// 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS
+// 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS; then, additive, the 16-bit result entries (*16, sm_download_web_u16)
 extern "C" int sm_version(void) { return (1 << 16) | 3; }
 
 extern "C" int sm_device_count(void)
@@ -412,7 +449,7 @@ extern "C" int sm_create_band(sm_ctx **out, int device, int width, int frame_hei
     warm_direct();
     warm_step3();
     if (bitslice_supports(c->half, c->D)) {
-        HotArgs a = hot_args(c, c->best, c->web);
+        HotArgs a = hot_args(c, {c->best, c->web});
         if ((rc = prepare_bitslice(a, c->num_sms)) < 0) return fail(rc);
         c->occ = rc;
     }
@@ -447,7 +484,8 @@ extern "C" int sm_destroy(sm_ctx *c)
             cudaStreamDestroy(st);
         }
     for (int k = 0; k < sm_ctx::NPIPE; k++) {
-        void *pp[] = {c->pipe.img[k], c->pipe.edg[k], c->pipe.web[k], c->pipe.best[k], c->pipe.web8[k]};
+        void *pp[] = {c->pipe.img[k], c->pipe.edg[k], c->pipe.web[k], c->pipe.best[k], c->pipe.web8[k],
+                      c->pipe.web16[k], c->pipe.best16[k]};
         for (void *p : pp)
             if (p) cudaFree(p);
         for (cudaEvent_t e : {c->pipe.ev_up[k], c->pipe.ev_comp[k], c->pipe.ev_down[k]})
@@ -457,7 +495,8 @@ extern "C" int sm_destroy(sm_ctx *c)
     if (c->minmax_host) cudaFreeHost(c->minmax_host);
     void *ptrs[] = {c->img_u8[0], nullptr,      c->img_f64[0], c->img_f64[1], c->edges[0], nullptr,  // [1] = [0] + npix
                     c->best,      c->web,       c->web2,       c->tmp,        c->out,      c->minmax,
-                    c->LA,        c->LB,        c->RB,         c->scratch_u8, c->scratch_i32};
+                    c->LA,        c->LB,        c->RB,         c->scratch_u8, c->scratch_i32,
+                    c->best16,    c->web16};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->prof_ev) profile_free(c);
@@ -476,6 +515,7 @@ extern "C" int sm_destroy(sm_ctx *c)
         if (c->pRB[k]) cudaFree(c->pRB[k]);
         if (c->ev_packed[k]) cudaEventDestroy(c->ev_packed[k]);
         if (c->ev_used[k]) cudaEventDestroy(c->ev_used[k]);
+        if (c->pBest16[k]) cudaFree(c->pBest16[k]);
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -530,7 +570,7 @@ extern "C" int sm_get_info(sm_ctx *c, int what)
     switch (what) {
     case SM_INFO_WARPS_PER_SM: return c->occ;
     case SM_INFO_PAIRS_PER_LAUNCH: return c->batch_group_cap;
-    case SM_INFO_TMEM_COLUMNS: return bitslice_supports(c->half, c->D) ? bitslice_tmem_columns(hot_args(c, c->best, c->web)) : 0;
+    case SM_INFO_TMEM_COLUMNS: return bitslice_supports(c->half, c->D) ? bitslice_tmem_columns(hot_args(c, {c->best, c->web})) : 0;
     case SM_INFO_KERNEL_SHAPE: return c->last_launch.shape;
     case SM_INFO_ROW_RUNS: return c->last_launch.row_runs;
     case SM_INFO_EDGE_THRESHOLDS: {
@@ -659,7 +699,7 @@ extern "C" int sm_match_wta(sm_ctx *c)
         set_error("sm_match_wta: no edges (call sm_edges or sm_set_edges first)");
         return SM_ERR_STATE;
     }
-    int rc = run_hot(c, c->edges[0], c->edges[1], c->best, c->web);
+    int rc = run_hot(c, c->edges[0], c->edges[1], {c->best, c->web});
     if (rc) return rc;
     c->have_web = true;
     c->web_may_have_holes = false;
@@ -672,20 +712,20 @@ extern "C" int sm_match_wta_dev(sm_ctx *c, const uint8_t *d_first_edges, const u
 {
     SM_ENTER(c);
     SM_REQUIRE(d_first_edges && d_second_edges && d_best && d_web, "sm_match_wta_dev: NULL pointer");
-    return run_hot(c, d_first_edges, d_second_edges, d_best, d_web);
+    return run_hot(c, d_first_edges, d_second_edges, {d_best, d_web});
 }
 
 // The batched hot path on device-resident inputs: either byte edge maps (packed by k_pack) or, with
 // from_images, the 8-bit images themselves (edges detected straight into the packed planes by k_edges_planes;
 // the byte maps never exist).  Producer launches run on a second stream one group ahead of the main kernels.
+// Results go to `out` (int32 or 16-bit), pair k's out_stride * k elements further.
 static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold, const uint8_t *d_first_edges,
-                      const uint8_t *d_second_edges, size_t edge_stride, int32_t *d_best, int32_t *d_web,
-                      size_t out_stride)
+                      const uint8_t *d_second_edges, size_t edge_stride, const Outputs &out, size_t out_stride)
 {
     constexpr int NPB = sm_ctx::NPB;
     const size_t pw = (size_t)c->g.ER * c->g.WPR;
-    int kk = c->kernel;
-    if (kk == SM_KERNEL_AUTO) kk = bitslice_supports(c->half, c->D) ? SM_KERNEL_BITSLICE : SM_KERNEL_DIRECT;
+    const int kk = hot_kernel(c);
+    const bool scratch_best = out.web16 && !out.best16 && stores_best(c);
     if (!c->batch_ready) {
         // Set-up of the batch path.  Every object is created only if it does not exist yet and the ready flag is
         // set last, so that a call that failed half way (out of memory on the plane sets, say) is simply resumed
@@ -694,7 +734,7 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         if (c->batch_group_cap == 0) {
             c->batch_group_cap = 1;
             if (bitslice_supports(c->half, c->D)) {
-                HotArgs a = hot_args(c, d_best, d_web);
+                HotArgs a = hot_args(c, out);
                 int pmax = 16;
 #ifdef SMB_DEV
                 if (getenv("SMB_PMAX")) pmax = atoi(getenv("SMB_PMAX"));  // experiment hook, development build only
@@ -715,6 +755,22 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
             if (!c->ev_used[k]) SM_CUDA(cudaEventCreateWithFlags(&c->ev_used[k], cudaEventDisableTiming));
         }
         c->batch_ready = true;
+    }
+    if (scratch_best) {
+        // pair k of a launch stores its best k * out_stride elements further, like its web (the 16-bit kernels take
+        // the int32 kernels' argument layout: one stride for both arrays)
+        const size_t need = out_stride * (size_t)c->batch_group_cap;
+        if (need > c->pbest16_elems)
+            for (int k = 0; k < NPB; k++)
+                if (c->pBest16[k]) {
+                    SM_CUDA(cudaFree(c->pBest16[k]));  // (waits for the device: no launch still uses it)
+                    c->pBest16[k] = nullptr;
+                }
+        for (int k = 0; k < NPB; k++) {
+            int rc;
+            if ((rc = dev_alloc(&c->pBest16[k], need > c->pbest16_elems ? need : c->pbest16_elems))) return rc;
+        }
+        if (need > c->pbest16_elems) c->pbest16_elems = need;
     }
     // the kernel may have been switched since the last call (sm_set_kernel): the literal kernel takes one pair
     // per launch, the bit-sliced one a group
@@ -751,14 +807,16 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
             SM_CUDA(cudaEventRecord(pe[0], ms));  // pack runs on the other stream: not timed here
             SM_CUDA(cudaEventRecord(pe[1], ms));
         }
-        HotArgs a = hot_args(c, d_best + (size_t)k * out_stride, d_web + (size_t)k * out_stride);
+        const Outputs o = out.pair((size_t)k, out_stride);
+        HotArgs a = hot_args(c, o);
+        if (scratch_best) a.best = c->pBest16[b];
         a.LA = c->pLA[b];
         a.LB = c->pLB[b];
         a.RB = c->pRB[b];
         a.npairs = np;
         a.plane_stride = pw;
         a.out_stride = out_stride;
-        rc = launch_main(c, a, ms);
+        rc = launch_main(c, a, o.web16 != nullptr, ms);
         if (rc < 0) return rc;
         launches += rc;
         if (pe) {
@@ -784,7 +842,18 @@ extern "C" int sm_match_wta_dev_batch(sm_ctx *c, int n_pairs, const uint8_t *d_f
     SM_REQUIRE(n_pairs >= 0 && d_first_edges && d_second_edges && d_best && d_web,
                "sm_match_wta_dev_batch: bad arguments");
     SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch: stride below frame size");
-    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, d_best, d_web, out_stride);
+    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, {d_best, d_web}, out_stride);
+}
+
+extern "C" int sm_match_wta_dev_batch16(sm_ctx *c, int n_pairs, const uint8_t *d_first_edges,
+                                        const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best,
+                                        uint16_t *d_web, size_t out_stride)
+{
+    SM_REQUIRE(n_pairs >= 0 && d_first_edges && d_second_edges && d_web, "sm_match_wta_dev_batch16: bad arguments");
+    SM_ENTER(c);
+    SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch16: stride below frame size");
+    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, {nullptr, nullptr, d_best, d_web},
+                      out_stride);
 }
 
 extern "C" int sm_elapsed_ms(sm_ctx *c, float *ms)
@@ -950,7 +1019,7 @@ extern "C" int sm_download(sm_ctx *c, int which, int shift, void *host)
         rc = launch_pack(c->edges[0], c->edges[1], c->FH, c->row0, c->variant, c->g, c->LA, c->LB, c->RB,
                          c->stream);
         if (rc < 0) return rc;
-        HotArgs a = hot_args(c, nullptr, nullptr);
+        HotArgs a = hot_args(c, Outputs{});
         rc = launch_planes(a, shift, which == SM_MATCH ? c->scratch_u8 : nullptr,
                            which == SM_SCORE_ALL ? c->scratch_i32 : nullptr,
                            which == SM_SCORE ? c->scratch_i32 : nullptr, c->stream);
@@ -992,7 +1061,7 @@ static int queue_web_u8(sm_ctx *c, uint8_t *host)
     int rc;
     if ((rc = dev_alloc(&c->scratch_u8, c->npix()))) return rc;
     size_t off = (size_t)c->row0 * c->W, n = (size_t)(c->row1 - c->row0) * c->W;
-    if ((rc = launch_i32_to_u8(c->web + off, c->scratch_u8 + off, n, c->stream)) < 0) return rc;
+    if ((rc = launch_narrow(c->web + off, c->scratch_u8 + off, n, c->stream)) < 0) return rc;
     return copy_band_d2h(c, host, c->scratch_u8);
 }
 
@@ -1011,16 +1080,41 @@ extern "C" int sm_download_web_u8(sm_ctx *c, uint8_t *host)
     return SM_OK;
 }
 
+extern "C" int sm_download_web_u16(sm_ctx *c, uint16_t *host)
+{
+    SM_REQUIRE(host, "sm_download_web_u16: NULL host pointer");
+    SM_ENTER(c);
+    if (!c->have_web) {
+        set_error("sm_download_web_u16: no web (call sm_match_wta first)");
+        return SM_ERR_STATE;
+    }
+    int rc;
+    if ((rc = dev_alloc(&c->web16, c->npix()))) return rc;
+    size_t off = (size_t)c->row0 * c->W, n = (size_t)(c->row1 - c->row0) * c->W;
+    if ((rc = launch_narrow(c->web + off, c->web16 + off, n, c->stream)) < 0) return rc;
+    if ((rc = copy_band_d2h(c, host, c->web16))) return rc;
+    SM_CUDA(cudaStreamSynchronize(c->stream));
+    return SM_OK;
+}
+
 // ---- whole pairs, batched ----------------------------------------------------------------
 
-extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
-                            double threshold, void *web_out, int web_u8, int32_t *best_out)
+// The result formats of the batch entries: int32 web and best; u8 web (narrowed after the hot path) and int32 best;
+// 16-bit web and best, written by the hot path itself.
+enum WebFormat { WEB_I32, WEB_U8, WEB_U16 };
+
+static size_t web_bytes(WebFormat f) { return f == WEB_U8 ? 1 : (f == WEB_U16 ? 2 : 4); }
+static size_t best_bytes(WebFormat f) { return f == WEB_U16 ? 2 : 4; }
+
+// sm_run_batch / sm_run_batch16 (fn: the entry's name, for the messages)
+static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                     double threshold, WebFormat fmt, void *web_out, void *best_out)
 {
     SM_ENTER(c);
-    SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "sm_run_batch: bad arguments");
-    SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "sm_run_batch: whole-frame contexts only");
-    SM_REQUIRE(!web_u8 || c->D <= 255, "sm_run_batch: u8 web needs num_shifts <= 255");
-    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch: threshold must be between 0 and 1");
+    SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
+    SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "%s: whole-frame contexts only", fn);
+    SM_REQUIRE(fmt != WEB_U8 || c->D <= 255, "%s: u8 web needs num_shifts <= 255", fn);
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "%s: threshold must be between 0 and 1", fn);
     constexpr int NP = sm_ctx::NPIPE;
     sm_ctx::Pipe &P = c->pipe;
     const size_t n = c->npix();
@@ -1035,18 +1129,24 @@ extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const 
         if (!P.up) SM_CUDA(cudaStreamCreateWithFlags(&P.up, cudaStreamNonBlocking));
         if (!P.down) SM_CUDA(cudaStreamCreateWithFlags(&P.down, cudaStreamNonBlocking));
         for (int k = 0; k < NP; k++) {
-            if ((rc = dev_alloc(&P.img[k], 2 * P.group * n)) || (rc = dev_alloc(&P.web[k], P.group * n)) ||
-                (rc = dev_alloc(&P.best[k], P.group * n)))
-                return rc;
+            if ((rc = dev_alloc(&P.img[k], 2 * P.group * n))) return rc;
             if (!P.ev_up[k]) SM_CUDA(cudaEventCreateWithFlags(&P.ev_up[k], cudaEventDisableTiming));
             if (!P.ev_comp[k]) SM_CUDA(cudaEventCreateWithFlags(&P.ev_comp[k], cudaEventDisableTiming));
             if (!P.ev_down[k]) SM_CUDA(cudaEventCreateWithFlags(&P.ev_down[k], cudaEventDisableTiming));
         }
         P.ready = true;
     }
-    if (web_u8)
-        for (int k = 0; k < NP; k++)
-            if ((rc = dev_alloc(&P.web8[k], P.group * n))) return rc;
+    // the hot path's outputs: int32 web and best (narrowed to u8 after it, for WEB_U8), or 16-bit web and, only when
+    // the caller wants it, best
+    for (int k = 0; k < NP; k++) {
+        if (fmt == WEB_U16) {
+            if ((rc = dev_alloc(&P.web16[k], P.group * n)) || (best_out && (rc = dev_alloc(&P.best16[k], P.group * n))))
+                return rc;
+        } else if ((rc = dev_alloc(&P.web[k], P.group * n)) || (rc = dev_alloc(&P.best[k], P.group * n))) {
+            return rc;
+        }
+        if (fmt == WEB_U8 && (rc = dev_alloc(&P.web8[k], P.group * n))) return rc;
+    }
     const bool use_lut = !c->edges_fp64_only;
     if (!use_lut)  // byte edge maps exist only on the FP64 cross-check path
         for (int k = 0; k < NP; k++)
@@ -1070,9 +1170,11 @@ extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const 
         SM_CUDA(cudaEventRecord(P.ev_up[b], P.up));
         // ---- stage 2, the context's stream: edges of all 2*np images, then the batched hot path
         SM_CUDA(cudaStreamWaitEvent(c->stream, P.ev_up[b], 0));
+        const Outputs out = fmt == WEB_U16 ? Outputs{nullptr, nullptr, best_out ? P.best16[b] : nullptr, P.web16[b]}
+                                           : Outputs{P.best[b], P.web[b]};
         if (use_lut) {
             // edges of all 2*np images straight into the packed planes, then the hot path: two kernels per group
-            if ((rc = batch_core(c, np, true, threshold, P.img[b], P.img[b] + (size_t)G * n, n, P.best[b], P.web[b], n)))
+            if ((rc = batch_core(c, np, true, threshold, P.img[b], P.img[b] + (size_t)G * n, n, out, n)))
                 return rc;
         } else {
             for (int j = 0; j < 2 * G; j++) {
@@ -1082,25 +1184,25 @@ extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const 
                 if (rc < 0) return rc;
                 launches += rc;
             }
-            if ((rc = batch_core(c, np, false, 0.0, P.edg[b], P.edg[b] + (size_t)G * n, n, P.best[b], P.web[b], n)))
+            if ((rc = batch_core(c, np, false, 0.0, P.edg[b], P.edg[b] + (size_t)G * n, n, out, n)))
                 return rc;
         }
         launches += c->last_launches;
-        if (web_u8) {
-            if ((rc = launch_i32_to_u8(P.web[b], P.web8[b], (size_t)np * n, c->stream)) < 0) return rc;
+        if (fmt == WEB_U8) {
+            if ((rc = launch_narrow(P.web[b], P.web8[b], (size_t)np * n, c->stream)) < 0) return rc;
             launches += rc;
         }
         SM_CUDA(cudaEventRecord(P.ev_comp[b], c->stream));
-        // ---- stage 3, download stream
+        // ---- stage 3, download stream: one copy per array
         SM_CUDA(cudaStreamWaitEvent(P.down, P.ev_comp[b], 0));
-        if (web_u8)
-            SM_CUDA(cudaMemcpyAsync((uint8_t *)web_out + (size_t)k * n, P.web8[b], (size_t)np * n,
-                                    cudaMemcpyDeviceToHost, P.down));
-        else
-            SM_CUDA(cudaMemcpyAsync((int32_t *)web_out + (size_t)k * n, P.web[b], (size_t)np * n * sizeof(int32_t),
-                                    cudaMemcpyDeviceToHost, P.down));
+        const void *web_dev = fmt == WEB_U8 ? (const void *)P.web8[b]
+                                            : (fmt == WEB_U16 ? (const void *)P.web16[b] : (const void *)P.web[b]);
+        const void *best_dev = fmt == WEB_U16 ? (const void *)P.best16[b] : (const void *)P.best[b];
+        const size_t wb = web_bytes(fmt), bb = best_bytes(fmt);
+        SM_CUDA(cudaMemcpyAsync((uint8_t *)web_out + (size_t)k * n * wb, web_dev, (size_t)np * n * wb,
+                                cudaMemcpyDeviceToHost, P.down));
         if (best_out)
-            SM_CUDA(cudaMemcpyAsync(best_out + (size_t)k * n, P.best[b], (size_t)np * n * sizeof(int32_t),
+            SM_CUDA(cudaMemcpyAsync((uint8_t *)best_out + (size_t)k * n * bb, best_dev, (size_t)np * n * bb,
                                     cudaMemcpyDeviceToHost, P.down));
         SM_CUDA(cudaEventRecord(P.ev_down[b], P.down));
     }
@@ -1109,6 +1211,21 @@ extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const 
     SM_CUDA(cudaStreamSynchronize(P.down));
     c->last_launches = launches;
     return SM_OK;
+}
+
+extern "C" int sm_run_batch(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                            double threshold, void *web_out, int web_u8, int32_t *best_out)
+{
+    return run_batch(__func__, c, n_pairs, first, second, threshold, web_u8 ? WEB_U8 : WEB_I32, web_out, best_out);
+}
+
+extern "C" int sm_run_batch16(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                              double threshold, uint16_t *web_out, uint16_t *best_out)
+{
+    // the checks that need no context first (and no device)
+    SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "sm_run_batch16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch16: threshold must be between 0 and 1");
+    return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out);
 }
 
 // ---- whole pairs over several GPUs of one box ------------------------------------------------
@@ -1242,21 +1359,22 @@ extern "C" int sm_multi_destroy(sm_multi *m)
 
 extern "C" int sm_multi_device_count(const sm_multi *m) { return m ? m->n : SM_ERR_ARG; }
 
-extern "C" int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
-                                  double threshold, void *web_out, int web_u8, int32_t *best_out)
+// sm_multi_run_batch / sm_multi_run_batch16
+static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                           double threshold, WebFormat fmt, void *web_out, void *best_out)
 {
-    SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out, "sm_multi_run_batch: bad arguments");
+    SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     const int N = m->n;
     std::vector<int> rcs((size_t)N, SM_OK);
     std::vector<std::string> errs((size_t)N);
-    const size_t n = m->ctx[0]->npix();
+    const size_t n = m->ctx[0]->npix(), wb = web_bytes(fmt), bb = best_bytes(fmt);
     auto work = [&](int d) {
         const int k0 = (int)((long long)n_pairs * d / N), k1 = (int)((long long)n_pairs * (d + 1) / N);
         if (k1 <= k0) return;
-        uint8_t *w8 = (uint8_t *)web_out;
-        void *wout = web_u8 ? (void *)(w8 + (size_t)k0 * n) : (void *)((int32_t *)web_out + (size_t)k0 * n);
-        rcs[(size_t)d] = sm_run_batch(m->ctx[d], k1 - k0, first + (size_t)k0 * n, second + (size_t)k0 * n, threshold, wout,
-                                      web_u8, best_out ? best_out + (size_t)k0 * n : nullptr);
+        void *wout = (uint8_t *)web_out + (size_t)k0 * n * wb;
+        void *bout = best_out ? (void *)((uint8_t *)best_out + (size_t)k0 * n * bb) : nullptr;
+        rcs[(size_t)d] = run_batch(fn, m->ctx[d], k1 - k0, first + (size_t)k0 * n, second + (size_t)k0 * n, threshold, fmt,
+                                   wout, bout);
         if (rcs[(size_t)d]) errs[(size_t)d] = sm_last_error();  // the message is per thread: carry it to the caller's
     };
     if (m->workers)
@@ -1265,10 +1383,22 @@ extern "C" int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first
         for (int d = 0; d < N; d++) work(d);
     for (int d = 0; d < N; d++)
         if (rcs[d]) {
-            set_error("sm_multi_run_batch: device slot %d: %s", d, errs[d].c_str());
+            set_error("%s: device slot %d: %s", fn, d, errs[d].c_str());
             return rcs[d];
         }
     return SM_OK;
+}
+
+extern "C" int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                  double threshold, void *web_out, int web_u8, int32_t *best_out)
+{
+    return multi_run_batch(__func__, m, n_pairs, first, second, threshold, web_u8 ? WEB_U8 : WEB_I32, web_out, best_out);
+}
+
+extern "C" int sm_multi_run_batch16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                    double threshold, uint16_t *web_out, uint16_t *best_out)
+{
+    return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out);
 }
 
 // ---- one pair, row bands over several GPUs of one box ----------------------------------------------
@@ -1326,10 +1456,27 @@ extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices
     return SM_OK;
 }
 
-extern "C" int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
-                            int32_t *web_out, int32_t *best_out)
+// One band context's 16-bit run: the hot path writes rows [row0, row1) of the context's frame-sized u16 arrays
+// (best16 when the caller wants best or the kernel stores it anyway); only those rows are downloaded.
+static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out)
 {
-    SM_REQUIRE(b && first && second && web_out, "sm_bands_run: bad arguments");
+    SM_ENTER(c);
+    int rc;
+    const bool with_best = best_out || stores_best(c);
+    if ((rc = dev_alloc(&c->web16, c->npix())) || (with_best && (rc = dev_alloc(&c->best16, c->npix())))) return rc;
+    if ((rc = run_hot(c, c->edges[0], c->edges[1], {nullptr, nullptr, with_best ? c->best16 : nullptr, c->web16})))
+        return rc;
+    if ((rc = copy_band_d2h(c, web_out, c->web16)) || (best_out && (rc = copy_band_d2h(c, best_out, c->best16))))
+        return rc;
+    SM_CUDA(cudaStreamSynchronize(c->stream));
+    return SM_OK;
+}
+
+// sm_bands_run / sm_bands_run16
+static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                     WebFormat fmt, void *web_out, void *best_out)
+{
+    SM_REQUIRE(b && first && second && web_out, "%s: bad arguments", fn);
     const int N = b->n;
     std::vector<int> rcs((size_t)N, SM_OK);
     std::vector<std::string> errs((size_t)N);
@@ -1337,9 +1484,13 @@ extern "C" int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *se
         sm_ctx *c = b->ctx[d];
         int rc = sm_upload_u8(c, first, second);  // a band context copies only the rows it needs
         if (!rc) rc = sm_edges(c, threshold);
-        if (!rc) rc = sm_match_wta(c);
-        if (!rc) rc = sm_download(c, SM_WEB, 0, web_out);  // ... and writes only its own rows
-        if (!rc && best_out) rc = sm_download(c, SM_BEST, 0, best_out);
+        if (fmt == WEB_U16) {
+            if (!rc) rc = band_run16(c, (uint16_t *)web_out, (uint16_t *)best_out);
+        } else {
+            if (!rc) rc = sm_match_wta(c);
+            if (!rc) rc = sm_download(c, SM_WEB, 0, web_out);  // ... and writes only its own rows
+            if (!rc && best_out) rc = sm_download(c, SM_BEST, 0, best_out);
+        }
         rcs[(size_t)d] = rc;
         if (rc) errs[(size_t)d] = sm_last_error();
     };
@@ -1349,8 +1500,20 @@ extern "C" int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *se
         for (int d = 0; d < N; d++) work(d);
     for (int d = 0; d < N; d++)
         if (rcs[d]) {
-            set_error("sm_bands_run: band %d: %s", d, errs[d].c_str());
+            set_error("%s: band %d: %s", fn, d, errs[d].c_str());
             return rcs[d];
         }
     return SM_OK;
+}
+
+extern "C" int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                            int32_t *web_out, int32_t *best_out)
+{
+    return bands_run(__func__, b, first, second, threshold, WEB_I32, web_out, best_out);
+}
+
+extern "C" int sm_bands_run16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                              uint16_t *web_out, uint16_t *best_out)
+{
+    return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out);
 }
