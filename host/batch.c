@@ -6,9 +6,11 @@
  * reference has no batch program; this one exists to exercise the multi-GPU entry of the C ABI
  * (sm_multi_*, include/stereo_b200.h) without Python.
  *
- *   stereobatch WIDTH HEIGHT NUM_SHIFTS SQUARE_WIDTH N_PAIRS [wrap|ghost] [u8|u16|i32] [n_gpus]
+ *   stereobatch WIDTH HEIGHT NUM_SHIFTS SQUARE_WIDTH N_PAIRS [wrap|ghost] [u8|u16|i32] [n_gpus] [min_shift]
  *
- * Input: the synthetic textured pairs of SURVEY 8(d) (seed 1234 + 2k for pair k), threshold 0.15.
+ * Input: the synthetic textured pairs of SURVEY 8(d) (seed 1234 + 2k for pair k), threshold 0.15.  With min_shift
+ * (m) the contexts search the shifts [m, m + NUM_SHIFTS) (sm_multi_create_range) and the pairs carry the disparities
+ * m + (hd mod NUM_SHIFTS) instead of hd mod NUM_SHIFTS; without it the run is the reference's range [0, NUM_SHIFTS).
  * Output line (stdout):
  *   gpus = G, pairs = N, elapsed = S, pairs_per_s = P, mde_per_s = M, web_crc32 = XXXXXXXX
  * `elapsed` covers H2D, edges, hot path and D2H of all pairs (second of two runs); the CRC is zlib's
@@ -49,14 +51,14 @@ static uint8_t left_at(uint64_t seed, int x, int y)
     return ((hk >> 8) & 7) == 0 ? (uint8_t)(hk & 0xFF) : 128;
 }
 
-static void synth_pair(uint64_t seed, int w, int h, int d, uint8_t *left, uint8_t *right)
+static void synth_pair(uint64_t seed, int w, int h, int m, int d, uint8_t *left, uint8_t *right)
 {
     const uint64_t K = 0xD6E8FEB86659FD93ull;
     const int tw = 4 * d > 240 ? 4 * d : 240, th = 120;
     for (int y = 0; y < h; y++)
         for (int x = 0; x < w; x++) {
             uint64_t hd = splitmix64((seed + 1) * K + (uint64_t)(y / th) * 4096 + (uint64_t)(x / tw));
-            int disp = (int)(hd % (uint64_t)d);
+            int disp = m + (int)(hd % (uint64_t)d);
             int xs = ((x - disp) % w + w) % w;
             left[(size_t)y * w + x] = left_at(seed, x, y);
             right[(size_t)y * w + x] = left_at(seed, xs, y);
@@ -73,7 +75,8 @@ static double now(void)
 int main(int argc, char **argv)
 {
     if (argc < 6) {
-        fprintf(stderr, "usage: %s width height num_shifts square_width n_pairs [wrap|ghost] [u8|u16|i32] [n_gpus]\n",
+        fprintf(stderr,
+                "usage: %s width height num_shifts square_width n_pairs [wrap|ghost] [u8|u16|i32] [n_gpus] [min_shift]\n",
                 argv[0]);
         return 1;
     }
@@ -87,8 +90,9 @@ int main(int argc, char **argv)
         return 1;
     }
     if (argc > 8 && atoi(argv[8]) >= 1 && atoi(argv[8]) < ngpu) ngpu = atoi(argv[8]);
-    if (w < 1 || h < 1 || d < 1 || sw < 1 || n < 1) {
-        fprintf(stderr, "error: arguments must be positive\n");
+    const int ms = argc > 9 ? atoi(argv[9]) : 0;
+    if (w < 1 || h < 1 || d < 1 || sw < 1 || n < 1 || ms < 0) {
+        fprintf(stderr, "error: arguments must be positive (min_shift non-negative)\n");
         return 1;
     }
     const size_t npix = (size_t)w * h;
@@ -97,12 +101,15 @@ int main(int argc, char **argv)
     CHECK(sm_host_alloc((void **)&first, npix * n));
     CHECK(sm_host_alloc((void **)&second, npix * n));
     CHECK(sm_host_alloc(&web, npix * n * elem));
-    for (int k = 0; k < n; k++) synth_pair(1234 + 2 * (uint64_t)k, w, h, d, first + npix * k, second + npix * k);
+    for (int k = 0; k < n; k++) synth_pair(1234 + 2 * (uint64_t)k, w, h, ms, d, first + npix * k, second + npix * k);
 
     int devices[64];
     for (int g = 0; g < ngpu && g < 64; g++) devices[g] = g;
     sm_multi *m;
-    CHECK(sm_multi_create(&m, devices, ngpu, w, h, d, sw, variant));
+    if (argc > 9)
+        CHECK(sm_multi_create_range(&m, devices, ngpu, w, h, ms, d, sw, variant));
+    else
+        CHECK(sm_multi_create(&m, devices, ngpu, w, h, d, sw, variant));
     double t1 = 0.0;
     for (int run = 0; run < 2; run++) { /* first run: buffers, kernels */
         t1 = now();

@@ -116,8 +116,9 @@ typedef enum sm_shape {
 /* Message of the last failure on this thread ("" if none). */
 const char *sm_last_error(void);
 /* ABI version: (major << 16) | minor.  The 16-bit result entries (sm_match_wta_dev_batch16, sm_run_batch16,
- * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16) are additions to 1.3 that leave every other entry as it
- * was; clients detect them by symbol. */
+ * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16) and the search-range creators (sm_create_range,
+ * sm_create_band_range, sm_multi_create_range, sm_bands_create_range) are additions to 1.3 that leave every other
+ * entry as it was; clients detect them by symbol. */
 int sm_version(void);
 /* Number of CUDA devices visible, or a negative sm_status. */
 int sm_device_count(void);
@@ -145,6 +146,22 @@ int sm_create(sm_ctx **ctx, int device, int width, int height, int num_shifts,
  * by sm_download*.  sm_create(...) == sm_create_band(..., 0, height). */
 int sm_create_band(sm_ctx **ctx, int device, int width, int frame_height, int row0, int row1,
                    int num_shifts, int square_width, int variant);
+
+/* Contexts that search the shifts [min_shift, min_shift + num_shifts) instead of [0, num_shifts): the disparity range
+ * of a rig whose scene lies at min_shift or more (OpenCV's minDisparity + numDisparities).  match_s(x, y) compares the
+ * first image at x with the second at x + s (WRAP: mod width, whatever the multiple; GHOST: 0 where x + s >= width);
+ * box sums and the centre mask are unchanged; best = max(0, max_s score_s) and web = 1 + the highest s whose score
+ * equals best, so a pixel whose scores are all zero gets web = min_shift + num_shifts, and web >= 1 + min_shift
+ * everywhere (sm_fill_web_holes stays the identity).  The debug planes of sm_download take the real shift s, which must
+ * lie in the range; SM_EDGES1/2 stay the whole, unshifted edge maps.  Limits: min_shift >= 0 and
+ * min_shift + num_shifts <= 65535 (the 16-bit web stays exact); the u8 web (sm_download_web_u8, web_u8 of the batch
+ * entries) needs min_shift + num_shifts <= 255.  The work is that of num_shifts shifts at any min_shift.  min_shift == 0 is the
+ * reference's range: sm_create(...) == sm_create_range(..., 0, num_shifts, ...), and likewise for the band, multi and
+ * bands creators.  All argument checks come before any device call. */
+int sm_create_range(sm_ctx **ctx, int device, int width, int height, int min_shift, int num_shifts,
+                    int square_width, int variant);
+int sm_create_band_range(sm_ctx **ctx, int device, int width, int frame_height, int row0, int row1, int min_shift,
+                         int num_shifts, int square_width, int variant);
 
 /* Replaces the cudaFree block at the end of algorithm() (stereo.cu:339-346). */
 int sm_destroy(sm_ctx *ctx);
@@ -251,7 +268,7 @@ int sm_draw_contour_map(sm_ctx *ctx, int lines, int32_t *web_min, int32_t *web_m
  * SM_MATCH / SM_SCORE_ALL / SM_SCORE planes are computed on demand for `shift`. */
 int sm_download(sm_ctx *ctx, int which, int shift, void *host);
 
-/* web as u8 (valid when num_shifts <= 255): a quarter of the D2H bytes. */
+/* web as u8 (valid when min_shift + num_shifts <= 255): a quarter of the D2H bytes. */
 int sm_download_web_u8(sm_ctx *ctx, uint8_t *host);
 /* web as u16 (any num_shifts): half the D2H bytes. */
 int sm_download_web_u16(sm_ctx *ctx, uint16_t *host);
@@ -279,6 +296,9 @@ int sm_run_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t
 typedef struct sm_multi sm_multi;
 int sm_multi_create(sm_multi **out, const int *devices, int n_devices, int width, int height,
                     int num_shifts, int square_width, int variant);
+/* The same with the search range [min_shift, min_shift + num_shifts) (see sm_create_range). */
+int sm_multi_create_range(sm_multi **out, const int *devices, int n_devices, int width, int height, int min_shift,
+                          int num_shifts, int square_width, int variant);
 int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
                        double threshold, void *web_out, int web_u8, int32_t *best_out);
 /* The same through sm_run_batch16 (best_out may be NULL). */
@@ -294,6 +314,9 @@ int sm_multi_destroy(sm_multi *m);
 typedef struct sm_bands sm_bands;
 int sm_bands_create(sm_bands **out, const int *devices, int n_devices, int width, int height,
                     int num_shifts, int square_width, int variant);
+/* The same with the search range [min_shift, min_shift + num_shifts) (see sm_create_range). */
+int sm_bands_create_range(sm_bands **out, const int *devices, int n_devices, int width, int height, int min_shift,
+                          int num_shifts, int square_width, int variant);
 int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                  int32_t *web_out, int32_t *best_out);
 /* The same with 16-bit web / best (best_out may be NULL): each band's hot kernel writes its rows as u16 and only

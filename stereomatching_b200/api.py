@@ -40,6 +40,7 @@ SYMBOLS = [
     "sm_download_web_u16", "sm_run_batch", "sm_run_batch16", "sm_band_rows",
     "sm_multi_create", "sm_multi_run_batch", "sm_multi_run_batch16", "sm_multi_device_count", "sm_multi_destroy",
     "sm_bands_create", "sm_bands_run", "sm_bands_run16", "sm_bands_destroy",
+    "sm_create_range", "sm_create_band_range", "sm_multi_create_range", "sm_bands_create_range",
 ]
 
 
@@ -65,6 +66,8 @@ def lib() -> C.CDLL:
         L.sm_host_free.argtypes = [vp]
         L.sm_create.argtypes = [C.POINTER(vp), i, i, i, i, i, i]
         L.sm_create_band.argtypes = [C.POINTER(vp), i, i, i, i, i, i, i, i]
+        L.sm_create_range.argtypes = [C.POINTER(vp), i, i, i, i, i, i, i]
+        L.sm_create_band_range.argtypes = [C.POINTER(vp), i, i, i, i, i, i, i, i, i]
         L.sm_destroy.argtypes = [vp]
         L.sm_set_stream.argtypes = [vp, vp]
         L.sm_set_kernel.argtypes = [vp, i]
@@ -93,11 +96,13 @@ def lib() -> C.CDLL:
         L.sm_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_band_rows.argtypes = [i, i, i, C.POINTER(i), C.POINTER(i)]
         L.sm_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
+        L.sm_multi_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
         L.sm_multi_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
         L.sm_multi_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_multi_device_count.argtypes = [vp]
         L.sm_multi_destroy.argtypes = [vp]
         L.sm_bands_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
+        L.sm_bands_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
         L.sm_bands_run.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_run16.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_destroy.argtypes = [vp]
@@ -149,15 +154,18 @@ class StereoContext:
 
     Mirrors the reference's algorithm() (src/stereo.cu:296-347): upload -> edges ->
     match_wta -> fill_web_holes -> draw_contour_map, every stage downloadable.
+    ``min_shift``: search the shifts [min_shift, min_shift + num_shifts) (sm_create_band_range); 0 is the
+    reference's range.
     """
 
     def __init__(self, width, height, num_shifts=30, square_width=21, variant=WRAP, device=0,
-                 rows=None, kernel=KERNEL_AUTO):
+                 rows=None, kernel=KERNEL_AUTO, min_shift=0):
         self.W, self.H, self.D, self.sw, self.variant = width, height, num_shifts, square_width, variant
+        self.min_shift = min_shift
         self.row0, self.row1 = rows if rows is not None else (0, height)
         self._c = C.c_void_p()
-        _check(lib().sm_create_band(C.byref(self._c), device, width, height, self.row0, self.row1,
-                                    num_shifts, square_width, variant))
+        _check(lib().sm_create_band_range(C.byref(self._c), device, width, height, self.row0, self.row1,
+                                          min_shift, num_shifts, square_width, variant))
         if kernel != KERNEL_AUTO:
             self.set_kernel(kernel)
 
@@ -327,14 +335,15 @@ def _run_batch(handle, run, run16, first, second, threshold, web_u8, want_best, 
 
 class MultiGpuBatch:
     """sm_multi_*: whole pairs sharded over several GPUs of one box from ONE process (one context and one host
-    thread per entry of `devices`); the C counterpart of launching one rank per GPU."""
+    thread per entry of `devices`); the C counterpart of launching one rank per GPU.  ``min_shift``: as for
+    StereoContext."""
 
-    def __init__(self, devices, width, height, num_shifts, square_width, variant=WRAP):
+    def __init__(self, devices, width, height, num_shifts, square_width, variant=WRAP, min_shift=0):
         self.W, self.H = width, height
         self._m = C.c_void_p()
         arr = (C.c_int * len(devices))(*devices)
-        _check(lib().sm_multi_create(C.byref(self._m), arr, len(devices), width, height, num_shifts, square_width,
-                                     variant))
+        _check(lib().sm_multi_create_range(C.byref(self._m), arr, len(devices), width, height, min_shift, num_shifts,
+                                           square_width, variant))
 
     def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False):
         first = np.ascontiguousarray(first, np.uint8)
@@ -357,14 +366,15 @@ class MultiGpuBatch:
 
 
 class MultiGpuBands:
-    """sm_bands_*: ONE pair split into row bands (with replicated halo rows) over several GPUs from one process."""
+    """sm_bands_*: ONE pair split into row bands (with replicated halo rows) over several GPUs from one process.
+    ``min_shift``: as for StereoContext."""
 
-    def __init__(self, devices, width, height, num_shifts, square_width, variant=WRAP):
+    def __init__(self, devices, width, height, num_shifts, square_width, variant=WRAP, min_shift=0):
         self.W, self.H = width, height
         self._b = C.c_void_p()
         arr = (C.c_int * len(devices))(*devices)
-        _check(lib().sm_bands_create(C.byref(self._b), arr, len(devices), width, height, num_shifts, square_width,
-                                     variant))
+        _check(lib().sm_bands_create_range(C.byref(self._b), arr, len(devices), width, height, min_shift, num_shifts,
+                                           square_width, variant))
 
     def run(self, first, second, threshold=0.15, want_best=False, web16=False):
         """web [and best] of one pair: int32, or uint16 with web16."""

@@ -722,15 +722,15 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                         for (int p = 0; p < PV; p++) V1[k * NW + w][0][p] = Vs[k][w][p];
                     }
                 const uint32_t vl1[1] = {valid_lo}, vh1[1] = {valid_hi};
-                // the upper half's lanes are 16..31 of the word: web = lane - 16 + 1
+                // the upper half's lanes are 16..31 of the word: web = M + lane - 16 + 1
                 int bl[NCH], wl[NCH], bh[NCH], wh[NCH];
-                wta<NCH, 1, PV, !MULTI>(V1, M1, vl1, one, 1, bl, wl);
-                wta<NCH, 1, PV, !MULTI>(V1, M1, vh1, one, 1 - 16, bh, wh);
+                wta<NCH, 1, PV, !MULTI>(V1, M1, vl1, one, a.h.M + 1, bl, wl);
+                wta<NCH, 1, PV, !MULTI>(V1, M1, vh1, one, a.h.M + 1 - 16, bh, wh);
 #pragma unroll
                 for (int k = 0; k < G_; k++) put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW);
             } else if constexpr (!C2) {
                 int best[G_], web[G_];
-                wta<G_, NW, PV, !MULTI>(Vs, Ms, valid, one, 32 * wg0 + 1, best, web);
+                wta<G_, NW, PV, !MULTI>(Vs, Ms, valid, one, a.h.M + 32 * wg0 + 1, best, web);
 #pragma unroll
                 for (int k = 0; k < G_; k++) put(best[k], web[k], prev[k]);
             } else {
@@ -745,7 +745,7 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                     }
                 const uint32_t valid1[1] = {valid[0]};
                 int best[2 * G_], web[2 * G_];
-                wta<2 * G_, 1, PV, !MULTI>(V1, M1, valid1, one, 1, best, web);
+                wta<2 * G_, 1, PV, !MULTI>(V1, M1, valid1, one, a.h.M + 1, best, web);
 #pragma unroll
                 for (int k = 0; k < G_; k++) put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1]);
             }

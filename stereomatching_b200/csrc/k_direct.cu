@@ -60,7 +60,7 @@ __device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *w
     }
     size_t p = (size_t)(a.row0 + j) * a.g.W + x;
     if (sizeof(T) == 4 || best_out) best_out[p] = (T)best;  // (the int32 kernel always has a best)
-    web_out[p] = (T)web;
+    web_out[p] = (T)(a.M + web);  // shift i of the planes is M + i
 }
 
 __global__ void __launch_bounds__(256) k_direct(HotArgs a)

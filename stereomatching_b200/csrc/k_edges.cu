@@ -218,10 +218,13 @@ struct RowWords {
 // The thread's own word and the words left and right of it, at byte columns xl, x4, xr of the row.  Where the words
 // beside come from is decided once per thread: the neighbouring word, or at the frame's border the row's last / first
 // word (WRAP: the torus) or any in-bounds word (GHOST: the pixel next to the border is decided without it).
-__device__ __forceinline__ RowWords load_row(const uint8_t *__restrict__ row, int xl, int x4, int xr)
+// sh = 8 * (first pixel - x4): a thread whose four pixels start 1..3 bytes into its word (the second image of a range
+// whose minimum shift is no multiple of 4) takes its 3 x 6 bytes from the same three words, funnel-shifted.
+__device__ __forceinline__ RowWords load_row(const uint8_t *__restrict__ row, int xl, int x4, int xr, int sh)
 {
-    return RowWords{__ldg(reinterpret_cast<const uint32_t *>(row + xl)), __ldg(reinterpret_cast<const uint32_t *>(row + x4)),
-                    __ldg(reinterpret_cast<const uint32_t *>(row + xr))};
+    const uint32_t a = __ldg(reinterpret_cast<const uint32_t *>(row + xl)), b = __ldg(reinterpret_cast<const uint32_t *>(row + x4)),
+                   c = __ldg(reinterpret_cast<const uint32_t *>(row + xr));
+    return RowWords{__funnelshift_r(a, b, sh), __funnelshift_r(b, c, sh), c >> sh};
 }
 
 __device__ __forceinline__ void unpack_row(const RowWords &r, int (&p)[6])
@@ -289,7 +292,7 @@ __device__ __noinline__ void edge_gather_ghost(const uint8_t *__restrict__ img, 
 template <int VARIANT, bool WRITE_U8, bool GENERIC>
 __global__ void __launch_bounds__(128, EP_BLOCKS_PER_SM)
 k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img2, int FH, int row0, PackedGeom g,
-               double thr, const uint32_t *__restrict__ lut, uint32_t *__restrict__ LA, uint32_t *__restrict__ LB,
+               int M, double thr, const uint32_t *__restrict__ lut, uint32_t *__restrict__ LA, uint32_t *__restrict__ LB,
                uint32_t *__restrict__ RB, uint8_t *__restrict__ edges1, uint8_t *__restrict__ edges2, size_t image_stride,
                size_t plane_stride)
 {
@@ -306,29 +309,41 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
     __syncthreads();
     const int pair = blockIdx.z >> 1, side = blockIdx.z & 1;
     const uint8_t *img = (side ? img2 : img1) + (size_t)pair * image_stride;
-    uint8_t *edges = WRITE_U8 ? (side ? edges2 : edges1) + (size_t)pair * image_stride : nullptr;
+    // (the second image's byte map when its planes are offset: the host writes it, launch_edges_planes)
+    uint8_t *edges = WRITE_U8 && (side == 0 || M == 0) ? (side ? edges2 : edges1) + (size_t)pair * image_stride : nullptr;
     const int W = g.W;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;  // thread <-> 4 pixels; 8 threads <-> one word
     const int wd = t >> 3;
     const int lane = threadIdx.x & 31;
     const int x4 = t * 4 - PADL;
+    // the thread's first pixel: the second image's planes start M columns further (the search range [M, M + D))
+    const int xc = side ? x4 + M : x4;
     const int pr0 = blockIdx.y * EP_ROWS, pr1 = min(g.ER, pr0 + EP_ROWS);
     // WRAP: a padding pixel IS the wrapped image pixel, so the thread works at its wrapped column xs (when the
     // width is a multiple of 4 its four pixels stay contiguous there).  Word path (widths that are a multiple of 4,
     // word-aligned images, frames of at least two rows): the thread's four pixels are inside the image; the words
     // beside them come through the torus (WRAP) and, GHOST, a pixel whose stencil touches the ghost area is an edge
     // without any arithmetic (below).  Everything else (GENERIC kernels only) is gathered byte by byte.
-    int xs = x4;
+    // An offset of the second image that is no multiple of 4 (M) puts the four pixels 1..3 bytes into the aligned
+    // word xs: the same three loads, funnel-shifted by fsh.  GHOST: such a thread at the frame's border has one to
+    // three of its pixels inside (vmask) and stays on the word path; its words outside the frame are replaced by an
+    // in-bounds one, whose bytes only reach pixels outside the frame or on its border.
+    int xw = xc;
     if (VARIANT == SM_WRAP) {
-        xs %= W;
-        if (xs < 0) xs += W;
+        xw %= W;
+        if (xw < 0) xw += W;
     }
-    const bool xfast = wd < g.WPR && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(img) & 3) == 0 && FH >= 2 && xs >= 0 &&
-                       xs + 4 <= W;
-    const int xl = xs >= 4 ? xs - 4 : (VARIANT == SM_WRAP ? W - 4 : xs);
-    const int xr = xs + 8 <= W ? xs + 4 : (VARIANT == SM_WRAP ? 0 : xs);
-    // GHOST: this thread's pixels at the frame's left / right border
-    const uint32_t xborder = VARIANT == SM_GHOST ? (xs == 0 ? 1u : 0u) | (xs + 4 == W ? 8u : 0u) : 0u;
+    const int fsh = 8 * (xw & 3), xs = xw - (xw & 3);
+    const bool xfast = wd < g.WPR && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(img) & 3) == 0 && FH >= 2 &&
+                       xw + 4 > 0 && xw < W;
+    const int xb = VARIANT == SM_WRAP ? xs : min(max(xs, 0), W - 4);
+    const int xl = xs >= 4 ? xs - 4 : (VARIANT == SM_WRAP ? W - 4 : xb);
+    const int xr = xs + 8 <= W ? xs + 4 : (VARIANT == SM_WRAP ? 0 : xb);
+    // GHOST: this thread's pixels inside the frame, and those at its left / right border
+    const uint32_t vmask = VARIANT == SM_GHOST ? (0xFu << min(4, max(0, -xw))) & (0xFu >> min(4, max(0, xw + 4 - W))) & 0xFu : 0xFu;
+    const uint32_t xborder = VARIANT == SM_GHOST ? ((xw <= 0 && xw > -4 ? 1u << -xw : 0u) |
+                                                    (xw + 4 >= W && xw < W ? 1u << (W - 1 - xw) : 0u))
+                                                 : 0u;
     auto frame_row = [&](int pr, bool &valid) {
         int y = row0 - g.half + pr;
         valid = true;
@@ -369,7 +384,7 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                 // GHOST, first or last row of the frame: every stencil touches the ghost area and fires (see the
                 // border rule below); nothing to load
                 have_y = -2;
-                e = v = 0xFu;
+                e = v = vmask;
             } else if (xfast && ym >= 0 && yp < FH) {
                 // consecutive padded rows are consecutive frame rows (mod FH): the window slides, one new row
                 // of three words per step, and that row was asked for during the previous step
@@ -377,14 +392,14 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                 if (ahead_y == yp) {
                     top = ahead;
                 } else {
-                    top = load_row(img + (size_t)yp * W, xl, xs, xr);
+                    top = load_row(img + (size_t)yp * W, xl, xb, xr, fsh);
                 }
                 if (have_y == ym) {
 #pragma unroll
                     for (int k = 0; k < 6; k++) p[0][k] = p[1][k], p[1][k] = p[2][k];
                 } else {
-                    unpack_row(load_row(img + (size_t)ym * W, xl, xs, xr), p[0]);
-                    unpack_row(load_row(img + (size_t)y * W, xl, xs, xr), p[1]);
+                    unpack_row(load_row(img + (size_t)ym * W, xl, xb, xr, fsh), p[0]);
+                    unpack_row(load_row(img + (size_t)y * W, xl, xb, xr, fsh), p[1]);
                 }
                 {
                     // the row below the next step's row (its `yp`), if that step slides on from this one
@@ -392,7 +407,7 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                     if (VARIANT == SM_WRAP) y2 = y2 >= FH ? y2 - FH : y2;
                     ahead_y = -2;
                     if (pr + 1 < pr1 && nvalid && yn == yp && y2 < FH) {
-                        ahead = load_row(img + (size_t)y2 * W, xl, xs, xr);
+                        ahead = load_row(img + (size_t)y2 * W, xl, xb, xr, fsh);
                         ahead_y = y2;
                     }
                 }
@@ -405,7 +420,7 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                 // (stereo-ghost.c: CLAMP, util.h:24-26).  It needs frames of at least 2 x 2: a one-pixel-wide or
                 // one-pixel-high frame has ghost cells on BOTH sides of a detector (those take the gather path).
                 e |= xborder;
-                v = 0xFu;
+                v = vmask;
             } else {
                 have_y = -2;
                 if (VARIANT == SM_WRAP && GENERIC) {
@@ -413,10 +428,7 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                     // wrap, all 18 loads independent (one memory round trip per row, not one per pixel)
                     int xk[6];
 #pragma unroll
-                    for (int k = 0; k < 6; k++) {
-                        int x = (x4 - 1 + k) % W;
-                        xk[k] = x < 0 ? x + W : x;
-                    }
+                    for (int k = 0; k < 6; k++) xk[k] = (xw - 1 + k + W) % W;  // (xw is in [0, W))
                     const int ys[3] = {ym, y, yp};
 #pragma unroll
                     for (int j = 0; j < 3; j++)
@@ -425,10 +437,10 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
                     e = thresholds_exact ? edge_nibble(p, edge_hi) : edge_nibble(p, edge_lut);
                     v = 0xFu;
                 } else if (VARIANT == SM_GHOST && GENERIC) {
-                    edge_gather_ghost(img, W, FH, x4, ym, y, yp, thr, lut, hi_s, thresholds_exact, e, v);
+                    edge_gather_ghost(img, W, FH, xc, ym, y, yp, thr, lut, hi_s, thresholds_exact, e, v);
                 }  // else: GHOST padding beside the frame, zero and invalid
             }
-            if (WRITE_U8) {
+            if (WRITE_U8 && edges) {
                 // the byte maps hold the frame itself: only the unwrapped in-image pixels of this word
                 if (x4 >= 0 && x4 + 4 <= W && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(edges) & 3) == 0) {
                     *reinterpret_cast<uint32_t *>(edges + (size_t)y * W + x4) =
@@ -442,8 +454,8 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
             have_y = -2;
         }
         // eight threads' nibbles -> one 32-pixel word (all 32 lanes take part)
-        const int sh = 4 * (lane & 7);
-        uint32_t ew = e << sh, vw = v << sh;
+        const int nsh = 4 * (lane & 7);
+        uint32_t ew = e << nsh, vw = v << nsh;
 #pragma unroll
         for (int m = 1; m <= 4; m <<= 1) {
             ew |= __shfl_xor_sync(0xFFFFFFFFu, ew, m);
@@ -464,7 +476,7 @@ k_edges_planes(const uint8_t *__restrict__ img1, const uint8_t *__restrict__ img
 }
 
 int launch_edges_planes(const uint8_t *img1, const uint8_t *img2, int FH, int row0, int variant, const PackedGeom &g,
-                        double threshold, const uint32_t *lut, uint32_t *LA, uint32_t *LB, uint32_t *RB, uint8_t *edges1,
+                        int M, double threshold, const uint32_t *lut, uint32_t *LA, uint32_t *LB, uint32_t *RB, uint8_t *edges1,
                         uint8_t *edges2, cudaStream_t s, int npairs, size_t image_stride, size_t plane_stride)
 {
     dim3 block(128);
@@ -474,7 +486,7 @@ int launch_edges_planes(const uint8_t *img1, const uint8_t *img2, int FH, int ro
     const bool regular = (g.W & 3) == 0 && FH >= 2 && ((reinterpret_cast<uintptr_t>(img1) | reinterpret_cast<uintptr_t>(img2)) & 3) == 0 &&
                          (npairs == 1 || (image_stride & 3) == 0);
 #define SM_EP(V, U, G) \
-    k_edges_planes<V, U, G><<<grid, block, 0, s>>>(img1, img2, FH, row0, g, threshold, lut, LA, LB, RB, edges1, edges2, \
+    k_edges_planes<V, U, G><<<grid, block, 0, s>>>(img1, img2, FH, row0, g, M, threshold, lut, LA, LB, RB, edges1, edges2, \
                                                    image_stride, plane_stride)
     if (variant == SM_WRAP && regular) {
         if (u8) SM_EP(SM_WRAP, true, false); else SM_EP(SM_WRAP, false, false);

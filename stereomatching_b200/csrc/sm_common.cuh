@@ -45,6 +45,10 @@ void set_error(const char *fmt, ...);
 //   columns: bit index PADL + x,  x in [-half, W + half + D)
 // WRAP fills the padding with the toroidally wrapped image (util.h:42-47), GHOST with
 // zeros.  After packing, the kernels are variant-agnostic.
+// A search range [M, M + D) that starts above zero (min_shift M) is absorbed by the
+// producers: bit PADL + x of RB holds the second image at column x + M (under the same
+// border policy), so RB[u+i] is shift M + i and the kernels only add M to the winning shift.
+//   match(u, i) = [first(u) == second(u + M + i)]
 constexpr int PADL = 32;  // left padding in bits (>= half, keeps x = 0 word aligned)
 
 struct PackedGeom {
@@ -85,6 +89,9 @@ struct HotArgs {
     int force_segs = 0;
     // resident warps per SM of the bit-sliced kernel this geometry uses (prepare_bitslice; 0 = ask)
     int blocks_per_sm = 0;
+    // min_shift: the planes hold shifts [M, M + D), the winner's web is M + 1 + its lane.  (Last, in the struct's
+    // tail padding: the offsets of the other fields, and with them the kernels' parameter loads, stay put.)
+    int M = 0;
 };
 
 // What a hot-path launch ran (SM_INFO_KERNEL_SHAPE, SM_INFO_ROW_RUNS): filled in by the launcher from the
@@ -96,7 +103,7 @@ struct LaunchRecord {
 
 // launchers (each returns the number of kernels launched, or a negative sm_status)
 int launch_pack(const uint8_t *e1, const uint8_t *e2, int FH, int row0, int variant,
-                const PackedGeom &g, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
+                const PackedGeom &g, int M, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
                 int npairs = 1, size_t edge_stride = 0, size_t plane_stride = 0);
 int launch_direct(const HotArgs &a, cudaStream_t s, bool out16 = false);  // out16: the 16-bit twin
 int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);
@@ -129,9 +136,10 @@ int launch_edges(const T *img, int W, int FH, int ystart, int nrows, int variant
 int launch_edge_lut(double threshold, uint32_t *lut, cudaStream_t s);
 size_t edge_lut_words();
 
-// both images of npairs pairs -> packed planes in one launch (edges1/edges2 non-NULL: the byte maps as well)
+// both images of npairs pairs -> packed planes in one launch (edges1/edges2 non-NULL: the byte maps as well; the
+// second image's only while M == 0).  M: min_shift, the second image's planes start M columns further
 int launch_edges_planes(const uint8_t *img1, const uint8_t *img2, int FH, int row0, int variant, const PackedGeom &g,
-                        double threshold, const uint32_t *lut, uint32_t *LA, uint32_t *LB, uint32_t *RB, uint8_t *edges1,
+                        int M, double threshold, const uint32_t *lut, uint32_t *LA, uint32_t *LB, uint32_t *RB, uint8_t *edges1,
                         uint8_t *edges2, cudaStream_t s, int npairs = 1, size_t image_stride = 0, size_t plane_stride = 0);
 
 int launch_fill_web_holes_step(const int32_t *src, int32_t *dst, int W, int H, cudaStream_t s);

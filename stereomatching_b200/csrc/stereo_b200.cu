@@ -38,6 +38,7 @@ struct sm_ctx {
     int W = 0, FH = 0;         // frame geometry
     int row0 = 0, row1 = 0;    // output rows owned by this context
     int D = 0, sw = 0, half = 0, variant = 0;
+    int M = 0;  // min_shift: the context searches shifts [M, M + D)
     int kernel = SM_KERNEL_AUTO;
     int num_sms = 148;
     PackedGeom g{};
@@ -241,6 +242,7 @@ HotArgs hot_args(sm_ctx *c, const Outputs &o)
     a.row0 = c->row0;
     a.force_segs = c->tuned_segs;
     a.blocks_per_sm = c->occ;
+    a.M = c->M;
     return a;
 }
 
@@ -290,7 +292,7 @@ int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, const Outputs &out)
     // sm_edges writes the packed planes itself (k_edges_planes): no pack launch then
     const bool packed = c->planes_valid && e1 == c->edges[0] && e2 == c->edges[1];
     if (!packed) {
-        rc = launch_pack(e1, e2, c->FH, c->row0, c->variant, c->g, c->LA, c->LB, c->RB, c->stream);
+        rc = launch_pack(e1, e2, c->FH, c->row0, c->variant, c->g, c->M, c->LA, c->LB, c->RB, c->stream);
         if (rc < 0) return rc;
         launches += rc;
     }
@@ -370,14 +372,17 @@ extern "C" int sm_band_rows(int height, int n_bands, int band, int *row0, int *r
 
 // ---- context -----------------------------------------------------------------------
 
-extern "C" int sm_create_band(sm_ctx **out, int device, int width, int frame_height, int row0,
-                              int row1, int num_shifts, int square_width, int variant)
+extern "C" int sm_create_band_range(sm_ctx **out, int device, int width, int frame_height, int row0, int row1,
+                                    int min_shift, int num_shifts, int square_width, int variant)
 {
     SM_REQUIRE(out, "sm_create: NULL ctx pointer");
     *out = nullptr;
     SM_REQUIRE(width > 0 && frame_height > 0, "sm_create: width/height must be positive");
     SM_REQUIRE((size_t)width * frame_height < ((size_t)1 << 31), "sm_create: frame too large");
     SM_REQUIRE(num_shifts >= 1 && num_shifts <= 512, "sm_create: num_shifts must be in [1, 512]");
+    // web = 1 + the winning shift <= min_shift + num_shifts must stay exact in 16 bits, and above step 3's hole (0)
+    SM_REQUIRE(min_shift >= 0 && min_shift <= 65535 - num_shifts,
+               "sm_create: min_shift must be >= 0 with min_shift + num_shifts <= 65535");
     // the reference takes any square_width up to the frame size (stereo.cu:395-398); its window is
     // half = square_width / 2 either side, so 0 (and -1) mean the 1x1 window.  Wider than 63 is not built here.
     SM_REQUIRE(square_width >= -1 && square_width <= 63, "sm_create: square_width must be in [0, 63]");
@@ -402,6 +407,7 @@ extern "C" int sm_create_band(sm_ctx **out, int device, int width, int frame_hei
     c->row0 = row0;
     c->row1 = row1;
     c->D = num_shifts;
+    c->M = min_shift;
     c->sw = square_width;
     c->half = square_width / 2;
     c->variant = variant;
@@ -467,10 +473,22 @@ extern "C" int sm_create_band(sm_ctx **out, int device, int width, int frame_hei
     return SM_OK;
 }
 
+extern "C" int sm_create_band(sm_ctx **ctx, int device, int width, int frame_height, int row0, int row1,
+                              int num_shifts, int square_width, int variant)
+{
+    return sm_create_band_range(ctx, device, width, frame_height, row0, row1, 0, num_shifts, square_width, variant);
+}
+
+extern "C" int sm_create_range(sm_ctx **ctx, int device, int width, int height, int min_shift, int num_shifts,
+                               int square_width, int variant)
+{
+    return sm_create_band_range(ctx, device, width, height, 0, height, min_shift, num_shifts, square_width, variant);
+}
+
 extern "C" int sm_create(sm_ctx **ctx, int device, int width, int height, int num_shifts,
                          int square_width, int variant)
 {
-    return sm_create_band(ctx, device, width, height, 0, height, num_shifts, square_width, variant);
+    return sm_create_band_range(ctx, device, width, height, 0, height, 0, num_shifts, square_width, variant);
 }
 
 extern "C" int sm_destroy(sm_ctx *c)
@@ -657,9 +675,16 @@ extern "C" int sm_edges(sm_ctx *c, double threshold)
     if (use_lut) {
         // both images in one launch, straight into the packed planes of the hot path; the byte maps are written
         // as well (sm_download(SM_EDGES*), debug planes)
-        int rc = launch_edges_planes(c->img_u8[0], c->img_u8[1], c->FH, c->row0, c->variant, c->g, threshold, c->edge_lut,
+        int rc = launch_edges_planes(c->img_u8[0], c->img_u8[1], c->FH, c->row0, c->variant, c->g, c->M, threshold, c->edge_lut,
                                      c->LA, c->LB, c->RB, c->edges[0], c->edges[1], c->stream);
         if (rc < 0) return rc;
+        // With a minimum shift the second image's planes start M columns into the frame, so their columns no longer
+        // cover the whole second map (columns [0, M - PADL) are in no plane word): that map comes from the byte-map
+        // detector, whose decisions are the table path's, bit for bit.
+        if (c->M != 0 &&
+            (rc = launch_edges<uint8_t>(c->img_u8[1], c->W, c->FH, ystart, nrows, c->variant, threshold, c->edges[1],
+                                        c->stream)) < 0)
+            return rc;
         c->planes_valid = true;
     } else {
         for (int k = 0; k < 2; k++) {
@@ -789,11 +814,11 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         if (group >= NPB) SM_CUDA(cudaStreamWaitEvent(c->pack_stream, c->ev_used[b], 0));  // set b is free again
         if (from_images)
             rc = launch_edges_planes(d_first_edges + (size_t)k * edge_stride, d_second_edges + (size_t)k * edge_stride,
-                                     c->FH, c->row0, c->variant, c->g, threshold, c->edge_lut, c->pLA[b], c->pLB[b],
+                                     c->FH, c->row0, c->variant, c->g, c->M, threshold, c->edge_lut, c->pLA[b], c->pLB[b],
                                      c->pRB[b], nullptr, nullptr, c->pack_stream, np, edge_stride, pw);
         else
             rc = launch_pack(d_first_edges + (size_t)k * edge_stride, d_second_edges + (size_t)k * edge_stride, c->FH,
-                             c->row0, c->variant, c->g, c->pLA[b], c->pLB[b], c->pRB[b], c->pack_stream, np,
+                             c->row0, c->variant, c->g, c->M, c->pLA[b], c->pLB[b], c->pRB[b], c->pack_stream, np,
                              edge_stride, pw);
         if (rc < 0) return rc;
         launches += rc;
@@ -1013,14 +1038,15 @@ extern "C" int sm_download(sm_ctx *c, int which, int shift, void *host)
     case SM_SCORE_ALL:
     case SM_SCORE: {
         if (!c->have_edges) goto state;
-        SM_REQUIRE(shift >= 0 && shift < c->D, "sm_download: shift %d out of [0, %d)", shift, c->D);
+        SM_REQUIRE(shift >= c->M && shift - c->M < c->D, "sm_download: shift %d out of [%d, %d)", shift, c->M,
+                   c->M + c->D);
         if ((rc = dev_alloc(&c->scratch_u8, c->npix())) || (rc = dev_alloc(&c->scratch_i32, c->npix())))
             return rc;
-        rc = launch_pack(c->edges[0], c->edges[1], c->FH, c->row0, c->variant, c->g, c->LA, c->LB, c->RB,
+        rc = launch_pack(c->edges[0], c->edges[1], c->FH, c->row0, c->variant, c->g, c->M, c->LA, c->LB, c->RB,
                          c->stream);
         if (rc < 0) return rc;
         HotArgs a = hot_args(c, Outputs{});
-        rc = launch_planes(a, shift, which == SM_MATCH ? c->scratch_u8 : nullptr,
+        rc = launch_planes(a, shift - c->M, which == SM_MATCH ? c->scratch_u8 : nullptr,
                            which == SM_SCORE_ALL ? c->scratch_i32 : nullptr,
                            which == SM_SCORE ? c->scratch_i32 : nullptr, c->stream);
         if (rc < 0) return rc;
@@ -1069,7 +1095,7 @@ extern "C" int sm_download_web_u8(sm_ctx *c, uint8_t *host)
 {
     SM_ENTER(c);
     SM_REQUIRE(host, "sm_download_web_u8: NULL host pointer");
-    SM_REQUIRE(c->D <= 255, "sm_download_web_u8: num_shifts %d does not fit 8 bits", c->D);
+    SM_REQUIRE(c->M + c->D <= 255, "sm_download_web_u8: min_shift + num_shifts = %d does not fit 8 bits", c->M + c->D);
     if (!c->have_web) {
         set_error("sm_download_web_u8: no web (call sm_match_wta first)");
         return SM_ERR_STATE;
@@ -1113,7 +1139,7 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
     SM_ENTER(c);
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "%s: whole-frame contexts only", fn);
-    SM_REQUIRE(fmt != WEB_U8 || c->D <= 255, "%s: u8 web needs num_shifts <= 255", fn);
+    SM_REQUIRE(fmt != WEB_U8 || c->M + c->D <= 255, "%s: u8 web needs min_shift + num_shifts <= 255", fn);
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "%s: threshold must be between 0 and 1", fn);
     constexpr int NP = sm_ctx::NPIPE;
     sm_ctx::Pipe &P = c->pipe;
@@ -1316,8 +1342,8 @@ struct sm_multi {
     SlotWorkers *workers = nullptr;
 };
 
-extern "C" int sm_multi_create(sm_multi **out, const int *devices, int n_devices, int width, int height,
-                               int num_shifts, int square_width, int variant)
+extern "C" int sm_multi_create_range(sm_multi **out, const int *devices, int n_devices, int width, int height,
+                                     int min_shift, int num_shifts, int square_width, int variant)
 {
     SM_REQUIRE(out && devices && n_devices >= 1 && n_devices <= 64, "sm_multi_create: bad arguments");
     *out = nullptr;
@@ -1334,7 +1360,7 @@ extern "C" int sm_multi_create(sm_multi **out, const int *devices, int n_devices
     }
     m->n = n_devices;
     for (int d = 0; d < n_devices; d++) {
-        int rc = sm_create(&m->ctx[d], devices[d], width, height, num_shifts, square_width, variant);
+        int rc = sm_create_range(&m->ctx[d], devices[d], width, height, min_shift, num_shifts, square_width, variant);
         if (rc) {
             for (int k = 0; k < d; k++) sm_destroy(m->ctx[k]);
             free(m->ctx);
@@ -1345,6 +1371,12 @@ extern "C" int sm_multi_create(sm_multi **out, const int *devices, int n_devices
     m->workers = new (std::nothrow) SlotWorkers(n_devices);
     *out = m;
     return SM_OK;
+}
+
+extern "C" int sm_multi_create(sm_multi **out, const int *devices, int n_devices, int width, int height,
+                               int num_shifts, int square_width, int variant)
+{
+    return sm_multi_create_range(out, devices, n_devices, width, height, 0, num_shifts, square_width, variant);
 }
 
 extern "C" int sm_multi_destroy(sm_multi *m)
@@ -1424,8 +1456,8 @@ extern "C" int sm_bands_destroy(sm_bands *b)
     return SM_OK;
 }
 
-extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices, int width, int height,
-                               int num_shifts, int square_width, int variant)
+extern "C" int sm_bands_create_range(sm_bands **out, const int *devices, int n_devices, int width, int height,
+                                     int min_shift, int num_shifts, int square_width, int variant)
 {
     SM_REQUIRE(out && devices && n_devices >= 1 && n_devices <= 64, "sm_bands_create: bad arguments");
     SM_REQUIRE(height >= n_devices, "sm_bands_create: fewer rows than bands");
@@ -1445,7 +1477,9 @@ extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices
     for (int d = 0; d < n_devices; d++) {
         int r0 = 0, r1 = 0;
         int rc = sm_band_rows(height, n_devices, d, &r0, &r1);
-        if (!rc) rc = sm_create_band(&b->ctx[d], devices[d], width, height, r0, r1, num_shifts, square_width, variant);
+        if (!rc)
+            rc = sm_create_band_range(&b->ctx[d], devices[d], width, height, r0, r1, min_shift, num_shifts, square_width,
+                                      variant);
         if (rc) {
             sm_bands_destroy(b);  // sm_destroy(NULL) is a no-op for the slots not created yet
             return rc;
@@ -1454,6 +1488,12 @@ extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices
     b->workers = new (std::nothrow) SlotWorkers(n_devices);
     *out = b;
     return SM_OK;
+}
+
+extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices, int width, int height,
+                               int num_shifts, int square_width, int variant)
+{
+    return sm_bands_create_range(out, devices, n_devices, width, height, 0, num_shifts, square_width, variant);
 }
 
 // One band context's 16-bit run: the hot path writes rows [row0, row1) of the context's frame-sized u16 arrays
