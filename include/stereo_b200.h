@@ -116,9 +116,10 @@ typedef enum sm_shape {
 /* Message of the last failure on this thread ("" if none). */
 const char *sm_last_error(void);
 /* ABI version: (major << 16) | minor.  The 16-bit result entries (sm_match_wta_dev_batch16, sm_run_batch16,
- * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16) and the search-range creators (sm_create_range,
- * sm_create_band_range, sm_multi_create_range, sm_bands_create_range) are additions to 1.3 that leave every other
- * entry as it was; clients detect them by symbol. */
+ * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16), the search-range creators (sm_create_range,
+ * sm_create_band_range, sm_multi_create_range, sm_bands_create_range) and the runner-up entries
+ * (sm_match_wta_dev_batch_ru16, sm_run_batch_ru16, sm_multi_run_batch_ru16, sm_bands_run_ru16) are additions to 1.3
+ * that leave every other entry as it was; clients detect them by symbol. */
 int sm_version(void);
 /* Number of CUDA devices visible, or a negative sm_status. */
 int sm_device_count(void);
@@ -228,6 +229,19 @@ int sm_match_wta_dev_batch(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edge
 int sm_match_wta_dev_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edges, const uint8_t *d_second_edges,
                              size_t edge_stride, uint16_t *d_best, uint16_t *d_web, size_t out_stride);
 
+/* The same, and each pixel's RUNNER-UP score, computed by the hot kernel's own winner-take-all: the second-largest
+ * value of the multiset of the pixel's masked scores over the context's shifts, i.e. the maximum over every shift
+ * but the one web names.  runner_up <= best everywhere; runner_up == best exactly where two or more shifts tie for
+ * best (pixels whose scores are all 0 included, for num_shifts >= 2); 0 with num_shifts == 1.  It does not depend
+ * on min_shift or on the tie rule, and web / best are those of sm_match_wta_dev_batch16.  The shifts next to the
+ * winner are NOT excluded: past 64 shifts the kernel merges 64-shift chunks in place, and (best, runner_up) of two
+ * chunks merge exactly while a runner-up outside an exclusion radius does not.  A uniqueness filter in the manner
+ * of OpenCV's uniquenessRatio u keeps best >= T && 100 * runner_up < (100 - u) * best.  d_runner_up (not NULL)
+ * takes pair k at k * out_stride, like d_web; 2 B per pixel. */
+int sm_match_wta_dev_batch_ru16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edges,
+                                const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best, uint16_t *d_web,
+                                uint16_t *d_runner_up, size_t out_stride);
+
 /* Device time of the last sm_match_wta* call on this context, CUDA events on the
  * context's stream (the reference brackets the whole algorithm() with
  * CLOCK_MONOTONIC instead, stereo.cu:308,334-335).  Waits for the call to finish. */
@@ -289,6 +303,10 @@ int sm_run_batch(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *
  * narrowing launch) and each comes back as one copy per group at 2 B per pixel.  best_out may be NULL. */
 int sm_run_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                    uint16_t *web_out, uint16_t *best_out);
+/* The same and the runner-up scores (see sm_match_wta_dev_batch_ru16) into runner_up_out (not NULL): n_pairs
+ * frames of u16, one more copy per group. */
+int sm_run_batch_ru16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                      uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
 
 /* The same over several GPUs of one box (SURVEY 8e, BASELINE config 4: whole pairs sharded across the
  * GPUs, inputs scattered from the host, no cross-device traffic): one context and one host thread per
@@ -304,6 +322,9 @@ int sm_multi_run_batch(sm_multi *m, int n_pairs, const uint8_t *first, const uin
 /* The same through sm_run_batch16 (best_out may be NULL). */
 int sm_multi_run_batch16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                          uint16_t *web_out, uint16_t *best_out);
+/* The same through sm_run_batch_ru16 (runner_up_out not NULL). */
+int sm_multi_run_batch_ru16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                            uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
 int sm_multi_device_count(const sm_multi *m);
 int sm_multi_destroy(sm_multi *m);
 
@@ -323,6 +344,10 @@ int sm_bands_run(sm_bands *b, const uint8_t *first, const uint8_t *second, doubl
  * those rows are copied back. */
 int sm_bands_run16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                    uint16_t *web_out, uint16_t *best_out);
+/* The same and the runner-up scores (see sm_match_wta_dev_batch_ru16): each band writes its own rows of the
+ * frame-sized runner_up_out (not NULL). */
+int sm_bands_run_ru16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                      uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
 int sm_bands_destroy(sm_bands *b);
 
 /* ---- geometry helpers (host-side, no GPU) --------------------------------------- */

@@ -41,6 +41,7 @@ SYMBOLS = [
     "sm_multi_create", "sm_multi_run_batch", "sm_multi_run_batch16", "sm_multi_device_count", "sm_multi_destroy",
     "sm_bands_create", "sm_bands_run", "sm_bands_run16", "sm_bands_destroy",
     "sm_create_range", "sm_create_band_range", "sm_multi_create_range", "sm_bands_create_range",
+    "sm_match_wta_dev_batch_ru16", "sm_run_batch_ru16", "sm_multi_run_batch_ru16", "sm_bands_run_ru16",
 ]
 
 
@@ -82,6 +83,7 @@ def lib() -> C.CDLL:
         L.sm_match_wta_dev.argtypes = [vp, vp, vp, vp, vp]
         L.sm_match_wta_dev_batch.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
         L.sm_match_wta_dev_batch16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
+        L.sm_match_wta_dev_batch_ru16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t]
         L.sm_elapsed_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.sm_last_launches.argtypes = [vp]
         L.sm_profile_begin.argtypes = [vp, i]
@@ -94,17 +96,20 @@ def lib() -> C.CDLL:
         L.sm_download_web_u16.argtypes = [vp, vp]
         L.sm_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
         L.sm_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
+        L.sm_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_band_rows.argtypes = [i, i, i, C.POINTER(i), C.POINTER(i)]
         L.sm_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_multi_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
         L.sm_multi_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
         L.sm_multi_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
+        L.sm_multi_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_multi_device_count.argtypes = [vp]
         L.sm_multi_destroy.argtypes = [vp]
         L.sm_bands_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_bands_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
         L.sm_bands_run.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_run16.argtypes = [vp, vp, vp, d, vp, vp]
+        L.sm_bands_run_ru16.argtypes = [vp, vp, vp, d, vp, vp, vp]
         L.sm_bands_destroy.argtypes = [vp]
         _lib = L
     return _lib
@@ -247,6 +252,14 @@ class StereoContext:
         _check(lib().sm_match_wta_dev_batch16(self._c, n_pairs, C.c_void_p(d_first_edges), C.c_void_p(d_second_edges),
                                               edge_stride, C.c_void_p(d_best or None), C.c_void_p(d_web), out_stride))
 
+    def match_wta_dev_batch_ru16(self, n_pairs: int, d_first_edges: int, d_second_edges: int, edge_stride: int,
+                                 d_best, d_web: int, d_runner_up: int, out_stride: int):
+        """match_wta_dev_batch16 that also writes each pixel's runner-up score (the second-largest of its scores over
+        the shifts; equal to best where shifts tie) to d_runner_up, uint16 with the web's pair stride."""
+        _check(lib().sm_match_wta_dev_batch_ru16(self._c, n_pairs, C.c_void_p(d_first_edges),
+                                                 C.c_void_p(d_second_edges), edge_stride, C.c_void_p(d_best or None),
+                                                 C.c_void_p(d_web), C.c_void_p(d_runner_up), out_stride))
+
     def elapsed_ms(self) -> float:
         ms = C.c_float()
         _check(lib().sm_elapsed_ms(self._c, C.byref(ms)))
@@ -298,15 +311,17 @@ class StereoContext:
         _check(lib().sm_download_web_u16(self._c, _ptr(out)))
         return out
 
-    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False):
+    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False,
+                  want_runner_up=False):
         """first/second: (n, H, W) u8.  Returns web (n, H, W) [and best]: int32, web as uint8 with web_u8, or (web16)
-        both as uint16, written by the hot kernel itself."""
+        both as uint16, written by the hot kernel itself.  want_runner_up (web16 only): also each pixel's runner-up
+        score, uint16, last in the result: (web, [best], runner_up)."""
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
-        return _run_batch(self._c, lib().sm_run_batch, lib().sm_run_batch16, first, second, threshold, web_u8,
-                          want_best, web_out, web16)
+        return _run_batch(self._c, lib().sm_run_batch, lib().sm_run_batch16, lib().sm_run_batch_ru16, first, second,
+                          threshold, web_u8, want_best, web_out, web16, want_runner_up)
 
     # -- convenience: the reference's whole step 2 on host edge maps -----------
     def match_wta_host(self, first_edges, second_edges):
@@ -315,16 +330,25 @@ class StereoContext:
         return self.download(BEST), self.download(WEB)
 
 
-def _run_batch(handle, run, run16, first, second, threshold, web_u8, want_best, web_out, web16):
-    """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16)."""
+def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, want_best, web_out, web16,
+               want_runner_up=False):
+    """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16), or with want_runner_up
+    their runner-up entries (run_ru)."""
     if web16 and web_u8:
         raise ValueError("web16 and web_u8 exclude each other")
+    if want_runner_up and not web16:
+        raise ValueError("want_runner_up needs web16=True (the runner-up comes with 16-bit results only)")
     n, H, W = first.shape
     dt = np.uint16 if web16 else (np.uint8 if web_u8 else np.int32)
     if web_out is None:
         web_out = np.zeros((n, H, W), dt)
     assert web_out.dtype == dt and web_out.shape == (n, H, W) and web_out.flags.c_contiguous
     best = np.zeros((n, H, W), np.uint16 if web16 else np.int32) if want_best else None
+    if want_runner_up:
+        ru = np.zeros((n, H, W), np.uint16)
+        _check(run_ru(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None,
+                      _ptr(ru)))
+        return (web_out, best, ru) if want_best else (web_out, ru)
     if web16:
         _check(run16(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None))
     else:
@@ -345,13 +369,14 @@ class MultiGpuBatch:
         _check(lib().sm_multi_create_range(C.byref(self._m), arr, len(devices), width, height, min_shift, num_shifts,
                                            square_width, variant))
 
-    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False):
+    def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False,
+                  want_runner_up=False):
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
-        return _run_batch(self._m, lib().sm_multi_run_batch, lib().sm_multi_run_batch16, first, second, threshold,
-                          web_u8, want_best, web_out, web16)
+        return _run_batch(self._m, lib().sm_multi_run_batch, lib().sm_multi_run_batch16, lib().sm_multi_run_batch_ru16,
+                          first, second, threshold, web_u8, want_best, web_out, web16, want_runner_up)
 
     def close(self):
         if self._m:
@@ -376,14 +401,22 @@ class MultiGpuBands:
         _check(lib().sm_bands_create_range(C.byref(self._b), arr, len(devices), width, height, min_shift, num_shifts,
                                            square_width, variant))
 
-    def run(self, first, second, threshold=0.15, want_best=False, web16=False):
-        """web [and best] of one pair: int32, or uint16 with web16."""
+    def run(self, first, second, threshold=0.15, want_best=False, web16=False, want_runner_up=False):
+        """web [and best] of one pair: int32, or uint16 with web16; want_runner_up (web16 only): also the runner-up
+        scores, uint16, last in the result: (web, [best], runner_up)."""
+        if want_runner_up and not web16:
+            raise ValueError("want_runner_up needs web16=True (the runner-up comes with 16-bit results only)")
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         assert first.shape == second.shape == (self.H, self.W)
         dt = np.uint16 if web16 else np.int32
         web = np.zeros((self.H, self.W), dt)
         best = np.zeros((self.H, self.W), dt) if want_best else None
+        if want_runner_up:
+            ru = np.zeros((self.H, self.W), np.uint16)
+            _check(lib().sm_bands_run_ru16(self._b, _ptr(first), _ptr(second), threshold, _ptr(web),
+                                           _ptr(best) if want_best else None, _ptr(ru)))
+            return (web, best, ru) if want_best else (web, ru)
         run = lib().sm_bands_run16 if web16 else lib().sm_bands_run
         _check(run(self._b, _ptr(first), _ptr(second), threshold, _ptr(web), _ptr(best) if want_best else None))
         return (web, best) if want_best else web

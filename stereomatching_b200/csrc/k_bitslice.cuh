@@ -1,6 +1,7 @@
-// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its two output families:
-// k_bitslice (int32 best / web, k_bitslice.cu) and k_bitslice16 (uint16_t, k_bitslice16.cu).  Each translation unit
-// instantiates one family through dispatch<OutT>, so that the two compile in parallel.
+// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its three output families:
+// k_bitslice (int32 best / web, k_bitslice.cu), k_bitslice16 (uint16_t, k_bitslice16.cu) and k_bitslice_ru (uint16_t
+// and the runner-up score, k_bitslice_ru.cu).  Each translation unit instantiates one family through dispatch, so
+// that the three compile in parallel.
 //
 // What it replaces: fillup_matches + 30x{memset, addup_pixels_in_square, record_score} +
 // find_highest_scoring_shifts of the reference (stereo.cu:127-225), i.e. per pixel and per
@@ -95,6 +96,11 @@ __host__ __device__ constexpr int pow2_at_least(int v)
 }
 
 template <int HALF, int NW, int SEG>
+constexpr bool ring_aligns();
+
+// ALIGNED_M (the runner-up family): the centre-match ring holds a whole number of blocks, so that the RB centre rows a
+// steady block reads are consecutive ring rows (see bitslice_body) -- where the larger ring costs no CTA per SM
+template <int HALF, int NW, int SEG, bool ALIGNED_M = false>
 struct WS {
     static constexpr int N = 2 * HALF + 1;       // window side
     static constexpr int KH = bits_for(N);       // planes of a horizontal count (<= N)
@@ -103,7 +109,13 @@ struct WS {
     static constexpr int NSEG = TW / SEG;        // walkers per (row, word)
     static constexpr int RB = 32 / (NW * NSEG);  // rows per block: 32 walkers
     static constexpr int NR = RB;                // H rows in shared memory: one block
-    static constexpr int NRM = RB + HALF + 1;    // centre-match ring rows
+    static constexpr bool M_ALIGNED = [] {
+        if constexpr (ALIGNED_M)
+            return ring_aligns<HALF, NW, SEG>();
+        else
+            return false;
+    }();
+    static constexpr int NRM = M_ALIGNED ? (RB + HALF + 1 + RB - 1) / RB * RB : RB + HALF + 1;  // centre-match ring rows
     static constexpr int HROW = TW + 1;          // uint4 per (ring row, word); +1 staggers banks
     // words per M ring row, +stagger; two words per lane: even, so that the LDS.64 stays aligned
     static constexpr int MROW = NW == 1 ? TW + 1 : TW * NW + 2;
@@ -128,6 +140,16 @@ struct WS {
     static_assert(STEPS + 32 <= 96 && STEPS < 64, "walker windows: 96 bits of RB, 64 bits of LA/LB");
     static_assert(N * EC <= 512, "the vertical window must fit one TMEM allocation");
 };
+
+// whether the centre-match ring rounded up to whole blocks leaves the CTAs per SM as they are
+template <int HALF, int NW, int SEG>
+constexpr bool ring_aligns()
+{
+    using P = WS<HALF, NW, SEG>;
+    constexpr int nrm = (P::NRM + P::RB - 1) / P::RB * P::RB;
+    constexpr size_t smem_cta = P::SMEM_CTA + (size_t)P::WPC * 4 * (size_t)(((nrm * P::MROW + 3) & ~3) - P::MQN);
+    return (int)((227 * 1024) / (smem_cta + 1024)) >= P::CTAS_PER_SM;
+}
 
 enum { MODE_LAUNCH = 0, MODE_PREPARE = 1, MODE_TMEM_COLUMNS = 2 };
 
@@ -425,9 +447,64 @@ __device__ __forceinline__ void walk(const uint32_t (&q)[3], const uint32_t (&lw
 // AS_WRITTEN (all but the MULTI kernels, which would spill at their 128 registers): the first plane's select and
 // the winning lane's index are kept off the ALU pipe too (below); otherwise ptxas makes the former three SELs per
 // row and the latter two FLO, a LOP3, a max and an add.
-template <int NR_, int NW, int PV, bool AS_WRITTEN>
+//
+// One plane of a bit-serial max: t = cand & V_p & M; if (t != 0) { cand = t; acc |= 1 << p }.  The "any lane left"
+// test is folded into the same LOP3s: the predicate output of one feeds the next (lop3.or d|p), so a plane costs NW
+// ALU instructions instead of NW + 1 (a separate OR-and-test); the selects are predicated multiply-adds.
+template <int NW>
+__device__ __forceinline__ void wta_plane(uint32_t (&cand)[NW], int &acc, const uint32_t (&Vp)[NW],
+                                          const uint32_t (&M)[NW], int one, int p)
+{
+    if (NW == 2) {
+        asm("{ .reg .pred q0, q; .reg .b32 t0, t1;\n\t"
+            "lop3.or.b32 t0|q0, %0, %3, %4, 0x80, 0;\n\t"
+            "lop3.or.b32 t1|q, %1, %5, %6, 0x80, q0;\n\t"
+            "@q mad.lo.u32 %0, t0, %7, 0;\n\t@q mad.lo.u32 %1, t1, %7, 0;\n\t@q mad.lo.s32 %2, %7, %8, %2; }"
+            : "+r"(cand[0]), "+r"(cand[NW - 1]), "+r"(acc)
+            : "r"(Vp[0]), "r"(M[0]), "r"(Vp[NW - 1]), "r"(M[NW - 1]), "r"(one), "r"(1 << p));
+    } else {
+        asm("{ .reg .pred q; .reg .b32 t0;\n\t"
+            "lop3.or.b32 t0|q, %0, %2, %3, 0x80, 0;\n\t"
+            "@q mad.lo.u32 %0, t0, %4, 0;\n\t@q mad.lo.s32 %1, %4, %5, %1; }"
+            : "+r"(cand[0]), "+r"(acc)
+            : "r"(Vp[0]), "r"(M[0]), "r"(one), "r"(1 << p));
+    }
+}
+
+// PTX shifts clamp the amount (to 32: the result is 0), which C++ shifts do not promise
+__device__ __forceinline__ uint32_t shr_clamp(uint32_t x, uint32_t n)
+{
+    uint32_t r;
+    asm("shr.b32 %0, %1, %2;" : "=r"(r) : "r"(x), "r"(n));
+    return r;
+}
+
+// The valid lanes but one of those that tie for best (cand, the survivors of the first chain, never empty): the lowest,
+// c & -c over the 32*NW lanes of the row.  The negation is a multiply by all ones (`ones`, opaque to ptxas), with two
+// words one 64-bit multiply: both run on the FMA pipe, and what is left is one LOP3 per word, valid ^ (c & -c).
+template <int NW>
+__device__ __forceinline__ void drop_one_tied(const uint32_t (&valid)[NW], const uint32_t (&cand)[NW], uint32_t ones,
+                                              uint32_t (&cand2)[NW])
+{
+    uint32_t n[NW];
+    if constexpr (NW == 2) {
+        asm("{ .reg .u64 c, o, n; mov.b64 c, {%2, %3}; mov.b64 o, {%4, %4}; mul.lo.u64 n, c, o; mov.b64 {%0, %1}, n; }"
+            : "=r"(n[0]), "=r"(n[1]) : "r"(cand[0]), "r"(cand[1]), "r"(ones));
+    } else {
+        asm("mad.lo.u32 %0, %1, %2, 0;" : "=r"(n[0]) : "r"(cand[0]), "r"(ones));
+    }
+#pragma unroll
+    for (int w = 0; w < NW; w++) cand2[w] = lop3<0x78>(valid[w], cand[w], n[w]);  // x ^ (y & z)
+}
+
+// RU (the runner-up family, k_bitslice_ru): ru[k] = the second-largest masked score of row k's lanes, i.e. the maximum
+// over every valid lane but the winner's.  A second bit-serial max from the top plane down runs over the valid lanes
+// but one of those that tie for best (drop_one_tied; which one does not change the value): where several lanes tie,
+// one of the others survives every plane best has, so ru == best there; with one lane, ru == 0.
+template <int NR_, int NW, int PV, bool AS_WRITTEN, bool RU = false>
 __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint32_t (&M)[NR_][NW],
-                                    const uint32_t (&valid)[NW], int one, int base, int (&best)[NR_], int (&web)[NR_])
+                                    const uint32_t (&valid)[NW], int one, int base, int (&best)[NR_], int (&web)[NR_],
+                                    int *ru = nullptr)
 {
     uint32_t cand[NR_][NW];
 #pragma unroll
@@ -466,22 +543,15 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
                         : "=r"(cand[k][0]), "+r"(best[k])
                         : "r"(valid[0]), "r"(V[k][0][p]), "r"(M[k][0]), "r"(one), "r"(1 << p));
                 }
-            } else if (NW == 2) {
-                asm("{ .reg .pred q0, q; .reg .b32 t0, t1;\n\t"
-                    "lop3.or.b32 t0|q0, %0, %3, %4, 0x80, 0;\n\t"
-                    "lop3.or.b32 t1|q, %1, %5, %6, 0x80, q0;\n\t"
-                    "@q mad.lo.u32 %0, t0, %7, 0;\n\t@q mad.lo.u32 %1, t1, %7, 0;\n\t@q mad.lo.s32 %2, %7, %8, %2; }"
-                    : "+r"(cand[k][0]), "+r"(cand[k][NW - 1]), "+r"(best[k])
-                    : "r"(V[k][0][p]), "r"(M[k][0]), "r"(V[k][NW - 1][p]), "r"(M[k][NW - 1]), "r"(one), "r"(1 << p));
             } else {
-                asm("{ .reg .pred q; .reg .b32 t0;\n\t"
-                    "lop3.or.b32 t0|q, %0, %2, %3, 0x80, 0;\n\t"
-                    "@q mad.lo.u32 %0, t0, %4, 0;\n\t@q mad.lo.s32 %1, %4, %5, %1; }"
-                    : "+r"(cand[k][0]), "+r"(best[k])
-                    : "r"(V[k][0][p]), "r"(M[k][0]), "r"(one), "r"(1 << p));
+                uint32_t Vp[NW];
+#pragma unroll
+                for (int w = 0; w < NW; w++) Vp[w] = V[k][w][p];
+                wta_plane<NW>(cand[k], best[k], Vp, M[k], one, p);
             }
         }
     }
+    uint32_t cand2[NR_][NW];  // RU: the valid lanes but one of those that tie for best
 #pragma unroll
     for (int k = 0; k < NR_; k++) {
         // web = base + the highest surviving lane; a later word holds higher shifts.  m = 32 * NW - 1 - lane, from
@@ -494,6 +564,7 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
             int idx = 31 - __clz(cand[k][0]);
             if (NW == 2) idx = max(idx, (31 - __clz(cand[k][NW - 1])) ^ 32);
             web[k] = base + idx;
+            if constexpr (RU) drop_one_tied<NW>(valid, cand[k], (uint32_t)-one, cand2[k]);
             continue;
         }
         uint32_t m, m1;
@@ -503,6 +574,29 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
             m = min(m1, m + 32u);
         }
         asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(web[k]) : "r"(m), "r"(-one), "r"(base + 32 * NW - 1));
+        if constexpr (RU) {
+            if constexpr (NW == 2) {
+                drop_one_tied<NW>(valid, cand[k], (uint32_t)-one, cand2[k]);
+            } else {
+                // one word (also the chains of C2 and HP): the winner's own bit, from its shift amount m (fewer
+                // registers there than the negation, which at 128 registers made some of those kernels spill)
+                cand2[k][0] = lop3<0x30>(valid[0], shr_clamp(0x80000000u, m), 0u);  // valid & ~bit
+            }
+        }
+    }
+    if constexpr (RU) {
+#pragma unroll
+        for (int k = 0; k < NR_; k++) ru[k] = 0;
+#pragma unroll
+        for (int p = PV - 1; p >= 0; p--) {
+#pragma unroll
+            for (int k = 0; k < NR_; k++) {
+                uint32_t Vp[NW];
+#pragma unroll
+                for (int w = 0; w < NW; w++) Vp[w] = V[k][w][p];
+                wta_plane<NW>(cand2[k], ru[k], Vp, M[k], one, p);
+            }
+        }
     }
 }
 
@@ -542,12 +636,14 @@ __device__ __forceinline__ void store_if(uint16_t *lane_base, int row, int row_b
 // per half, the winner-take-all runs one chain per half, and lane l of a strip stands for the pixel columns
 // 32*(l/16) + l%16 and that + 16 (so a walker's 16-pixel segment covers 32 columns and a strip is twice as wide).
 //
-// The body of both kernel families; OutT (int32_t or uint16_t) is the type of the stored best and web.  Pair z's
-// outputs are z * best_stride (best) and z * out_stride (web) elements further.
-template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
-__device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, OutT *out_web, size_t best_stride)
+// The body of the kernel families; OutT (int32_t or uint16_t) is the type of the stored best and web.  Pair z's
+// outputs are z * best_stride (best) and z * out_stride (web, runner-up) elements further.  RU (k_bitslice_ru, 16-bit):
+// the runner-up score goes to out_ru as well.
+template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP, bool RU = false>
+__device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, OutT *out_web, size_t best_stride,
+                                              uint16_t *out_ru = nullptr)
 {
-    using C = WS<HALF, NW, SEG>;
+    using C = WS<HALF, NW, SEG, RU && !C2 && !HP>;  // (C2 / HP: the aligned ring costs them registers and spills)
     constexpr int N = C::N, KH = C::KH, PV = C::PV, TW = C::TW, RB = C::RB, NR = C::NR, NRM = C::NRM;
     constexpr int HROW = C::HROW, MROW = C::MROW, STEPS = C::STEPS, EC = C::EC, WPC = C::WPC;
 
@@ -584,6 +680,8 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
     static_assert(std::is_same<OutT, int32_t>::value || std::is_same<OutT, uint16_t>::value, "int32 or 16-bit outputs");
     out_best += blockIdx.z * best_stride;
     out_web += blockIdx.z * a.h.out_stride;
+    static_assert(!RU || std::is_same<OutT, uint16_t>::value, "runner-up: 16-bit outputs only");
+    if constexpr (RU) out_ru += blockIdx.z * a.h.out_stride;
     const PackedGeom &g = a.h.g;
     static_assert(!C2 || (NW == 2 && !MULTI), "column pairs: two words, one 32-shift chunk");
     static_assert(!HP || (!MULTI && SEG == 16 && (C2 || NW == 1)), "half-word pairs: one chunk, 16-pixel segments");
@@ -662,19 +760,29 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 
         WalkRaw in = {};
         if (ja + wr < last_pr) load_walk_raw(in, a.h, ja + wr, rbit, lbit);
-        int mslot0 = 0;  // centre-match ring slot of padded row p0
+        // centre-match ring slot of padded row p0.  C::M_ALIGNED (RU): started so that the centre rows of every steady block begin at a
+        // multiple of RB (p0 - ja is (2*HALF) % RB plus whole blocks there), and with NRM a multiple of RB they never wrap
+        // within the block: one ring slot per block instead of a compare-and-select per row (which ptxas keeps on the
+        // ALU pipe in this family)
+        int mslot0 = C::M_ALIGNED ? ((HALF - (2 * HALF) % RB) % RB + RB) % RB : 0;
         // next output row of the frame, and the lane's own column of the two output arrays
         int orow = a.h.row0 + ja;
         const int row_bytes = (int)sizeof(OutT) * g.W;
         OutT *const lane_best = out_best + ximg, *const lane_web = out_web + ximg;
+        uint16_t *const lane_ru = RU ? out_ru + ximg : nullptr;
 
-        // store a finished row (best, web) and advance the output pointers.  MULTI: a later chunk holds higher
-        // shifts, so it wins ties against what the earlier chunks left in `best` (prev)
-        auto put = [&](int best, int web, int prev) {
+        // store a finished row (best, web[, runner-up]) and advance the output pointers.  MULTI: a later chunk holds
+        // higher shifts, so it wins ties against what the earlier chunks left in `best` (prev).  The runner-up of the
+        // shifts so far is the larger of the loser's best and the winner's runner-up (prev_ru: the earlier chunks')
+        auto put = [&](int best, int web, int prev, int ru, int prev_ru) {
             bool st = store_ok;
             if (MULTI && chunk != 0) st = st && best >= prev;
             store_if<0>(lane_best, orow, row_bytes, best, st);
             store_if<0>(lane_web, orow, row_bytes, web, st);
+            if constexpr (RU) {
+                if (MULTI) ru = max(min(best, prev), best >= prev ? ru : prev_ru);  // (chunk 0: prev == prev_ru == 0)
+                store_if<0>(lane_ru, orow, row_bytes, ru, store_ok);
+            }
             orow++;
         };
         // what the earlier chunks left in `best` for the next output row + k (only read where it is stored)
@@ -683,32 +791,50 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
             if (MULTI && chunk != 0 && store_ok) v = lane_best[(size_t)(orow + k) * g.W];
             return v;
         };
+        // ... and in the runner-up
+        auto load_prev_ru = [&](int k) {
+            int v = 0;
+            if (RU && MULTI && chunk != 0 && store_ok) v = lane_ru[(size_t)(orow + k) * g.W];
+            return v;
+        };
         // C2: the two pixels of a lane (columns ximg and ximg + 32) of one finished row
-        auto put2 = [&](int best0, int web0, int best1, int web1) {
+        auto put2 = [&](int best0, int web0, int best1, int web1, int ru0, int ru1) {
             store_if<0>(lane_best, orow, row_bytes, best0, store_ok);
             store_if<0>(lane_web, orow, row_bytes, web0, store_ok);
             store_if<TW>(lane_best, orow, row_bytes, best1, store_ok2);
             store_if<TW>(lane_web, orow, row_bytes, web1, store_ok2);
+            if constexpr (RU) {
+                store_if<0>(lane_ru, orow, row_bytes, ru0, store_ok);
+                store_if<TW>(lane_ru, orow, row_bytes, ru1, store_ok2);
+            }
             orow++;
         };
         // HP: the 2 * NW pixels of a lane of one finished row: word w covers columns ximg + w * WCOLS and that + 16
-        auto put_hp = [&](const int *bl, const int *wl, const int *bh, const int *wh) {
+        auto put_hp = [&](const int *bl, const int *wl, const int *bh, const int *wh, const int *rl, const int *rh) {
             store_if<0>(lane_best, orow, row_bytes, bl[0], ximg < g.W);
             store_if<0>(lane_web, orow, row_bytes, wl[0], ximg < g.W);
             store_if<16>(lane_best, orow, row_bytes, bh[0], ximg + 16 < g.W);
             store_if<16>(lane_web, orow, row_bytes, wh[0], ximg + 16 < g.W);
+            if constexpr (RU) {
+                store_if<0>(lane_ru, orow, row_bytes, rl[0], ximg < g.W);
+                store_if<16>(lane_ru, orow, row_bytes, rh[0], ximg + 16 < g.W);
+            }
             if constexpr (NW == 2) {
                 store_if<WCOLS>(lane_best, orow, row_bytes, bl[NW - 1], ximg + WCOLS < g.W);
                 store_if<WCOLS>(lane_web, orow, row_bytes, wl[NW - 1], ximg + WCOLS < g.W);
                 store_if<WCOLS + 16>(lane_best, orow, row_bytes, bh[NW - 1], ximg + WCOLS + 16 < g.W);
                 store_if<WCOLS + 16>(lane_web, orow, row_bytes, wh[NW - 1], ximg + WCOLS + 16 < g.W);
+                if constexpr (RU) {
+                    store_if<WCOLS>(lane_ru, orow, row_bytes, rl[NW - 1], ximg + WCOLS < g.W);
+                    store_if<WCOLS + 16>(lane_ru, orow, row_bytes, rh[NW - 1], ximg + WCOLS + 16 < g.W);
+                }
             }
             orow++;
         };
         // winner-take-all of G rows held as Vs[G][NW][PV] / Ms[G][NW], then the stores: one WTA over both words
         // of a pixel, or (C2) one per word, the 2*G single-word chains interleaved like rows, or (HP) one per
         // half word: the lower halves of all words first, then the upper halves
-        auto finish_rows = [&](auto gtag, const auto &Vs, const auto &Ms, const int *prev) {
+        auto finish_rows = [&](auto gtag, const auto &Vs, const auto &Ms, const int *prev, const int *prev_ru) {
             constexpr int G_ = decltype(gtag)::value;
             if constexpr (HP) {
                 constexpr int NCH = G_ * NW;
@@ -723,16 +849,17 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                     }
                 const uint32_t vl1[1] = {valid_lo}, vh1[1] = {valid_hi};
                 // the upper half's lanes are 16..31 of the word: web = M + lane - 16 + 1
-                int bl[NCH], wl[NCH], bh[NCH], wh[NCH];
-                wta<NCH, 1, PV, !MULTI>(V1, M1, vl1, one, a.h.M + 1, bl, wl);
-                wta<NCH, 1, PV, !MULTI>(V1, M1, vh1, one, a.h.M + 1 - 16, bh, wh);
+                int bl[NCH], wl[NCH], bh[NCH], wh[NCH], rl[NCH], rh[NCH];
+                wta<NCH, 1, PV, !MULTI, RU>(V1, M1, vl1, one, a.h.M + 1, bl, wl, rl);
+                wta<NCH, 1, PV, !MULTI, RU>(V1, M1, vh1, one, a.h.M + 1 - 16, bh, wh, rh);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW);
+                for (int k = 0; k < G_; k++)
+                    put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW, rl + k * NW, rh + k * NW);
             } else if constexpr (!C2) {
-                int best[G_], web[G_];
-                wta<G_, NW, PV, !MULTI>(Vs, Ms, valid, one, a.h.M + 32 * wg0 + 1, best, web);
+                int best[G_], web[G_], ru[G_];
+                wta<G_, NW, PV, !MULTI, RU>(Vs, Ms, valid, one, a.h.M + 32 * wg0 + 1, best, web, ru);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put(best[k], web[k], prev[k]);
+                for (int k = 0; k < G_; k++) put(best[k], web[k], prev[k], ru[k], prev_ru[k]);
             } else {
                 uint32_t V1[2 * G_][1][PV], M1[2 * G_][1];
 #pragma unroll
@@ -744,10 +871,11 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                         for (int p = 0; p < PV; p++) V1[2 * k + w][0][p] = Vs[k][w][p];
                     }
                 const uint32_t valid1[1] = {valid[0]};
-                int best[2 * G_], web[2 * G_];
-                wta<2 * G_, 1, PV, !MULTI>(V1, M1, valid1, one, a.h.M + 1, best, web);
+                int best[2 * G_], web[2 * G_], ru[2 * G_];
+                wta<2 * G_, 1, PV, !MULTI, RU>(V1, M1, valid1, one, a.h.M + 1, best, web, ru);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1]);
+                for (int k = 0; k < G_; k++)
+                    put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1], ru[2 * k], ru[2 * k + 1]);
             }
         };
         auto load_m = [&](int mslot_c, uint32_t (&M)[NW]) {
@@ -832,9 +960,11 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 
             // MULTI: the earlier chunks' `best` of the rows this block finishes, asked for now so that the loads
             // are back long before the stores that depend on them (they used to be one exposed L2 round trip per row)
-            int prev[RB];
+            int prev[RB], prev_ru[RB];
 #pragma unroll
             for (int r = 0; r < RB; r++) prev[r] = steady ? load_prev(r) : 0;
+#pragma unroll
+            for (int r = 0; r < RB; r++) prev_ru[r] = RU && steady ? load_prev_ru(r) : 0;
 
             pass_a(p0, nrows);
 
@@ -844,6 +974,7 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                 // Rows go in groups of G so that their winner-take-all chains interleave.
                 constexpr int G = (RB % 4 == 0) ? 4 : ((RB % 2 == 0) ? 2 : 1);
                 constexpr int GT = N < G ? 1 : G;  // a group's rows must be distinct ring rows
+                const int mbase = C::M_ALIGNED ? wrap_m(mslot0 - HALF) : 0;  // the ring row of the block's first centre row
 #pragma unroll
                 for (int r = 0; r < RB; r += G) {
                     uint32_t Vs[G][NW][PV], Ms[G][NW];
@@ -882,9 +1013,12 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 #pragma unroll
                             for (int p = 0; p < PV; p++) Vs[k][w][p] = V[w][p];
                         }
-                        load_m(wrap_m(mslot0 + r + k - HALF), Ms[k]);
+                        if constexpr (C::M_ALIGNED)
+                            load_m(mbase + r + k, Ms[k]);
+                        else
+                            load_m(wrap_m(mslot0 + r + k - HALF), Ms[k]);
                     }
-                    finish_rows(std::integral_constant<int, G>{}, Vs, Ms, prev + r);
+                    finish_rows(std::integral_constant<int, G>{}, Vs, Ms, prev + r, prev_ru + r);
                 }
             } else if (filling) {
                 fill_rows(RB);
@@ -921,8 +1055,8 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 #pragma unroll
                             for (int p = 0; p < PV; p++) Vs[0][w][p] = V[w][p];
                         load_m(wrap_m(mslot0 + r - HALF), Ms[0]);  // centre row j + HALF
-                        const int pv = load_prev(0);
-                        finish_rows(std::integral_constant<int, 1>{}, Vs, Ms, &pv);
+                        const int pv = load_prev(0), pvr = load_prev_ru(0);
+                        finish_rows(std::integral_constant<int, 1>{}, Vs, Ms, &pv, &pvr);
                     }
                 }
             }
@@ -957,19 +1091,48 @@ k_bitslice16(BitsliceArgs a)
                                                           static_cast<uint16_t *>(a.h.web), a.h.out_stride);
 }
 
-template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+// uint16_t best / web and the runner-up score: the 16-bit kernels' argument and the runner-up array (HotArgs and
+// BitsliceArgs stay as they are: a field there moves the other families' registers)
+struct BitsliceRuArgs {
+    BitsliceArgs b;
+    uint16_t *runner_up;  // [pairs][FH][W], pair z out_stride elements further
+};
+
+// CTAs per SM of a runner-up kernel: its 16-bit sibling's, but one fewer for the MULTI kernels of windows 9 to 15.
+// At the sibling's 4 CTAs (128 registers) those spill 36 to 128 bytes more than it; 12 and 16 warps per SM run alike.
+template <int HALF, int NW, int SEG, bool MULTI>
+constexpr int ru_ctas_per_sm()
+{
+    constexpr int c = WS<HALF, NW, SEG, true>::CTAS_PER_SM;
+    return MULTI && HALF >= 4 && HALF <= 7 && c == 4 ? c - 1 : c;
+}
+
+template <int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+__global__ void __launch_bounds__(32 * WS<HALF, NW, SEG, true>::WPC, (ru_ctas_per_sm<HALF, NW, SEG, MULTI>()))
+k_bitslice_ru(BitsliceRuArgs a)
+{
+    bitslice_body<uint16_t, HALF, NW, SEG, MULTI, C2, HP, true>(a.b, static_cast<uint16_t *>(a.b.h.best),
+                                                                static_cast<uint16_t *>(a.b.h.web), a.b.h.out_stride,
+                                                                a.runner_up);
+}
+
+// the family: int32 (k_bitslice), 16-bit (k_bitslice16) or 16-bit with the runner-up (RU, k_bitslice_ru)
+template <typename OutT, bool RU, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
 constexpr auto kernel_of()
 {
-    if constexpr (std::is_same<OutT, uint16_t>::value)
+    static_assert(!RU || std::is_same<OutT, uint16_t>::value, "runner-up: 16-bit outputs only");
+    if constexpr (RU)
+        return k_bitslice_ru<HALF, NW, SEG, MULTI, C2, HP>;
+    else if constexpr (std::is_same<OutT, uint16_t>::value)
         return k_bitslice16<HALF, NW, SEG, MULTI, C2, HP>;
     else
         return k_bitslice<HALF, NW, SEG, MULTI, C2, HP>;
 }
 
-template <typename OutT, int HALF, int NW, int SEG, bool C2, bool HP>
-int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec)
+template <typename OutT, bool RU, int HALF, int NW, int SEG, bool C2, bool HP>
+int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec, uint16_t *runner_up)
 {
-    using C = WS<HALF, NW, SEG>;
+    using C = WS<HALF, NW, SEG, RU && !C2 && !HP>;  // (bitslice_body's layout: its centre-match ring, its shared memory)
     if (mode == MODE_TMEM_COLUMNS) return C::TCOLS;
     // MULTI: more than one chunk of 32*NW shifts, i.e. (best, web) are merged across passes
     // (one word per lane is only chosen for 32 shifts or fewer: no MULTI flavour of it is instantiated)
@@ -982,14 +1145,16 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
         set_error("bit-sliced kernel: half-word pairs hold at most 16 shifts, not %d", h.g.D);
         return SM_ERR_ARG;
     }
-    auto kern = (C2 || HP) ? kernel_of<OutT, HALF, NW, SEG, false, C2, HP>()
-                           : (multi ? kernel_of<OutT, HALF, NW, SEG, NW == 2 && !HP, false, false>()
-                                    : kernel_of<OutT, HALF, NW, SEG, false, false, false>());
+    auto kern = (C2 || HP) ? kernel_of<OutT, RU, HALF, NW, SEG, false, C2, HP>()
+                           : (multi ? kernel_of<OutT, RU, HALF, NW, SEG, NW == 2 && !HP, false, false>()
+                                    : kernel_of<OutT, RU, HALF, NW, SEG, false, false, false>());
     // resident warps per SM of this instantiation: what shared memory, the 512 TMEM columns and the register file
     // allow, all known at compile time (WS::CTAS_PER_SM is also the kernel's __launch_bounds__).  (The occupancy
     // API is not asked: it answers 1 CTA per SM for these kernels, whatever carve-out is set, while the
     // hardware runs the 4 that ncu's launch__occupancy_limit_* report.)
-    const int warps_per_sm = C::CTAS_PER_SM * C::WPC;
+    // (the runner-up family's MULTI kernels may hold fewer: ru_ctas_per_sm)
+    const int ctas_per_sm = RU && multi ? ru_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>() : C::CTAS_PER_SM;
+    const int warps_per_sm = ctas_per_sm * C::WPC;
     if (mode == MODE_PREPARE) {
         SM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_REQ));
         SM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -1043,7 +1208,7 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
             const int ctas = ctas_per_run * got;
             const int per_sm_max = (ctas + num_sms - 1) / num_sms;
             const double per_sm = 10 * ctas < 17 * slots ? (double)per_sm_max : (double)ctas / num_sms + 0.05;
-            const int resident = (per_sm_max < C::CTAS_PER_SM ? per_sm_max : C::CTAS_PER_SM) * C::WPC;
+            const int resident = (per_sm_max < ctas_per_sm ? per_sm_max : ctas_per_sm) * C::WPC;
             const double cost = per_sm * (rows + 0.5 * fill_rows + start_rows) / eff_of(resident);
             if (best_cost < 0 || cost < best_cost) best_cost = cost, segs = got;
             if (ctas > 6 * slots) break;
@@ -1059,6 +1224,12 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
     }
     segs = shape(segs, a.rows_per_seg);
     dim3 grid((strips + C::WPC - 1) / C::WPC, segs, h.npairs);
+    // the kernel's argument: BitsliceArgs, or with RU that and the runner-up array
+    typename std::conditional<RU, BitsliceRuArgs, BitsliceArgs>::type arg;
+    if constexpr (RU)
+        arg = BitsliceRuArgs{a, runner_up};
+    else
+        arg = a;
     if (h.after_pack) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = grid;
@@ -1070,9 +1241,9 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        SM_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
+        SM_CUDA(cudaLaunchKernelEx(&cfg, kern, arg));
     } else {
-        kern<<<grid, 32 * C::WPC, C::SMEM_REQ, s>>>(a);
+        kern<<<grid, 32 * C::WPC, C::SMEM_REQ, s>>>(arg);
     }
     SM_CUDA(cudaGetLastError());
     if (rec) {
@@ -1129,9 +1300,10 @@ static Shape pick_shape(const HotArgs &h, int num_sms)
     return sh;
 }
 
-// the kernel of the geometry, from the family that stores OutT
-template <typename OutT>
-int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec = nullptr)
+// the kernel of the geometry, from the family that stores OutT (RU: and the runner-up, to runner_up)
+template <typename OutT, bool RU = false>
+int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec = nullptr,
+             uint16_t *runner_up = nullptr)
 {
     if (mode == MODE_PREPARE && h.npairs == 1) {
         // a context launches one pair at a time AND batches: prepare the batch flavour too if it is another kernel
@@ -1139,7 +1311,7 @@ int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchReco
         hb.npairs = 2;
         const Shape a = pick_shape(h, num_sms), b = pick_shape(hb, num_sms);
         if (a.seg != b.seg || a.nw != b.nw || a.c2 != b.c2 || a.hp != b.hp) {
-            const int rc = dispatch<OutT>(hb, num_sms, s, mode);
+            const int rc = dispatch<OutT, RU>(hb, num_sms, s, mode);
             if (rc < 0) return rc;
         }
     }
@@ -1147,7 +1319,7 @@ int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchReco
     const int half = h.g.half;
 #define SM_SHAPE(HF, NW_, SEG_, C2_, HP_) \
     if (half == HF && sh.nw == NW_ && sh.seg == SEG_ && sh.c2 == C2_ && sh.hp == HP_) \
-        return launch_one<OutT, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec);
+        return launch_one<OutT, RU, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec, runner_up);
 #define SM_HALVES(M, ...) \
     M(0, __VA_ARGS__) M(1, __VA_ARGS__) M(2, __VA_ARGS__) M(3, __VA_ARGS__) M(4, __VA_ARGS__) M(5, __VA_ARGS__) \
     M(6, __VA_ARGS__) M(7, __VA_ARGS__) M(8, __VA_ARGS__) M(9, __VA_ARGS__) M(10, __VA_ARGS__) M(11, __VA_ARGS__) \

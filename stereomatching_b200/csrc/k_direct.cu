@@ -41,26 +41,31 @@ __device__ __forceinline__ void window(const HotArgs &a, int x, int j, int i, in
     }
 }
 
-// best / web of pixel x of band row j, stored as T; best may be NULL (16-bit outputs: web only)
-template <typename T>
-__device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *web_out)
+// best / web of pixel x of band row j, stored as T; best may be NULL (16-bit outputs: web only).  RU: also the
+// runner-up score (the second largest of the pixel's scores, best again where two shifts tie for it)
+template <typename T, bool RU = false>
+__device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *web_out, uint16_t *ru_out = nullptr)
 {
     int x = blockIdx.x * blockDim.x + threadIdx.x;
     int j = blockIdx.y * blockDim.y + threadIdx.y;
     if (x >= a.g.W || j >= a.g.BH) return;
-    int best = 0, web = 0;
+    int best = 0, web = 0, ru = 0;
     for (int i = 0; i < a.g.D; i++) {
         int box, centre;
         window(a, x, j, i, box, centre);
         int score = centre ? box : 0;  // record_score: only where the centre matched
         if (score >= best) {           // last equal maximum wins -> highest shift
+            if (RU) ru = best;
             best = score;
             web = i + 1;
+        } else if (RU) {
+            ru = max(ru, score);
         }
     }
     size_t p = (size_t)(a.row0 + j) * a.g.W + x;
     if (sizeof(T) == 4 || best_out) best_out[p] = (T)best;  // (the int32 kernel always has a best)
     web_out[p] = (T)(a.M + web);  // shift i of the planes is M + i
+    if (RU) ru_out[p] = (uint16_t)ru;
 }
 
 __global__ void __launch_bounds__(256) k_direct(HotArgs a)
@@ -74,11 +79,19 @@ __global__ void __launch_bounds__(256) k_direct16(HotArgs a)
     direct_pixel(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web));
 }
 
-int launch_direct(const HotArgs &a, cudaStream_t s, bool out16)
+// the 16-bit twin with the runner-up score (a.best may be NULL; runner_up may not)
+__global__ void __launch_bounds__(256) k_direct16_ru(HotArgs a, uint16_t *runner_up)
+{
+    direct_pixel<uint16_t, true>(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web), runner_up);
+}
+
+int launch_direct(const HotArgs &a, cudaStream_t s, bool out16, uint16_t *runner_up)
 {
     dim3 block(32, 8);
     dim3 grid((a.g.W + block.x - 1) / block.x, (a.g.BH + block.y - 1) / block.y);
-    if (out16)
+    if (runner_up)
+        k_direct16_ru<<<grid, block, 0, s>>>(a, runner_up);
+    else if (out16)
         k_direct16<<<grid, block, 0, s>>>(a);
     else
         k_direct<<<grid, block, 0, s>>>(a);
@@ -117,6 +130,7 @@ void warm_direct()
 {
     warm_kernel(k_direct);
     warm_kernel(k_direct16);
+    warm_kernel(k_direct16_ru);
     warm_kernel(k_planes);
 }
 

@@ -105,12 +105,16 @@ struct LaunchRecord {
 int launch_pack(const uint8_t *e1, const uint8_t *e2, int FH, int row0, int variant,
                 const PackedGeom &g, int M, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
                 int npairs = 1, size_t edge_stride = 0, size_t plane_stride = 0);
-int launch_direct(const HotArgs &a, cudaStream_t s, bool out16 = false);  // out16: the 16-bit twin
+// out16: the 16-bit twin; runner_up (16-bit outputs only): the twin that also stores the runner-up score there
+int launch_direct(const HotArgs &a, cudaStream_t s, bool out16 = false, uint16_t *runner_up = nullptr);
 int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);
 int launch_bitslice16(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);  // uint16_t outputs
+// uint16_t outputs and the runner-up score [pairs][FH][W], pair z a.out_stride elements further
+int launch_bitslice_ru(const HotArgs &a, uint16_t *runner_up, int num_sms, cudaStream_t s, LaunchRecord *rec);
 bool bitslice_supports(int half, int D);
 int prepare_bitslice(const HotArgs &a, int num_sms);
 int prepare_bitslice16(const HotArgs &a, int num_sms);
+int prepare_bitslice_ru(const HotArgs &a, int num_sms);
 int bitslice_tmem_columns(const HotArgs &a);
 int bitslice_pairs_per_launch(const HotArgs &a, int num_sms, int max_pairs);
 // force the (lazily loaded) kernels of each translation unit into the context

@@ -70,7 +70,9 @@ struct sm_ctx {
     bool have_web = false;
     // frame-sized 16-bit arrays: sm_bands_run16's results, sm_download_web_u16's narrowed web
     uint16_t *best16 = nullptr, *web16 = nullptr;
+    uint16_t *ru16 = nullptr;  // sm_bands_run_ru16's runner-up scores
     bool prepared16 = false;  // the 16-bit bit-sliced kernels of this geometry are loaded (prepare_bitslice16)
+    int occ_ru = 0;           // ... the runner-up kernels (prepare_bitslice_ru; 0: not yet): their resident warps per SM
     int32_t *web2 = nullptr, *tmp = nullptr;  // step 3 ping-pong
     const int32_t *web_filled = nullptr;      // result of fill_web_holes (may alias web)
     bool have_web2 = false;
@@ -117,6 +119,7 @@ struct sm_ctx {
         uint8_t *web8[NPIPE] = {nullptr, nullptr, nullptr};   // [group][npix], only for the u8 result
         // the 16-bit results, written by the hot path itself ([group][npix]; best16 only when the caller wants best)
         uint16_t *web16[NPIPE] = {nullptr, nullptr, nullptr}, *best16[NPIPE] = {nullptr, nullptr, nullptr};
+        uint16_t *ru16[NPIPE] = {nullptr, nullptr, nullptr};  // the runner-up scores, only when the caller wants them
         cudaEvent_t ev_up[NPIPE] = {nullptr, nullptr, nullptr}, ev_comp[NPIPE] = {nullptr, nullptr, nullptr},
                     ev_down[NPIPE] = {nullptr, nullptr, nullptr};
     } pipe;
@@ -218,15 +221,17 @@ int copy_band_d2h(sm_ctx *c, T *host, const T *dev)
     return SM_OK;
 }
 
-// Where a hot-path call writes best / web: int32 arrays, or (web16 set) 16-bit ones, best16 possibly NULL.
+// Where a hot-path call writes best / web: int32 arrays, or (web16 set) 16-bit ones, best16 possibly NULL.  With
+// 16-bit ones, runner_up (if set) receives the runner-up scores (the runner-up kernels).
 struct Outputs {
     int32_t *best = nullptr, *web = nullptr;
     uint16_t *best16 = nullptr, *web16 = nullptr;
+    uint16_t *runner_up = nullptr;
     // pair k of a batch: every array k * stride elements further
     Outputs pair(size_t k, size_t stride) const
     {
         auto at = [&](auto *p) { return p ? p + k * stride : p; };
-        return {at(best), at(web), at(best16), at(web16)};
+        return {at(best), at(web), at(best16), at(web16), at(runner_up)};
     }
 };
 
@@ -256,8 +261,21 @@ int hot_kernel(const sm_ctx *c)
 // its 16-bit family registers): a 16-bit call without a best of the caller's gives it a scratch array.
 bool stores_best(const sm_ctx *c) { return hot_kernel(c) == SM_KERNEL_BITSLICE; }
 
-// The main kernel: of the 16-bit family with out16, else of the int32 one.
-int launch_main(sm_ctx *c, const HotArgs &a, bool out16, cudaStream_t st)
+// Loads the runner-up kernels of the context's geometry (once); their resident warps per SM go to c->occ_ru.
+int prepare_ru(sm_ctx *c)
+{
+    if (c->occ_ru > 0) return SM_OK;
+    int occ = c->occ;
+    if (hot_kernel(c) == SM_KERNEL_BITSLICE && bitslice_supports(c->half, c->D)) {
+        occ = prepare_bitslice_ru(hot_args(c, Outputs{}), c->num_sms);
+        if (occ < 0) return occ;
+    }
+    c->occ_ru = occ > 0 ? occ : 1;
+    return SM_OK;
+}
+
+// The main kernel: of the runner-up family with runner_up, of the 16-bit one with out16, else of the int32 one.
+int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cudaStream_t st)
 {
     const int k = hot_kernel(c);
     if (k == SM_KERNEL_BITSLICE) {
@@ -265,17 +283,23 @@ int launch_main(sm_ctx *c, const HotArgs &a, bool out16, cudaStream_t st)
             set_error("bit-sliced kernel does not cover square_width %d / num_shifts %d", c->sw, c->D);
             return SM_ERR_ARG;
         }
-        if (out16 && !c->prepared16) {  // (sm_create prepared the int32 family)
+        if (out16 && !runner_up && !c->prepared16) {  // (sm_create prepared the int32 family)
             const int rc = prepare_bitslice16(hot_args(c, Outputs{}), c->num_sms);
             if (rc < 0) return rc;
             c->prepared16 = true;
         }
+        if (runner_up) {
+            const int rc = prepare_ru(c);
+            if (rc < 0) return rc;
+        }
         LaunchRecord rec;
-        const int rc = out16 ? launch_bitslice16(a, c->num_sms, st, &rec) : launch_bitslice(a, c->num_sms, st, &rec);
+        const int rc = runner_up ? launch_bitslice_ru(a, runner_up, c->num_sms, st, &rec)
+                       : out16   ? launch_bitslice16(a, c->num_sms, st, &rec)
+                                 : launch_bitslice(a, c->num_sms, st, &rec);
         if (rc >= 0) c->last_launch = rec;
         return rc;
     }
-    const int rc = launch_direct(a, st, out16);
+    const int rc = launch_direct(a, st, out16, runner_up);
     if (rc >= 0) {
         c->last_launch.shape = SM_SHAPE_DIRECT;
         c->last_launch.row_runs = 0;
@@ -307,7 +331,7 @@ int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, const Outputs &out)
     // per-kernel profile put an event in between: the main kernel may start as its programmatic dependent.
     // (It waits for every earlier grid of the stream to complete before it reads anything, whatever that grid is.)
     a.after_pack = pe == nullptr && !no_pdl;
-    rc = launch_main(c, a, out.web16 != nullptr, c->stream);
+    rc = launch_main(c, a, out.web16 != nullptr, out.runner_up, c->stream);
     if (rc < 0) return rc;
     launches += rc;
     SM_CUDA(cudaEventRecord(c->ev1, c->stream));
@@ -336,7 +360,8 @@ void profile_free(sm_ctx *c)
 extern "C" const char *sm_last_error(void) { return g_err; }
 
 // 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out;
-// 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS; then, additive, the 16-bit result entries (*16, sm_download_web_u16)
+// 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS; then, additive, the 16-bit result entries (*16, sm_download_web_u16),
+// the search-range creators (*_range) and the runner-up entries (*_ru16)
 extern "C" int sm_version(void) { return (1 << 16) | 3; }
 
 extern "C" int sm_device_count(void)
@@ -503,7 +528,7 @@ extern "C" int sm_destroy(sm_ctx *c)
         }
     for (int k = 0; k < sm_ctx::NPIPE; k++) {
         void *pp[] = {c->pipe.img[k], c->pipe.edg[k], c->pipe.web[k], c->pipe.best[k], c->pipe.web8[k],
-                      c->pipe.web16[k], c->pipe.best16[k]};
+                      c->pipe.web16[k], c->pipe.best16[k], c->pipe.ru16[k]};
         for (void *p : pp)
             if (p) cudaFree(p);
         for (cudaEvent_t e : {c->pipe.ev_up[k], c->pipe.ev_comp[k], c->pipe.ev_down[k]})
@@ -514,7 +539,7 @@ extern "C" int sm_destroy(sm_ctx *c)
     void *ptrs[] = {c->img_u8[0], nullptr,      c->img_f64[0], c->img_f64[1], c->edges[0], nullptr,  // [1] = [0] + npix
                     c->best,      c->web,       c->web2,       c->tmp,        c->out,      c->minmax,
                     c->LA,        c->LB,        c->RB,         c->scratch_u8, c->scratch_i32,
-                    c->best16,    c->web16};
+                    c->best16,    c->web16,     c->ru16};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->prof_ev) profile_free(c);
@@ -800,6 +825,18 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
     // the kernel may have been switched since the last call (sm_set_kernel): the literal kernel takes one pair
     // per launch, the bit-sliced one a group
     c->batch_group = kk == SM_KERNEL_BITSLICE ? c->batch_group_cap : 1;
+    if (out.runner_up && kk == SM_KERNEL_BITSLICE) {
+        // the runner-up kernels may hold fewer warps per SM than the int32 ones the group was sized for: the pairs
+        // per launch of their own (never more than the plane sets hold)
+        int rc;
+        if ((rc = prepare_ru(c)) < 0) return rc;
+        if (c->occ_ru != c->occ) {
+            HotArgs a = hot_args(c, out);
+            a.blocks_per_sm = c->occ_ru;
+            const int g = bitslice_pairs_per_launch(a, c->num_sms, c->batch_group_cap);
+            c->batch_group = g < c->batch_group_cap ? g : c->batch_group_cap;
+        }
+    }
     const int G = c->batch_group;
     // everything queued on the context's stream so far (the producers of the edge maps) comes first
     SM_CUDA(cudaEventRecord(c->ev0, c->stream));
@@ -841,7 +878,7 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         a.npairs = np;
         a.plane_stride = pw;
         a.out_stride = out_stride;
-        rc = launch_main(c, a, o.web16 != nullptr, ms);
+        rc = launch_main(c, a, o.web16 != nullptr, o.runner_up, ms);
         if (rc < 0) return rc;
         launches += rc;
         if (pe) {
@@ -879,6 +916,18 @@ extern "C" int sm_match_wta_dev_batch16(sm_ctx *c, int n_pairs, const uint8_t *d
     SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch16: stride below frame size");
     return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, {nullptr, nullptr, d_best, d_web},
                       out_stride);
+}
+
+extern "C" int sm_match_wta_dev_batch_ru16(sm_ctx *c, int n_pairs, const uint8_t *d_first_edges,
+                                           const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best,
+                                           uint16_t *d_web, uint16_t *d_runner_up, size_t out_stride)
+{
+    SM_REQUIRE(n_pairs >= 0 && d_first_edges && d_second_edges && d_web && d_runner_up,
+               "sm_match_wta_dev_batch_ru16: bad arguments");
+    SM_ENTER(c);
+    SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch_ru16: stride below frame size");
+    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride,
+                      {nullptr, nullptr, d_best, d_web, d_runner_up}, out_stride);
 }
 
 extern "C" int sm_elapsed_ms(sm_ctx *c, float *ms)
@@ -1132,12 +1181,14 @@ enum WebFormat { WEB_I32, WEB_U8, WEB_U16 };
 static size_t web_bytes(WebFormat f) { return f == WEB_U8 ? 1 : (f == WEB_U16 ? 2 : 4); }
 static size_t best_bytes(WebFormat f) { return f == WEB_U16 ? 2 : 4; }
 
-// sm_run_batch / sm_run_batch16 (fn: the entry's name, for the messages)
+// sm_run_batch / sm_run_batch16 / sm_run_batch_ru16 (fn: the entry's name, for the messages; ru_out: the runner-up
+// scores, WEB_U16 only)
 static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
-                     double threshold, WebFormat fmt, void *web_out, void *best_out)
+                     double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
 {
     SM_ENTER(c);
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
+    SM_REQUIRE(!ru_out || fmt == WEB_U16, "%s: the runner-up needs 16-bit results", fn);
     SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "%s: whole-frame contexts only", fn);
     SM_REQUIRE(fmt != WEB_U8 || c->M + c->D <= 255, "%s: u8 web needs min_shift + num_shifts <= 255", fn);
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "%s: threshold must be between 0 and 1", fn);
@@ -1166,7 +1217,8 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
     // the caller wants it, best
     for (int k = 0; k < NP; k++) {
         if (fmt == WEB_U16) {
-            if ((rc = dev_alloc(&P.web16[k], P.group * n)) || (best_out && (rc = dev_alloc(&P.best16[k], P.group * n))))
+            if ((rc = dev_alloc(&P.web16[k], P.group * n)) || (best_out && (rc = dev_alloc(&P.best16[k], P.group * n))) ||
+                (ru_out && (rc = dev_alloc(&P.ru16[k], P.group * n))))
                 return rc;
         } else if ((rc = dev_alloc(&P.web[k], P.group * n)) || (rc = dev_alloc(&P.best[k], P.group * n))) {
             return rc;
@@ -1196,7 +1248,8 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
         SM_CUDA(cudaEventRecord(P.ev_up[b], P.up));
         // ---- stage 2, the context's stream: edges of all 2*np images, then the batched hot path
         SM_CUDA(cudaStreamWaitEvent(c->stream, P.ev_up[b], 0));
-        const Outputs out = fmt == WEB_U16 ? Outputs{nullptr, nullptr, best_out ? P.best16[b] : nullptr, P.web16[b]}
+        const Outputs out = fmt == WEB_U16 ? Outputs{nullptr, nullptr, best_out ? P.best16[b] : nullptr, P.web16[b],
+                                                     ru_out ? P.ru16[b] : nullptr}
                                            : Outputs{P.best[b], P.web[b]};
         if (use_lut) {
             // edges of all 2*np images straight into the packed planes, then the hot path: two kernels per group
@@ -1230,6 +1283,9 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
         if (best_out)
             SM_CUDA(cudaMemcpyAsync((uint8_t *)best_out + (size_t)k * n * bb, best_dev, (size_t)np * n * bb,
                                     cudaMemcpyDeviceToHost, P.down));
+        if (ru_out)
+            SM_CUDA(cudaMemcpyAsync(ru_out + (size_t)k * n, P.ru16[b], (size_t)np * n * sizeof(uint16_t),
+                                    cudaMemcpyDeviceToHost, P.down));
         SM_CUDA(cudaEventRecord(P.ev_down[b], P.down));
     }
     SM_CUDA(cudaStreamSynchronize(P.up));
@@ -1252,6 +1308,15 @@ extern "C" int sm_run_batch16(sm_ctx *c, int n_pairs, const uint8_t *first, cons
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "sm_run_batch16: bad arguments");
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch16: threshold must be between 0 and 1");
     return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out);
+}
+
+extern "C" int sm_run_batch_ru16(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                 double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out)
+{
+    // the checks that need no context first (and no device)
+    SM_REQUIRE(n_pairs >= 0 && first && second && web_out && runner_up_out, "sm_run_batch_ru16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch_ru16: threshold must be between 0 and 1");
+    return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
 }
 
 // ---- whole pairs over several GPUs of one box ------------------------------------------------
@@ -1391,9 +1456,9 @@ extern "C" int sm_multi_destroy(sm_multi *m)
 
 extern "C" int sm_multi_device_count(const sm_multi *m) { return m ? m->n : SM_ERR_ARG; }
 
-// sm_multi_run_batch / sm_multi_run_batch16
+// sm_multi_run_batch / sm_multi_run_batch16 / sm_multi_run_batch_ru16
 static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
-                           double threshold, WebFormat fmt, void *web_out, void *best_out)
+                           double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
 {
     SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     const int N = m->n;
@@ -1405,8 +1470,9 @@ static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8
         if (k1 <= k0) return;
         void *wout = (uint8_t *)web_out + (size_t)k0 * n * wb;
         void *bout = best_out ? (void *)((uint8_t *)best_out + (size_t)k0 * n * bb) : nullptr;
+        uint16_t *rout = ru_out ? ru_out + (size_t)k0 * n : nullptr;
         rcs[(size_t)d] = run_batch(fn, m->ctx[d], k1 - k0, first + (size_t)k0 * n, second + (size_t)k0 * n, threshold, fmt,
-                                   wout, bout);
+                                   wout, bout, rout);
         if (rcs[(size_t)d]) errs[(size_t)d] = sm_last_error();  // the message is per thread: carry it to the caller's
     };
     if (m->workers)
@@ -1431,6 +1497,15 @@ extern "C" int sm_multi_run_batch16(sm_multi *m, int n_pairs, const uint8_t *fir
                                     double threshold, uint16_t *web_out, uint16_t *best_out)
 {
     return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out);
+}
+
+extern "C" int sm_multi_run_batch_ru16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                       double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out)
+{
+    // the checks that need no handle first (and no device)
+    SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out && runner_up_out, "sm_multi_run_batch_ru16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_multi_run_batch_ru16: threshold must be between 0 and 1");
+    return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
 }
 
 // ---- one pair, row bands over several GPUs of one box ----------------------------------------------
@@ -1497,24 +1572,28 @@ extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices
 }
 
 // One band context's 16-bit run: the hot path writes rows [row0, row1) of the context's frame-sized u16 arrays
-// (best16 when the caller wants best or the kernel stores it anyway); only those rows are downloaded.
-static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out)
+// (best16 when the caller wants best or the kernel stores it anyway; ru16 with ru_out); only those rows are downloaded.
+static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out, uint16_t *ru_out)
 {
     SM_ENTER(c);
     int rc;
     const bool with_best = best_out || stores_best(c);
-    if ((rc = dev_alloc(&c->web16, c->npix())) || (with_best && (rc = dev_alloc(&c->best16, c->npix())))) return rc;
-    if ((rc = run_hot(c, c->edges[0], c->edges[1], {nullptr, nullptr, with_best ? c->best16 : nullptr, c->web16})))
+    if ((rc = dev_alloc(&c->web16, c->npix())) || (with_best && (rc = dev_alloc(&c->best16, c->npix()))) ||
+        (ru_out && (rc = dev_alloc(&c->ru16, c->npix()))))
         return rc;
-    if ((rc = copy_band_d2h(c, web_out, c->web16)) || (best_out && (rc = copy_band_d2h(c, best_out, c->best16))))
+    if ((rc = run_hot(c, c->edges[0], c->edges[1],
+                      {nullptr, nullptr, with_best ? c->best16 : nullptr, c->web16, ru_out ? c->ru16 : nullptr})))
+        return rc;
+    if ((rc = copy_band_d2h(c, web_out, c->web16)) || (best_out && (rc = copy_band_d2h(c, best_out, c->best16))) ||
+        (ru_out && (rc = copy_band_d2h(c, ru_out, c->ru16))))
         return rc;
     SM_CUDA(cudaStreamSynchronize(c->stream));
     return SM_OK;
 }
 
-// sm_bands_run / sm_bands_run16
+// sm_bands_run / sm_bands_run16 / sm_bands_run_ru16
 static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
-                     WebFormat fmt, void *web_out, void *best_out)
+                     WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
 {
     SM_REQUIRE(b && first && second && web_out, "%s: bad arguments", fn);
     const int N = b->n;
@@ -1525,7 +1604,7 @@ static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const ui
         int rc = sm_upload_u8(c, first, second);  // a band context copies only the rows it needs
         if (!rc) rc = sm_edges(c, threshold);
         if (fmt == WEB_U16) {
-            if (!rc) rc = band_run16(c, (uint16_t *)web_out, (uint16_t *)best_out);
+            if (!rc) rc = band_run16(c, (uint16_t *)web_out, (uint16_t *)best_out, ru_out);
         } else {
             if (!rc) rc = sm_match_wta(c);
             if (!rc) rc = sm_download(c, SM_WEB, 0, web_out);  // ... and writes only its own rows
@@ -1556,4 +1635,12 @@ extern "C" int sm_bands_run16(sm_bands *b, const uint8_t *first, const uint8_t *
                               uint16_t *web_out, uint16_t *best_out)
 {
     return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out);
+}
+
+extern "C" int sm_bands_run_ru16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                                 uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out)
+{
+    SM_REQUIRE(b && first && second && web_out && runner_up_out, "sm_bands_run_ru16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_bands_run_ru16: threshold must be between 0 and 1");
+    return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
 }

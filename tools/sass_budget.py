@@ -2,10 +2,11 @@
 """tools/sass_budget.py -- static ALU-pipe budget of the hot kernel's two steady blocks, from the SASS of the built
 library (no GPU, no profiler).
 
-    python tools/sass_budget.py [--lib stereomatching_b200/libstereo_b200.so] [--kernel 4,2,16,0,0,0] [--json]
+    python tools/sass_budget.py [--lib stereomatching_b200/libstereo_b200.so] [--kernel 4,2,16,0,0,0]
+                                [--family k_bitslice|k_bitslice16|k_bitslice_ru] [--json]
 
-`--kernel` names a k_bitslice instantiation by its template arguments HALF,NW,SEG,MULTI,C2,HP (default: config 2,
-window 9, 64 shifts).  The SASS (`cuobjdump -sass`) is cut into basic blocks; of those,
+`--kernel` names an instantiation by its template arguments HALF,NW,SEG,MULTI,C2,HP (default: config 2,
+window 9, 64 shifts), `--family` the output family (default: k_bitslice, the int32 one).  The SASS (`cuobjdump -sass`) is cut into basic blocks; of those,
   - pass A is the steady walk: among the blocks with the most STS (one per H word and centre word of a walk),
     the one with the fewest ALU-pipe instructions (the VALID_ALL walk, without the validity selects);
   - pass B is the steady block: the largest block that reads tensor memory (LDTM), RB rows x NW words.
@@ -35,8 +36,12 @@ def bits_for(v):
     return b
 
 
-def mangled(half, nw, seg, multi, c2, hp):
-    return "k_bitsliceILi%dELi%dELi%dELb%dELb%dELb%dE" % (half, nw, seg, multi, c2, hp)
+FAMILIES = ("k_bitslice", "k_bitslice16", "k_bitslice_ru")
+
+
+def mangled(half, nw, seg, multi, c2, hp, family="k_bitslice"):
+    return "%dk_bitslice" % len(family) + family[len("k_bitslice"):] + \
+        "ILi%dELi%dELi%dELb%dELb%dELb%dE" % (half, nw, seg, multi, c2, hp)
 
 
 def opcode(text):
@@ -91,9 +96,9 @@ def classes(ops):
             "alu_ops": dict(sorted(((k, v) for k, v in ops.items() if k in ALU), key=lambda kv: -kv[1]))}
 
 
-def budget(lib, args):
+def budget(lib, args, family="k_bitslice"):
     half, nw, seg, multi, c2, hp = args
-    blocks = basic_blocks(function_sass(lib, mangled(*args)))
+    blocks = basic_blocks(function_sass(lib, mangled(*args, family=family)))
     most_sts = max(b["STS"] for b in blocks)
     alu = lambda b: sum(v for k, v in b.items() if k in ALU)  # noqa: E731
     pass_a = min((b for b in blocks if b["STS"] == most_sts), key=alu)
@@ -102,7 +107,7 @@ def budget(lib, args):
     strip_cols = 32 * (2 if hp else 1) * (nw if c2 else 1)
     pixels = rb * strip_cols
     a, b = classes(pass_a), classes(pass_b)
-    return {"kernel": "k_bitslice<%s>" % ",".join(map(str, args)), "library": lib,
+    return {"kernel": "%s<%s>" % (family, ",".join(map(str, args))), "library": lib,
             "planes": {"KH": bits_for(2 * half + 1), "PV": bits_for((2 * half + 1) ** 2)},
             "pixels_per_warp_block": pixels, "pass_a": a, "pass_b": b,
             "alu_per_pixel": {"pass_a": 32.0 * a["alu"] / pixels, "pass_b": 32.0 * b["alu"] / pixels,
@@ -114,9 +119,10 @@ def main():
     ap.add_argument("--lib", default=os.path.join(ROOT, "stereomatching_b200", "libstereo_b200.so"),
                     help="built library or cubin")
     ap.add_argument("--kernel", default="4,2,16,0,0,0", help="HALF,NW,SEG,MULTI,C2,HP")
+    ap.add_argument("--family", default="k_bitslice", choices=FAMILIES, help="output family")
     ap.add_argument("--json", action="store_true", help="print the result as JSON")
     o = ap.parse_args()
-    r = budget(o.lib, tuple(int(x) for x in o.kernel.split(",")))
+    r = budget(o.lib, tuple(int(x) for x in o.kernel.split(",")), o.family)
     if o.json:
         json.dump(r, sys.stdout, indent=1)
         print()
