@@ -118,8 +118,9 @@ const char *sm_last_error(void);
 /* ABI version: (major << 16) | minor.  The 16-bit result entries (sm_match_wta_dev_batch16, sm_run_batch16,
  * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16), the search-range creators (sm_create_range,
  * sm_create_band_range, sm_multi_create_range, sm_bands_create_range) and the runner-up entries
- * (sm_match_wta_dev_batch_ru16, sm_run_batch_ru16, sm_multi_run_batch_ru16, sm_bands_run_ru16) are additions to 1.3
- * that leave every other entry as it was; clients detect them by symbol. */
+ * (sm_match_wta_dev_batch_ru16, sm_run_batch_ru16, sm_multi_run_batch_ru16, sm_bands_run_ru16) and the sub-pixel
+ * entries (sm_match_wta_dev_batch_sub16, sm_run_batch_sub16, sm_multi_run_batch_sub16, sm_bands_run_sub16) are
+ * additions to 1.3 that leave every other entry as it was; clients detect them by symbol. */
 int sm_version(void);
 /* Number of CUDA devices visible, or a negative sm_status. */
 int sm_device_count(void);
@@ -242,6 +243,24 @@ int sm_match_wta_dev_batch_ru16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first
                                 const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best, uint16_t *d_web,
                                 uint16_t *d_runner_up, size_t out_stride);
 
+/* The same (best / web exactly those of sm_match_wta_dev_batch16), and each pixel's web in SIXTEENTHS of a shift,
+ * interpolated by the hot kernel from the scores next to the winner (the fixed-point format of OpenCV's block
+ * matchers, 4 fractional bits).  With the context's range [m, m + D), s(t) the masked score at shift t (the value
+ * the winner-take-all maximises: the box sum where the centre matched, else 0) and w = web - 1 the winning shift:
+ *   - w == m or w == m + D - 1 (no neighbour inside the range; also D == 1 and pixels whose scores are all 0):
+ *     frac = 0;
+ *   - else s- = s(w - 1), s+ = s(w + 1), den = 2 * best - s- - s+ (>= 1: ties go to the highest shift) and
+ *     frac = min(7, floor((16 * (s+ - s-) + den) / (2 * den))), the vertex of the parabola through the three scores
+ *     in sixteenths, rounded half up, in [-8, 7];
+ *   - web_sub = 16 * web + frac.  So web_sub / 16 is a refined web and web_sub / 16 - 1 the disparity in pixels;
+ *     (web_sub + 8) >> 4 == web and web_sub >= 16 * (m + 1) - 8 > 0 everywhere.
+ * Integer arithmetic on exact counts: bit-exact.  Needs m + D <= 4095 (web_sub fits 16 bits), else SM_ERR_ARG
+ * before any device call.  d_web_sub (not NULL) takes pair k at k * out_stride, like d_web; 2 B per pixel.  d_best
+ * may be NULL. */
+int sm_match_wta_dev_batch_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edges,
+                                 const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best, uint16_t *d_web,
+                                 uint16_t *d_web_sub, size_t out_stride);
+
 /* Device time of the last sm_match_wta* call on this context, CUDA events on the
  * context's stream (the reference brackets the whole algorithm() with
  * CLOCK_MONOTONIC instead, stereo.cu:308,334-335).  Waits for the call to finish. */
@@ -307,6 +326,10 @@ int sm_run_batch16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t
  * frames of u16, one more copy per group. */
 int sm_run_batch_ru16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                       uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
+/* The same and web_sub (see sm_match_wta_dev_batch_sub16) into web_sub_out (not NULL): n_pairs frames of u16, one
+ * more copy per group.  min_shift + num_shifts <= 4095. */
+int sm_run_batch_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                       uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
 
 /* The same over several GPUs of one box (SURVEY 8e, BASELINE config 4: whole pairs sharded across the
  * GPUs, inputs scattered from the host, no cross-device traffic): one context and one host thread per
@@ -325,6 +348,9 @@ int sm_multi_run_batch16(sm_multi *m, int n_pairs, const uint8_t *first, const u
 /* The same through sm_run_batch_ru16 (runner_up_out not NULL). */
 int sm_multi_run_batch_ru16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                             uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
+/* The same through sm_run_batch_sub16 (web_sub_out not NULL). */
+int sm_multi_run_batch_sub16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                             uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
 int sm_multi_device_count(const sm_multi *m);
 int sm_multi_destroy(sm_multi *m);
 
@@ -348,6 +374,10 @@ int sm_bands_run16(sm_bands *b, const uint8_t *first, const uint8_t *second, dou
  * frame-sized runner_up_out (not NULL). */
 int sm_bands_run_ru16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                       uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out);
+/* The same and web_sub (see sm_match_wta_dev_batch_sub16): each band writes its own rows of the frame-sized
+ * web_sub_out (not NULL). */
+int sm_bands_run_sub16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                       uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
 int sm_bands_destroy(sm_bands *b);
 
 /* ---- geometry helpers (host-side, no GPU) --------------------------------------- */

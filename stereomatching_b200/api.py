@@ -42,6 +42,7 @@ SYMBOLS = [
     "sm_bands_create", "sm_bands_run", "sm_bands_run16", "sm_bands_destroy",
     "sm_create_range", "sm_create_band_range", "sm_multi_create_range", "sm_bands_create_range",
     "sm_match_wta_dev_batch_ru16", "sm_run_batch_ru16", "sm_multi_run_batch_ru16", "sm_bands_run_ru16",
+    "sm_match_wta_dev_batch_sub16", "sm_run_batch_sub16", "sm_multi_run_batch_sub16", "sm_bands_run_sub16",
 ]
 
 
@@ -84,6 +85,7 @@ def lib() -> C.CDLL:
         L.sm_match_wta_dev_batch.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
         L.sm_match_wta_dev_batch16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
         L.sm_match_wta_dev_batch_ru16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t]
+        L.sm_match_wta_dev_batch_sub16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t]
         L.sm_elapsed_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.sm_last_launches.argtypes = [vp]
         L.sm_profile_begin.argtypes = [vp, i]
@@ -97,12 +99,14 @@ def lib() -> C.CDLL:
         L.sm_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
         L.sm_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
+        L.sm_run_batch_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_band_rows.argtypes = [i, i, i, C.POINTER(i), C.POINTER(i)]
         L.sm_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_multi_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
         L.sm_multi_run_batch.argtypes = [vp, i, vp, vp, d, vp, i, vp]
         L.sm_multi_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_multi_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
+        L.sm_multi_run_batch_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_multi_device_count.argtypes = [vp]
         L.sm_multi_destroy.argtypes = [vp]
         L.sm_bands_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
@@ -110,6 +114,7 @@ def lib() -> C.CDLL:
         L.sm_bands_run.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_run16.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_run_ru16.argtypes = [vp, vp, vp, d, vp, vp, vp]
+        L.sm_bands_run_sub16.argtypes = [vp, vp, vp, d, vp, vp, vp]
         L.sm_bands_destroy.argtypes = [vp]
         _lib = L
     return _lib
@@ -260,6 +265,15 @@ class StereoContext:
                                                  C.c_void_p(d_second_edges), edge_stride, C.c_void_p(d_best or None),
                                                  C.c_void_p(d_web), C.c_void_p(d_runner_up), out_stride))
 
+    def match_wta_dev_batch_sub16(self, n_pairs: int, d_first_edges: int, d_second_edges: int, edge_stride: int,
+                                  d_best, d_web: int, d_web_sub: int, out_stride: int):
+        """match_wta_dev_batch16 that also writes each pixel's web in sixteenths of a shift (16 * web + frac, frac in
+        [-8, 7] from a parabola through the scores next to the winner; see the C header) to d_web_sub, uint16 with the
+        web's pair stride.  min_shift + num_shifts <= 4095."""
+        _check(lib().sm_match_wta_dev_batch_sub16(self._c, n_pairs, C.c_void_p(d_first_edges),
+                                                  C.c_void_p(d_second_edges), edge_stride, C.c_void_p(d_best or None),
+                                                  C.c_void_p(d_web), C.c_void_p(d_web_sub), out_stride))
+
     def elapsed_ms(self) -> float:
         ms = C.c_float()
         _check(lib().sm_elapsed_ms(self._c, C.byref(ms)))
@@ -312,16 +326,18 @@ class StereoContext:
         return out
 
     def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False,
-                  want_runner_up=False):
+                  want_runner_up=False, want_subpixel=False):
         """first/second: (n, H, W) u8.  Returns web (n, H, W) [and best]: int32, web as uint8 with web_u8, or (web16)
         both as uint16, written by the hot kernel itself.  want_runner_up (web16 only): also each pixel's runner-up
-        score, uint16, last in the result: (web, [best], runner_up)."""
+        score, uint16, last in the result: (web, [best], runner_up).  want_subpixel (web16 only, not with
+        want_runner_up): also web_sub, the web in sixteenths of a shift, uint16, last: (web, [best], web_sub)."""
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
         return _run_batch(self._c, lib().sm_run_batch, lib().sm_run_batch16, lib().sm_run_batch_ru16, first, second,
-                          threshold, web_u8, want_best, web_out, web16, want_runner_up)
+                          threshold, web_u8, want_best, web_out, web16, want_runner_up, lib().sm_run_batch_sub16,
+                          want_subpixel)
 
     # -- convenience: the reference's whole step 2 on host edge maps -----------
     def match_wta_host(self, first_edges, second_edges):
@@ -330,14 +346,22 @@ class StereoContext:
         return self.download(BEST), self.download(WEB)
 
 
-def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, want_best, web_out, web16,
-               want_runner_up=False):
-    """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16), or with want_runner_up
-    their runner-up entries (run_ru)."""
-    if web16 and web_u8:
-        raise ValueError("web16 and web_u8 exclude each other")
+def _check_extras(web16, want_runner_up, want_subpixel):
     if want_runner_up and not web16:
         raise ValueError("want_runner_up needs web16=True (the runner-up comes with 16-bit results only)")
+    if want_subpixel and not web16:
+        raise ValueError("want_subpixel needs web16=True (web_sub comes with 16-bit results only)")
+    if want_subpixel and want_runner_up:
+        raise ValueError("want_subpixel and want_runner_up exclude each other")
+
+
+def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, want_best, web_out, web16,
+               want_runner_up=False, run_sub=None, want_subpixel=False):
+    """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16), or with want_runner_up
+    their runner-up entries (run_ru), or with want_subpixel their sub-pixel entries (run_sub)."""
+    if web16 and web_u8:
+        raise ValueError("web16 and web_u8 exclude each other")
+    _check_extras(web16, want_runner_up, want_subpixel)
     n, H, W = first.shape
     dt = np.uint16 if web16 else (np.uint8 if web_u8 else np.int32)
     if web_out is None:
@@ -349,6 +373,11 @@ def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, wan
         _check(run_ru(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None,
                       _ptr(ru)))
         return (web_out, best, ru) if want_best else (web_out, ru)
+    if want_subpixel:
+        ws = np.zeros((n, H, W), np.uint16)
+        _check(run_sub(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None,
+                       _ptr(ws)))
+        return (web_out, best, ws) if want_best else (web_out, ws)
     if web16:
         _check(run16(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None))
     else:
@@ -370,13 +399,14 @@ class MultiGpuBatch:
                                            square_width, variant))
 
     def run_batch(self, first, second, threshold=0.15, web_u8=False, want_best=False, web_out=None, web16=False,
-                  want_runner_up=False):
+                  want_runner_up=False, want_subpixel=False):
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         n = first.shape[0]
         assert first.shape == second.shape == (n, self.H, self.W)
         return _run_batch(self._m, lib().sm_multi_run_batch, lib().sm_multi_run_batch16, lib().sm_multi_run_batch_ru16,
-                          first, second, threshold, web_u8, want_best, web_out, web16, want_runner_up)
+                          first, second, threshold, web_u8, want_best, web_out, web16, want_runner_up,
+                          lib().sm_multi_run_batch_sub16, want_subpixel)
 
     def close(self):
         if self._m:
@@ -401,11 +431,12 @@ class MultiGpuBands:
         _check(lib().sm_bands_create_range(C.byref(self._b), arr, len(devices), width, height, min_shift, num_shifts,
                                            square_width, variant))
 
-    def run(self, first, second, threshold=0.15, want_best=False, web16=False, want_runner_up=False):
+    def run(self, first, second, threshold=0.15, want_best=False, web16=False, want_runner_up=False,
+            want_subpixel=False):
         """web [and best] of one pair: int32, or uint16 with web16; want_runner_up (web16 only): also the runner-up
-        scores, uint16, last in the result: (web, [best], runner_up)."""
-        if want_runner_up and not web16:
-            raise ValueError("want_runner_up needs web16=True (the runner-up comes with 16-bit results only)")
+        scores, uint16, last in the result: (web, [best], runner_up); want_subpixel (web16 only, not with
+        want_runner_up): web_sub instead, the web in sixteenths of a shift: (web, [best], web_sub)."""
+        _check_extras(web16, want_runner_up, want_subpixel)
         first = np.ascontiguousarray(first, np.uint8)
         second = np.ascontiguousarray(second, np.uint8)
         assert first.shape == second.shape == (self.H, self.W)
@@ -417,6 +448,11 @@ class MultiGpuBands:
             _check(lib().sm_bands_run_ru16(self._b, _ptr(first), _ptr(second), threshold, _ptr(web),
                                            _ptr(best) if want_best else None, _ptr(ru)))
             return (web, best, ru) if want_best else (web, ru)
+        if want_subpixel:
+            ws = np.zeros((self.H, self.W), np.uint16)
+            _check(lib().sm_bands_run_sub16(self._b, _ptr(first), _ptr(second), threshold, _ptr(web),
+                                            _ptr(best) if want_best else None, _ptr(ws)))
+            return (web, best, ws) if want_best else (web, ws)
         run = lib().sm_bands_run16 if web16 else lib().sm_bands_run
         _check(run(self._b, _ptr(first), _ptr(second), threshold, _ptr(web), _ptr(best) if want_best else None))
         return (web, best) if want_best else web

@@ -1,7 +1,8 @@
-// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its three output families:
-// k_bitslice (int32 best / web, k_bitslice.cu), k_bitslice16 (uint16_t, k_bitslice16.cu) and k_bitslice_ru (uint16_t
-// and the runner-up score, k_bitslice_ru.cu).  Each translation unit instantiates one family through dispatch, so
-// that the three compile in parallel.
+// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its four output families:
+// k_bitslice (int32 best / web, k_bitslice.cu), k_bitslice16 (uint16_t, k_bitslice16.cu), k_bitslice_ru (uint16_t
+// and the runner-up score, k_bitslice_ru.cu) and k_bitslice_sub (uint16_t and the web in sixteenths of a shift,
+// k_bitslice_sub.cu).  Each translation unit instantiates one family through dispatch, so that the four compile in
+// parallel.
 //
 // What it replaces: fillup_matches + 30x{memset, addup_pixels_in_square, record_score} +
 // find_highest_scoring_shifts of the reference (stereo.cu:127-225), i.e. per pixel and per
@@ -497,14 +498,117 @@ __device__ __forceinline__ void drop_one_tied(const uint32_t (&valid)[NW], const
     for (int w = 0; w < NW; w++) cand2[w] = lop3<0x78>(valid[w], cand[w], n[w]);  // x ^ (y & z)
 }
 
+// SUB (the sub-pixel family, k_bitslice_sub): the masked score of the lane set in nb (one lane of the NW words, or
+// none), NEGATED: -sum_p [V_p & M & nb != 0] << p.  One lop3.or per word and plane, the words chained through its
+// predicate output as in wta_plane; the sum is a predicated multiply-add (FMA pipe).
+template <int NW, int PV>
+__device__ __forceinline__ int sub_gather(const uint32_t (&V)[NW][PV], const uint32_t (&M)[NW], const uint32_t (&nb)[NW],
+                                          int one)
+{
+    int acc = 0;
+#pragma unroll
+    for (int p = PV - 1; p >= 0; p--) {
+        if (NW == 2) {
+            asm("{ .reg .pred q0, q; .reg .b32 t0, t1;\n\t"
+                "lop3.or.b32 t0|q0, %1, %2, %3, 0x80, 0;\n\t"
+                "lop3.or.b32 t1|q, %4, %5, %6, 0x80, q0;\n\t"
+                "@q mad.lo.s32 %0, %7, %8, %0; }"
+                : "+r"(acc)
+                : "r"(V[0][p]), "r"(M[0]), "r"(nb[0]), "r"(V[NW - 1][p]), "r"(M[NW - 1]), "r"(nb[NW - 1]), "r"(one),
+                  "r"(-(1 << p)));
+        } else {
+            asm("{ .reg .pred q; .reg .b32 t0;\n\t"
+                "lop3.or.b32 t0|q, %1, %2, %3, 0x80, 0;\n\t"
+                "@q mad.lo.s32 %0, %4, %5, %0; }"
+                : "+r"(acc) : "r"(V[0][p]), "r"(M[0]), "r"(nb[0]), "r"(one), "r"(-(1 << p)));
+        }
+    }
+    return acc;
+}
+
+// SUB: the lanes next to the winner, from its shift amount m (31 - its bit in the word, or with two words 63 - its
+// lane): nbm = lane - 1, nbp = lane + 1, empty past either end of the words.  With two words the winner's bit of each
+// word is one shift each (an empty word's amount is clamped out); the rest are multiply-adds on the FMA pipe (x * 2 is
+// x * one + x; x >> 1 and x >> 31 are the high words of x * 2^31 and x * 2).
+template <int NW>
+__device__ __forceinline__ void sub_neighbours(uint32_t m, int one, uint32_t (&nbm)[NW], uint32_t (&nbp)[NW])
+{
+    if constexpr (NW == 2) {
+        uint32_t m32;  // m - 32, a multiply-add (an immediate add is a VIADD on the ALU pipe)
+        asm("mad.lo.u32 %0, %1, %2, -32;" : "=r"(m32) : "r"(m), "r"(one));
+        const uint32_t b1 = shr_clamp(0x80000000u, m), b0 = shr_clamp(0x80000000u, m32);
+        // (the multipliers 2 and 2^31 come from `one`, opaque to ptxas: as immediates the high-word multiply-adds
+        // become LEA.HI on the ALU pipe)
+        asm("{ .reg .b32 t;\n\t"
+            "mad.lo.u32 %0, %4, %6, %4;\n\t"                 // nbp0 = b0 * 2
+            "mad.hi.u32 t, %4, %7, %5;\n\t"                  // b1 + (b0 >> 31)
+            "mad.lo.u32 %1, %5, %6, t;\n\t"                  // nbp1 = b1 * 2 + (b0 >> 31)
+            "mul.hi.u32 %3, %5, %8;\n\t"                     // nbm1 = b1 >> 1
+            "mad.lo.u32 t, %5, %8, 0;\n\t"                   // b1 << 31
+            "mad.hi.u32 %2, %4, %8, t; }"                    // nbm0 = (b0 >> 1) + (b1 << 31)
+            : "=r"(nbp[0]), "=r"(nbp[NW - 1]), "=r"(nbm[0]), "=r"(nbm[NW - 1])
+            : "r"(b0), "r"(b1), "r"(one), "r"(2 * one), "r"((uint32_t)one << 31));
+    } else {
+        const uint32_t b = shr_clamp(0x80000000u, m);
+        asm("mad.lo.u32 %0, %2, %3, %2;\n\tmul.hi.u32 %1, %2, %4;"
+            : "=r"(nbp[0]), "=r"(nbm[0]) : "r"(b), "r"(one), "r"((uint32_t)one << 31));
+    }
+}
+
+// SUB: web_sub = 16 * web + frac from the winner's masked score s0 and its neighbours' NEGATED scores nsm = -s(w - 1),
+// nsp = -s(w + 1).  frac is the largest f in [-8, 7] with (2f - 1) * den <= 16 * (s+ - s-), den = 2 * s0 - s- - s+,
+// i.e. min(7, floor((16 * (s+ - s-) + den) / (2 * den))): a 4-step search on g = (2f - 1) * den - 16 * (s+ - s-),
+// one compare per step (ISETP), everything else multiply-adds.  Where the winner is the range's first or last shift
+// (web == M + 1: c1 = -(M + 2); web == M + D: c2 = M + D - 1) den gains 2^20 - 1 (the high word of 2^20 * (2^32 - 1)),
+// far above 16 * |s+ - s-| <= 16 * 63^2, so f == 0 whatever the missing neighbour's lane held.  den >= 1 everywhere
+// else (ties go to the highest shift: s+ < s0, s- <= s0), and f >= -8 always (|s+ - s-| <= den).
+__device__ __forceinline__ int sub_frac(int s0, int nsm, int nsp, int web, int c1, int c2, int one)
+{
+    // (multipliers that are powers of two come from `one`, opaque to ptxas: with immediates it makes them LEAs, which
+    // run on the ALU pipe)
+    int ws;
+    asm("{ .reg .pred p; .reg .s32 den, d2, d4, d8, d16, g, t, y;\n\t"
+        "mad.lo.s32 den, %1, %7, %2;\n\t"           // s0 - s-
+        "mad.lo.s32 den, %1, %7, den;\n\t"          // 2 s0 - s-
+        "mad.lo.s32 den, %3, %7, den;\n\t"          // - s+
+        "mad.lo.s32 y, %4, %7, %5;\n\t"             // web - (M + 2): -1 where w == M (no s-)
+        "mad.hi.u32 den, y, %10, den;\n\t"          // + 2^20 - 1 there
+        "mad.lo.s32 y, %4, %8, %6;\n\t"             // (M + D - 1) - web: -1 where w == M + D - 1 (no s+)
+        "mad.hi.u32 den, y, %10, den;\n\t"
+        "mad.lo.s32 d2, den, %7, den;\n\t"
+        "mad.lo.s32 d4, d2, %7, d2;\n\t"
+        "mad.lo.s32 d8, d4, %7, d4;\n\t"
+        "mad.lo.s32 d16, d8, %7, d8;\n\t"
+        "mad.lo.s32 y, %2, %8, %3;\n\t"             // s- - s+
+        "mad.lo.s32 g, den, -17, 0;\n\t"
+        "mad.lo.s32 g, y, %9, g;\n\t"               // g = -17 den - 16 (s+ - s-)
+        "mad.lo.s32 %0, %4, %9, -8;\n\t"            // 16 web - 8
+        "mad.lo.s32 t, d16, %7, g;\n\tsetp.le.s32 p, t, 0;\n\t@p mad.lo.s32 g, t, %7, 0;\n\t@p mad.lo.s32 %0, %7, 8, %0;\n\t"
+        "mad.lo.s32 t, d8, %7, g;\n\tsetp.le.s32 p, t, 0;\n\t@p mad.lo.s32 g, t, %7, 0;\n\t@p mad.lo.s32 %0, %7, 4, %0;\n\t"
+        "mad.lo.s32 t, d4, %7, g;\n\tsetp.le.s32 p, t, 0;\n\t@p mad.lo.s32 g, t, %7, 0;\n\t@p mad.lo.s32 %0, %7, 2, %0;\n\t"
+        "mad.lo.s32 t, d2, %7, g;\n\tsetp.le.s32 p, t, 0;\n\t@p mad.lo.s32 %0, %7, 1, %0; }"
+        : "=r"(ws)
+        : "r"(s0), "r"(nsm), "r"(nsp), "r"(web), "r"(c1), "r"(c2), "r"(one), "r"(-one), "r"(16 * one), "r"(one << 20));
+    return ws;
+}
+
+// What the sub-pixel family's winner-take-all hands on per row (SUB).  One chunk: ws = web_sub.  MULTI: the chunk's
+// own neighbour scores of its winner (nsm / nsp, negated; 0 past the chunk's lanes) and the scores of its first and
+// last lane (f / l), for the merge in bitslice_body.
+struct SubOut {
+    int *ws, *nsm, *nsp, *f, *l;
+    int c1, c2;  // sub_frac's range ends
+};
+
 // RU (the runner-up family, k_bitslice_ru): ru[k] = the second-largest masked score of row k's lanes, i.e. the maximum
 // over every valid lane but the winner's.  A second bit-serial max from the top plane down runs over the valid lanes
 // but one of those that tie for best (drop_one_tied; which one does not change the value): where several lanes tie,
 // one of the others survives every plane best has, so ru == best there; with one lane, ru == 0.
-template <int NR_, int NW, int PV, bool AS_WRITTEN, bool RU = false>
+// SUB (the sub-pixel family): the winner's neighbours' scores gathered from V & M after the first chain (SubOut).
+template <int NR_, int NW, int PV, bool AS_WRITTEN, bool RU = false, bool SUB = false>
 __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint32_t (&M)[NR_][NW],
                                     const uint32_t (&valid)[NW], int one, int base, int (&best)[NR_], int (&web)[NR_],
-                                    int *ru = nullptr)
+                                    int *ru = nullptr, const SubOut *so = nullptr)
 {
     uint32_t cand[NR_][NW];
 #pragma unroll
@@ -565,6 +669,17 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
             if (NW == 2) idx = max(idx, (31 - __clz(cand[k][NW - 1])) ^ 32);
             web[k] = base + idx;
             if constexpr (RU) drop_one_tied<NW>(valid, cand[k], (uint32_t)-one, cand2[k]);
+            if constexpr (SUB) {
+                // the chunk merge (MULTI) resolves what lies outside this chunk's lanes
+                uint32_t nbm[NW], nbp[NW];
+                sub_neighbours<NW>((uint32_t)(32 * NW - 1 - idx), one, nbm, nbp);
+                so->nsm[k] = sub_gather<NW, PV>(V[k], M[k], nbm, one);
+                so->nsp[k] = sub_gather<NW, PV>(V[k], M[k], nbp, one);
+                const uint32_t first[1] = {(uint32_t)one}, last[1] = {0x80000000u};
+                const uint32_t m0[1] = {M[k][0]}, m1[1] = {M[k][NW - 1]};
+                so->f[k] = -sub_gather<1, PV>(reinterpret_cast<const uint32_t(&)[1][PV]>(V[k][0]), m0, first, one);
+                so->l[k] = -sub_gather<1, PV>(reinterpret_cast<const uint32_t(&)[1][PV]>(V[k][NW - 1]), m1, last, one);
+            }
             continue;
         }
         uint32_t m, m1;
@@ -582,6 +697,12 @@ __device__ __forceinline__ void wta(const uint32_t (&V)[NR_][NW][PV], const uint
                 // registers there than the negation, which at 128 registers made some of those kernels spill)
                 cand2[k][0] = lop3<0x30>(valid[0], shr_clamp(0x80000000u, m), 0u);  // valid & ~bit
             }
+        }
+        if constexpr (SUB) {
+            uint32_t nbm[NW], nbp[NW];
+            sub_neighbours<NW>(m, one, nbm, nbp);
+            const int nsm = sub_gather<NW, PV>(V[k], M[k], nbm, one), nsp = sub_gather<NW, PV>(V[k], M[k], nbp, one);
+            so->ws[k] = sub_frac(best[k], nsm, nsp, web[k], so->c1, so->c2, one);
         }
     }
     if constexpr (RU) {
@@ -637,13 +758,15 @@ __device__ __forceinline__ void store_if(uint16_t *lane_base, int row, int row_b
 // 32*(l/16) + l%16 and that + 16 (so a walker's 16-pixel segment covers 32 columns and a strip is twice as wide).
 //
 // The body of the kernel families; OutT (int32_t or uint16_t) is the type of the stored best and web.  Pair z's
-// outputs are z * best_stride (best) and z * out_stride (web, runner-up) elements further.  RU (k_bitslice_ru, 16-bit):
-// the runner-up score goes to out_ru as well.
-template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP, bool RU = false>
+// outputs are z * best_stride (best) and z * out_stride (web, runner-up, web_sub) elements further.  RU (k_bitslice_ru,
+// 16-bit): the runner-up score goes to out_ru as well.  SUB (k_bitslice_sub, 16-bit): web_sub goes to out_ws, and MULTI
+// carries one u16 per pixel between chunks in out_carry (see put).
+template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP, bool RU = false, bool SUB = false>
 __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, OutT *out_web, size_t best_stride,
-                                              uint16_t *out_ru = nullptr)
+                                              uint16_t *out_ru = nullptr, uint16_t *out_ws = nullptr,
+                                              uint16_t *out_carry = nullptr)
 {
-    using C = WS<HALF, NW, SEG, RU && !C2 && !HP>;  // (C2 / HP: the aligned ring costs them registers and spills)
+    using C = WS<HALF, NW, SEG, (RU || SUB) && !C2 && !HP>;  // (C2 / HP: the aligned ring costs them registers and spills)
     constexpr int N = C::N, KH = C::KH, PV = C::PV, TW = C::TW, RB = C::RB, NR = C::NR, NRM = C::NRM;
     constexpr int HROW = C::HROW, MROW = C::MROW, STEPS = C::STEPS, EC = C::EC, WPC = C::WPC;
 
@@ -682,6 +805,11 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
     out_web += blockIdx.z * a.h.out_stride;
     static_assert(!RU || std::is_same<OutT, uint16_t>::value, "runner-up: 16-bit outputs only");
     if constexpr (RU) out_ru += blockIdx.z * a.h.out_stride;
+    static_assert(!SUB || (std::is_same<OutT, uint16_t>::value && !RU), "sub-pixel: 16-bit outputs, no runner-up");
+    if constexpr (SUB) {
+        out_ws += blockIdx.z * a.h.out_stride;
+        if (MULTI) out_carry += blockIdx.z * a.h.out_stride;
+    }
     const PackedGeom &g = a.h.g;
     static_assert(!C2 || (NW == 2 && !MULTI), "column pairs: two words, one 32-shift chunk");
     static_assert(!HP || (!MULTI && SEG == 16 && (C2 || NW == 1)), "half-word pairs: one chunk, 16-pixel segments");
@@ -770,18 +898,44 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
         const int row_bytes = (int)sizeof(OutT) * g.W;
         OutT *const lane_best = out_best + ximg, *const lane_web = out_web + ximg;
         uint16_t *const lane_ru = RU ? out_ru + ximg : nullptr;
+        uint16_t *const lane_ws = SUB ? out_ws + ximg : nullptr;
+        uint16_t *const lane_carry = SUB && MULTI ? out_carry + ximg : nullptr;
+        // SUB: sub_frac's range ends, web == M + 1 and web == M + D
+        const int sub_c1 = -(a.h.M + 2), sub_c2 = a.h.M + g.D - 1;
 
         // store a finished row (best, web[, runner-up]) and advance the output pointers.  MULTI: a later chunk holds
         // higher shifts, so it wins ties against what the earlier chunks left in `best` (prev).  The runner-up of the
         // shifts so far is the larger of the loser's best and the winner's runner-up (prev_ru: the earlier chunks')
-        auto put = [&](int best, int web, int prev, int ru, int prev_ru) {
+        //
+        // SUB, one chunk: ws is web_sub.  MULTI: between chunks a pixel's winner is SETTLED (web_sub final; the carry
+        // holds the score of the previous chunk's last lane) or PENDING (on its chunk's last lane, whose score is then
+        // best itself; web_sub holds 0, which no final value is, and the carry the winner's s-).  A winner on this
+        // chunk's first lane takes s- from there; a pending one that survives this chunk takes s+ = its first lane (f).
+        auto put = [&](int best, int web, int prev, int ru, int prev_ru, int ws, int nsm, int nsp, int f, int l,
+                       int prev_ws, int prev_carry) {
             bool st = store_ok;
-            if (MULTI && chunk != 0) st = st && best >= prev;
+            const bool wins = !MULTI || chunk == 0 || best >= prev;
+            if (MULTI && chunk != 0) st = st && wins;
             store_if<0>(lane_best, orow, row_bytes, best, st);
             store_if<0>(lane_web, orow, row_bytes, web, st);
             if constexpr (RU) {
                 if (MULTI) ru = max(min(best, prev), best >= prev ? ru : prev_ru);  // (chunk 0: prev == prev_ru == 0)
                 store_if<0>(lane_ru, orow, row_bytes, ru, store_ok);
+            }
+            if constexpr (SUB) {
+                if constexpr (MULTI) {
+                    const int cbase = a.h.M + 32 * wg0;  // web of this chunk's first lane is cbase + 1
+                    const bool pending_prev = chunk != 0 && prev_ws == 0;
+                    const int last_prev = pending_prev ? prev : prev_carry;  // score of the previous chunk's last lane
+                    const bool pending = wins && web == cbase + 32 * NW && chunk + 1 < nchunks;
+                    const int s0 = wins ? best : prev, w = wins ? web : cbase;
+                    const int nm = wins ? (chunk != 0 && web == cbase + 1 ? -last_prev : nsm) : -prev_carry;
+                    const int np = wins ? nsp : -f;
+                    const int wsn = sub_frac(s0, nm, np, w, sub_c1, sub_c2, one);
+                    ws = pending ? 0 : (wins || pending_prev ? wsn : prev_ws);
+                    store_if<0>(lane_carry, orow, row_bytes, pending ? -nsm : l, store_ok);
+                }
+                store_if<0>(lane_ws, orow, row_bytes, ws, store_ok);
             }
             orow++;
         };
@@ -797,8 +951,19 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
             if (RU && MULTI && chunk != 0 && store_ok) v = lane_ru[(size_t)(orow + k) * g.W];
             return v;
         };
+        // ... and (SUB) in web_sub and the carry
+        auto load_prev_ws = [&](int k) {
+            int v = 0;
+            if (SUB && MULTI && chunk != 0 && store_ok) v = lane_ws[(size_t)(orow + k) * g.W];
+            return v;
+        };
+        auto load_prev_carry = [&](int k) {
+            int v = 0;
+            if (SUB && MULTI && chunk != 0 && store_ok) v = lane_carry[(size_t)(orow + k) * g.W];
+            return v;
+        };
         // C2: the two pixels of a lane (columns ximg and ximg + 32) of one finished row
-        auto put2 = [&](int best0, int web0, int best1, int web1, int ru0, int ru1) {
+        auto put2 = [&](int best0, int web0, int best1, int web1, int ru0, int ru1, int ws0, int ws1) {
             store_if<0>(lane_best, orow, row_bytes, best0, store_ok);
             store_if<0>(lane_web, orow, row_bytes, web0, store_ok);
             store_if<TW>(lane_best, orow, row_bytes, best1, store_ok2);
@@ -807,10 +972,15 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                 store_if<0>(lane_ru, orow, row_bytes, ru0, store_ok);
                 store_if<TW>(lane_ru, orow, row_bytes, ru1, store_ok2);
             }
+            if constexpr (SUB) {
+                store_if<0>(lane_ws, orow, row_bytes, ws0, store_ok);
+                store_if<TW>(lane_ws, orow, row_bytes, ws1, store_ok2);
+            }
             orow++;
         };
         // HP: the 2 * NW pixels of a lane of one finished row: word w covers columns ximg + w * WCOLS and that + 16
-        auto put_hp = [&](const int *bl, const int *wl, const int *bh, const int *wh, const int *rl, const int *rh) {
+        auto put_hp = [&](const int *bl, const int *wl, const int *bh, const int *wh, const int *rl, const int *rh,
+                          const int *sl, const int *sh) {
             store_if<0>(lane_best, orow, row_bytes, bl[0], ximg < g.W);
             store_if<0>(lane_web, orow, row_bytes, wl[0], ximg < g.W);
             store_if<16>(lane_best, orow, row_bytes, bh[0], ximg + 16 < g.W);
@@ -818,6 +988,10 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
             if constexpr (RU) {
                 store_if<0>(lane_ru, orow, row_bytes, rl[0], ximg < g.W);
                 store_if<16>(lane_ru, orow, row_bytes, rh[0], ximg + 16 < g.W);
+            }
+            if constexpr (SUB) {
+                store_if<0>(lane_ws, orow, row_bytes, sl[0], ximg < g.W);
+                store_if<16>(lane_ws, orow, row_bytes, sh[0], ximg + 16 < g.W);
             }
             if constexpr (NW == 2) {
                 store_if<WCOLS>(lane_best, orow, row_bytes, bl[NW - 1], ximg + WCOLS < g.W);
@@ -828,13 +1002,18 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                     store_if<WCOLS>(lane_ru, orow, row_bytes, rl[NW - 1], ximg + WCOLS < g.W);
                     store_if<WCOLS + 16>(lane_ru, orow, row_bytes, rh[NW - 1], ximg + WCOLS + 16 < g.W);
                 }
+                if constexpr (SUB) {
+                    store_if<WCOLS>(lane_ws, orow, row_bytes, sl[NW - 1], ximg + WCOLS < g.W);
+                    store_if<WCOLS + 16>(lane_ws, orow, row_bytes, sh[NW - 1], ximg + WCOLS + 16 < g.W);
+                }
             }
             orow++;
         };
         // winner-take-all of G rows held as Vs[G][NW][PV] / Ms[G][NW], then the stores: one WTA over both words
         // of a pixel, or (C2) one per word, the 2*G single-word chains interleaved like rows, or (HP) one per
         // half word: the lower halves of all words first, then the upper halves
-        auto finish_rows = [&](auto gtag, const auto &Vs, const auto &Ms, const int *prev, const int *prev_ru) {
+        auto finish_rows = [&](auto gtag, const auto &Vs, const auto &Ms, const int *prev, const int *prev_ru,
+                               const int *prev_ws, const int *prev_carry) {
             constexpr int G_ = decltype(gtag)::value;
             if constexpr (HP) {
                 constexpr int NCH = G_ * NW;
@@ -849,17 +1028,23 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                     }
                 const uint32_t vl1[1] = {valid_lo}, vh1[1] = {valid_hi};
                 // the upper half's lanes are 16..31 of the word: web = M + lane - 16 + 1
-                int bl[NCH], wl[NCH], bh[NCH], wh[NCH], rl[NCH], rh[NCH];
-                wta<NCH, 1, PV, !MULTI, RU>(V1, M1, vl1, one, a.h.M + 1, bl, wl, rl);
-                wta<NCH, 1, PV, !MULTI, RU>(V1, M1, vh1, one, a.h.M + 1 - 16, bh, wh, rh);
+                int bl[NCH], wl[NCH], bh[NCH], wh[NCH], rl[NCH], rh[NCH], sl[NCH], sh[NCH];
+                const SubOut sol = {sl, nullptr, nullptr, nullptr, nullptr, sub_c1, sub_c2};
+                const SubOut soh = {sh, nullptr, nullptr, nullptr, nullptr, sub_c1, sub_c2};
+                wta<NCH, 1, PV, !MULTI, RU, SUB>(V1, M1, vl1, one, a.h.M + 1, bl, wl, rl, &sol);
+                wta<NCH, 1, PV, !MULTI, RU, SUB>(V1, M1, vh1, one, a.h.M + 1 - 16, bh, wh, rh, &soh);
 #pragma unroll
                 for (int k = 0; k < G_; k++)
-                    put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW, rl + k * NW, rh + k * NW);
+                    put_hp(bl + k * NW, wl + k * NW, bh + k * NW, wh + k * NW, rl + k * NW, rh + k * NW, sl + k * NW,
+                           sh + k * NW);
             } else if constexpr (!C2) {
-                int best[G_], web[G_], ru[G_];
-                wta<G_, NW, PV, !MULTI, RU>(Vs, Ms, valid, one, a.h.M + 32 * wg0 + 1, best, web, ru);
+                int best[G_], web[G_], ru[G_], ws[G_], nsm[G_], nsp[G_], f[G_], l[G_];
+                const SubOut so = {ws, nsm, nsp, f, l, sub_c1, sub_c2};
+                wta<G_, NW, PV, !MULTI, RU, SUB>(Vs, Ms, valid, one, a.h.M + 32 * wg0 + 1, best, web, ru, &so);
 #pragma unroll
-                for (int k = 0; k < G_; k++) put(best[k], web[k], prev[k], ru[k], prev_ru[k]);
+                for (int k = 0; k < G_; k++)
+                    put(best[k], web[k], prev[k], ru[k], prev_ru[k], ws[k], nsm[k], nsp[k], f[k], l[k], prev_ws[k],
+                        prev_carry[k]);
             } else {
                 uint32_t V1[2 * G_][1][PV], M1[2 * G_][1];
 #pragma unroll
@@ -871,11 +1056,13 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                         for (int p = 0; p < PV; p++) V1[2 * k + w][0][p] = Vs[k][w][p];
                     }
                 const uint32_t valid1[1] = {valid[0]};
-                int best[2 * G_], web[2 * G_], ru[2 * G_];
-                wta<2 * G_, 1, PV, !MULTI, RU>(V1, M1, valid1, one, a.h.M + 1, best, web, ru);
+                int best[2 * G_], web[2 * G_], ru[2 * G_], ws[2 * G_];
+                const SubOut so = {ws, nullptr, nullptr, nullptr, nullptr, sub_c1, sub_c2};
+                wta<2 * G_, 1, PV, !MULTI, RU, SUB>(V1, M1, valid1, one, a.h.M + 1, best, web, ru, &so);
 #pragma unroll
                 for (int k = 0; k < G_; k++)
-                    put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1], ru[2 * k], ru[2 * k + 1]);
+                    put2(best[2 * k], web[2 * k], best[2 * k + 1], web[2 * k + 1], ru[2 * k], ru[2 * k + 1], ws[2 * k],
+                         ws[2 * k + 1]);
             }
         };
         auto load_m = [&](int mslot_c, uint32_t (&M)[NW]) {
@@ -960,11 +1147,15 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 
             // MULTI: the earlier chunks' `best` of the rows this block finishes, asked for now so that the loads
             // are back long before the stores that depend on them (they used to be one exposed L2 round trip per row)
-            int prev[RB], prev_ru[RB];
+            int prev[RB], prev_ru[RB], prev_ws[RB], prev_carry[RB];
 #pragma unroll
             for (int r = 0; r < RB; r++) prev[r] = steady ? load_prev(r) : 0;
 #pragma unroll
             for (int r = 0; r < RB; r++) prev_ru[r] = RU && steady ? load_prev_ru(r) : 0;
+#pragma unroll
+            for (int r = 0; r < RB; r++) prev_ws[r] = SUB && steady ? load_prev_ws(r) : 0;
+#pragma unroll
+            for (int r = 0; r < RB; r++) prev_carry[r] = SUB && steady ? load_prev_carry(r) : 0;
 
             pass_a(p0, nrows);
 
@@ -1018,7 +1209,8 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
                         else
                             load_m(wrap_m(mslot0 + r + k - HALF), Ms[k]);
                     }
-                    finish_rows(std::integral_constant<int, G>{}, Vs, Ms, prev + r, prev_ru + r);
+                    finish_rows(std::integral_constant<int, G>{}, Vs, Ms, prev + r, prev_ru + r, prev_ws + r,
+                                prev_carry + r);
                 }
             } else if (filling) {
                 fill_rows(RB);
@@ -1055,8 +1247,8 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
 #pragma unroll
                             for (int p = 0; p < PV; p++) Vs[0][w][p] = V[w][p];
                         load_m(wrap_m(mslot0 + r - HALF), Ms[0]);  // centre row j + HALF
-                        const int pv = load_prev(0), pvr = load_prev_ru(0);
-                        finish_rows(std::integral_constant<int, 1>{}, Vs, Ms, &pv, &pvr);
+                        const int pv = load_prev(0), pvr = load_prev_ru(0), pvs = load_prev_ws(0), pvc = load_prev_carry(0);
+                        finish_rows(std::integral_constant<int, 1>{}, Vs, Ms, &pv, &pvr, &pvs, &pvc);
                     }
                 }
             }
@@ -1116,12 +1308,44 @@ k_bitslice_ru(BitsliceRuArgs a)
                                                                 a.runner_up);
 }
 
-// the family: int32 (k_bitslice), 16-bit (k_bitslice16) or 16-bit with the runner-up (RU, k_bitslice_ru)
-template <typename OutT, bool RU, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+// uint16_t best / web and web_sub, the web in sixteenths of a shift: the 16-bit kernels' argument, the web_sub array
+// and (MULTI) the u16 per pixel that carries a winner's neighbour scores between chunks
+struct BitsliceSubArgs {
+    BitsliceArgs b;
+    uint16_t *web_sub;  // [pairs][FH][W], pair z out_stride elements further
+    uint16_t *carry;    // the same layout, MULTI only (scratch of the caller's)
+};
+
+// CTAs per SM of a sub-pixel kernel: its 16-bit sibling's, but one fewer for the MULTI kernels of windows 5 to 15.  At
+// the sibling's 4 CTAs (128 registers) those spill (windows 5 and 7: 104 and 52 bytes of stores)
+template <int HALF, int NW, int SEG, bool MULTI>
+constexpr int sub_ctas_per_sm()
+{
+    constexpr int c = WS<HALF, NW, SEG, true>::CTAS_PER_SM;
+    return MULTI && HALF >= 2 && HALF <= 7 && c == 4 ? c - 1 : c;
+}
+
+template <int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+__global__ void __launch_bounds__(32 * WS<HALF, NW, SEG, true>::WPC, (sub_ctas_per_sm<HALF, NW, SEG, MULTI>()))
+k_bitslice_sub(BitsliceSubArgs a)
+{
+    bitslice_body<uint16_t, HALF, NW, SEG, MULTI, C2, HP, false, true>(a.b, static_cast<uint16_t *>(a.b.h.best),
+                                                                       static_cast<uint16_t *>(a.b.h.web),
+                                                                       a.b.h.out_stride, nullptr, a.web_sub, a.carry);
+}
+
+// which outputs a family stores beyond best / web
+enum Extra { EXTRA_NONE = 0, EXTRA_RU = 1, EXTRA_SUB = 2 };
+
+// the family: int32 (k_bitslice), 16-bit (k_bitslice16), 16-bit with the runner-up (RU, k_bitslice_ru) or with web_sub
+// (SUB, k_bitslice_sub)
+template <typename OutT, int X, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
 constexpr auto kernel_of()
 {
-    static_assert(!RU || std::is_same<OutT, uint16_t>::value, "runner-up: 16-bit outputs only");
-    if constexpr (RU)
+    static_assert(X == EXTRA_NONE || std::is_same<OutT, uint16_t>::value, "runner-up / sub-pixel: 16-bit outputs only");
+    if constexpr (X == EXTRA_SUB)
+        return k_bitslice_sub<HALF, NW, SEG, MULTI, C2, HP>;
+    else if constexpr (X == EXTRA_RU)
         return k_bitslice_ru<HALF, NW, SEG, MULTI, C2, HP>;
     else if constexpr (std::is_same<OutT, uint16_t>::value)
         return k_bitslice16<HALF, NW, SEG, MULTI, C2, HP>;
@@ -1129,10 +1353,13 @@ constexpr auto kernel_of()
         return k_bitslice<HALF, NW, SEG, MULTI, C2, HP>;
 }
 
-template <typename OutT, bool RU, int HALF, int NW, int SEG, bool C2, bool HP>
-int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec, uint16_t *runner_up)
+// extra: the runner-up array (X == EXTRA_RU) or web_sub (EXTRA_SUB); carry: EXTRA_SUB's chunk carry
+template <typename OutT, int X, int HALF, int NW, int SEG, bool C2, bool HP>
+int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec, uint16_t *extra,
+               uint16_t *carry)
 {
-    using C = WS<HALF, NW, SEG, RU && !C2 && !HP>;  // (bitslice_body's layout: its centre-match ring, its shared memory)
+    constexpr bool RU = X == EXTRA_RU, SUB = X == EXTRA_SUB;
+    using C = WS<HALF, NW, SEG, (RU || SUB) && !C2 && !HP>;  // (bitslice_body's layout: its centre-match ring, its shared memory)
     if (mode == MODE_TMEM_COLUMNS) return C::TCOLS;
     // MULTI: more than one chunk of 32*NW shifts, i.e. (best, web) are merged across passes
     // (one word per lane is only chosen for 32 shifts or fewer: no MULTI flavour of it is instantiated)
@@ -1145,15 +1372,17 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
         set_error("bit-sliced kernel: half-word pairs hold at most 16 shifts, not %d", h.g.D);
         return SM_ERR_ARG;
     }
-    auto kern = (C2 || HP) ? kernel_of<OutT, RU, HALF, NW, SEG, false, C2, HP>()
-                           : (multi ? kernel_of<OutT, RU, HALF, NW, SEG, NW == 2 && !HP, false, false>()
-                                    : kernel_of<OutT, RU, HALF, NW, SEG, false, false, false>());
+    auto kern = (C2 || HP) ? kernel_of<OutT, X, HALF, NW, SEG, false, C2, HP>()
+                           : (multi ? kernel_of<OutT, X, HALF, NW, SEG, NW == 2 && !HP, false, false>()
+                                    : kernel_of<OutT, X, HALF, NW, SEG, false, false, false>());
     // resident warps per SM of this instantiation: what shared memory, the 512 TMEM columns and the register file
     // allow, all known at compile time (WS::CTAS_PER_SM is also the kernel's __launch_bounds__).  (The occupancy
     // API is not asked: it answers 1 CTA per SM for these kernels, whatever carve-out is set, while the
     // hardware runs the 4 that ncu's launch__occupancy_limit_* report.)
-    // (the runner-up family's MULTI kernels may hold fewer: ru_ctas_per_sm)
-    const int ctas_per_sm = RU && multi ? ru_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>() : C::CTAS_PER_SM;
+    // (the runner-up and sub-pixel families' MULTI kernels may hold fewer: ru_ctas_per_sm, sub_ctas_per_sm)
+    const int ctas_per_sm = RU && multi    ? ru_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>()
+                            : SUB && multi ? sub_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>()
+                                           : C::CTAS_PER_SM;
     const int warps_per_sm = ctas_per_sm * C::WPC;
     if (mode == MODE_PREPARE) {
         SM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_REQ));
@@ -1224,10 +1453,12 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
     }
     segs = shape(segs, a.rows_per_seg);
     dim3 grid((strips + C::WPC - 1) / C::WPC, segs, h.npairs);
-    // the kernel's argument: BitsliceArgs, or with RU that and the runner-up array
-    typename std::conditional<RU, BitsliceRuArgs, BitsliceArgs>::type arg;
+    // the kernel's argument: BitsliceArgs, or with RU that and the runner-up array, with SUB web_sub and the carry
+    typename std::conditional<RU, BitsliceRuArgs, typename std::conditional<SUB, BitsliceSubArgs, BitsliceArgs>::type>::type arg;
     if constexpr (RU)
-        arg = BitsliceRuArgs{a, runner_up};
+        arg = BitsliceRuArgs{a, extra};
+    else if constexpr (SUB)
+        arg = BitsliceSubArgs{a, extra, carry};
     else
         arg = a;
     if (h.after_pack) {
@@ -1300,10 +1531,11 @@ static Shape pick_shape(const HotArgs &h, int num_sms)
     return sh;
 }
 
-// the kernel of the geometry, from the family that stores OutT (RU: and the runner-up, to runner_up)
-template <typename OutT, bool RU = false>
+// the kernel of the geometry, from the family that stores OutT (X: and the runner-up or web_sub, to extra; the
+// sub-pixel family's chunk carry to carry)
+template <typename OutT, int X = EXTRA_NONE>
 int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec = nullptr,
-             uint16_t *runner_up = nullptr)
+             uint16_t *extra = nullptr, uint16_t *carry = nullptr)
 {
     if (mode == MODE_PREPARE && h.npairs == 1) {
         // a context launches one pair at a time AND batches: prepare the batch flavour too if it is another kernel
@@ -1311,7 +1543,7 @@ int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchReco
         hb.npairs = 2;
         const Shape a = pick_shape(h, num_sms), b = pick_shape(hb, num_sms);
         if (a.seg != b.seg || a.nw != b.nw || a.c2 != b.c2 || a.hp != b.hp) {
-            const int rc = dispatch<OutT, RU>(hb, num_sms, s, mode);
+            const int rc = dispatch<OutT, X>(hb, num_sms, s, mode);
             if (rc < 0) return rc;
         }
     }
@@ -1319,7 +1551,7 @@ int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchReco
     const int half = h.g.half;
 #define SM_SHAPE(HF, NW_, SEG_, C2_, HP_) \
     if (half == HF && sh.nw == NW_ && sh.seg == SEG_ && sh.c2 == C2_ && sh.hp == HP_) \
-        return launch_one<OutT, RU, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec, runner_up);
+        return launch_one<OutT, X, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec, extra, carry);
 #define SM_HALVES(M, ...) \
     M(0, __VA_ARGS__) M(1, __VA_ARGS__) M(2, __VA_ARGS__) M(3, __VA_ARGS__) M(4, __VA_ARGS__) M(5, __VA_ARGS__) \
     M(6, __VA_ARGS__) M(7, __VA_ARGS__) M(8, __VA_ARGS__) M(9, __VA_ARGS__) M(10, __VA_ARGS__) M(11, __VA_ARGS__) \

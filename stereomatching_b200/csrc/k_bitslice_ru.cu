@@ -6,10 +6,10 @@ namespace smb {
 
 int launch_bitslice_ru(const HotArgs &h, uint16_t *runner_up, int num_sms, cudaStream_t s, LaunchRecord *rec)
 {
-    return dispatch<uint16_t, true>(h, num_sms, s, MODE_LAUNCH, rec, runner_up);
+    return dispatch<uint16_t, EXTRA_RU>(h, num_sms, s, MODE_LAUNCH, rec, runner_up);
 }
 
 // the runner-up counterpart of prepare_bitslice16: run once per context, before its first runner-up launch
-int prepare_bitslice_ru(const HotArgs &h, int num_sms) { return dispatch<uint16_t, true>(h, num_sms, nullptr, MODE_PREPARE); }
+int prepare_bitslice_ru(const HotArgs &h, int num_sms) { return dispatch<uint16_t, EXTRA_RU>(h, num_sms, nullptr, MODE_PREPARE); }
 
 }  // namespace smb

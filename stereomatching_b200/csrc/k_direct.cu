@@ -42,14 +42,18 @@ __device__ __forceinline__ void window(const HotArgs &a, int x, int j, int i, in
 }
 
 // best / web of pixel x of band row j, stored as T; best may be NULL (16-bit outputs: web only).  RU: also the
-// runner-up score (the second largest of the pixel's scores, best again where two shifts tie for it)
-template <typename T, bool RU = false>
-__device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *web_out, uint16_t *ru_out = nullptr)
+// runner-up score (the second largest of the pixel's scores, best again where two shifts tie for it).  SUB: also
+// web_sub, the web in sixteenths of a shift (k_bitslice.cuh, sub_frac), from the scores next to the winner: the shift
+// before it, kept when it wins, and the one after it, captured when no new winner takes it
+template <typename T, bool RU = false, bool SUB = false>
+__device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *web_out, uint16_t *ru_out = nullptr,
+                                             uint16_t *sub_out = nullptr)
 {
     int x = blockIdx.x * blockDim.x + threadIdx.x;
     int j = blockIdx.y * blockDim.y + threadIdx.y;
     if (x >= a.g.W || j >= a.g.BH) return;
     int best = 0, web = 0, ru = 0;
+    int sm = 0, sp = 0, last = 0;  // SUB: s(w - 1), s(w + 1), the previous shift's score
     for (int i = 0; i < a.g.D; i++) {
         int box, centre;
         window(a, x, j, i, box, centre);
@@ -58,14 +62,27 @@ __device__ __forceinline__ void direct_pixel(const HotArgs &a, T *best_out, T *w
             if (RU) ru = best;
             best = score;
             web = i + 1;
-        } else if (RU) {
-            ru = max(ru, score);
+            if (SUB) sm = last;
+        } else {
+            if (RU) ru = max(ru, score);
+            if (SUB && i == web) sp = score;  // the shift after the winner (web = winner + 1)
         }
+        if (SUB) last = score;
     }
     size_t p = (size_t)(a.row0 + j) * a.g.W + x;
     if (sizeof(T) == 4 || best_out) best_out[p] = (T)best;  // (the int32 kernel always has a best)
     web_out[p] = (T)(a.M + web);  // shift i of the planes is M + i
     if (RU) ru_out[p] = (uint16_t)ru;
+    if (SUB) {
+        // frac = min(7, floor((16 * (s+ - s-) + den) / (2 * den))), den = 2 * best - s- - s+ >= 1; 0 at the range ends
+        int frac = 0;
+        if (web > 1 && web < a.g.D) {
+            const int den = 2 * best - sm - sp, num = 16 * (sp - sm) + den;
+            const int q = num >= 0 ? num / (2 * den) : -((-num + 2 * den - 1) / (2 * den));
+            frac = min(7, q);
+        }
+        sub_out[p] = (uint16_t)(16 * (a.M + web) + frac);
+    }
 }
 
 __global__ void __launch_bounds__(256) k_direct(HotArgs a)
@@ -85,11 +102,20 @@ __global__ void __launch_bounds__(256) k_direct16_ru(HotArgs a, uint16_t *runner
     direct_pixel<uint16_t, true>(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web), runner_up);
 }
 
-int launch_direct(const HotArgs &a, cudaStream_t s, bool out16, uint16_t *runner_up)
+// the 16-bit twin with web_sub (a.best may be NULL; web_sub may not)
+__global__ void __launch_bounds__(256) k_direct16_sub(HotArgs a, uint16_t *web_sub)
+{
+    direct_pixel<uint16_t, false, true>(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web), nullptr,
+                                        web_sub);
+}
+
+int launch_direct(const HotArgs &a, cudaStream_t s, bool out16, uint16_t *runner_up, uint16_t *web_sub)
 {
     dim3 block(32, 8);
     dim3 grid((a.g.W + block.x - 1) / block.x, (a.g.BH + block.y - 1) / block.y);
-    if (runner_up)
+    if (web_sub)
+        k_direct16_sub<<<grid, block, 0, s>>>(a, web_sub);
+    else if (runner_up)
         k_direct16_ru<<<grid, block, 0, s>>>(a, runner_up);
     else if (out16)
         k_direct16<<<grid, block, 0, s>>>(a);
@@ -131,6 +157,7 @@ void warm_direct()
     warm_kernel(k_direct);
     warm_kernel(k_direct16);
     warm_kernel(k_direct16_ru);
+    warm_kernel(k_direct16_sub);
     warm_kernel(k_planes);
 }
 

@@ -71,8 +71,11 @@ struct sm_ctx {
     // frame-sized 16-bit arrays: sm_bands_run16's results, sm_download_web_u16's narrowed web
     uint16_t *best16 = nullptr, *web16 = nullptr;
     uint16_t *ru16 = nullptr;  // sm_bands_run_ru16's runner-up scores
+    uint16_t *sub16 = nullptr;    // sm_bands_run_sub16's web_sub
+    uint16_t *carry16 = nullptr;  // the sub-pixel kernels' chunk carry of one-pair launches (more than 64 shifts)
     bool prepared16 = false;  // the 16-bit bit-sliced kernels of this geometry are loaded (prepare_bitslice16)
     int occ_ru = 0;           // ... the runner-up kernels (prepare_bitslice_ru; 0: not yet): their resident warps per SM
+    int occ_sub = 0;          // ... the sub-pixel kernels (prepare_bitslice_sub; 0: not yet)
     int32_t *web2 = nullptr, *tmp = nullptr;  // step 3 ping-pong
     const int32_t *web_filled = nullptr;      // result of fill_web_holes (may alias web)
     bool have_web2 = false;
@@ -101,6 +104,9 @@ struct sm_ctx {
     // (with the caller's pair stride, out_stride: pbest16_elems elements each)
     uint16_t *pBest16[NPB] = {nullptr, nullptr, nullptr};
     size_t pbest16_elems = 0;
+    // the sub-pixel kernels' chunk carry (more than 64 shifts), sized and ordered like pBest16
+    uint16_t *pCarry16[NPB] = {nullptr, nullptr, nullptr};
+    size_t pcarry16_elems = 0;
     // scratch for on-demand debug planes / u8 web
     uint8_t *scratch_u8 = nullptr;
     int32_t *scratch_i32 = nullptr;
@@ -120,6 +126,7 @@ struct sm_ctx {
         // the 16-bit results, written by the hot path itself ([group][npix]; best16 only when the caller wants best)
         uint16_t *web16[NPIPE] = {nullptr, nullptr, nullptr}, *best16[NPIPE] = {nullptr, nullptr, nullptr};
         uint16_t *ru16[NPIPE] = {nullptr, nullptr, nullptr};  // the runner-up scores, only when the caller wants them
+        uint16_t *sub16[NPIPE] = {nullptr, nullptr, nullptr};  // web_sub, only when the caller wants it
         cudaEvent_t ev_up[NPIPE] = {nullptr, nullptr, nullptr}, ev_comp[NPIPE] = {nullptr, nullptr, nullptr},
                     ev_down[NPIPE] = {nullptr, nullptr, nullptr};
     } pipe;
@@ -222,16 +229,18 @@ int copy_band_d2h(sm_ctx *c, T *host, const T *dev)
 }
 
 // Where a hot-path call writes best / web: int32 arrays, or (web16 set) 16-bit ones, best16 possibly NULL.  With
-// 16-bit ones, runner_up (if set) receives the runner-up scores (the runner-up kernels).
+// 16-bit ones, runner_up (if set) receives the runner-up scores (the runner-up kernels), or web_sub (if set) the web in
+// sixteenths of a shift (the sub-pixel kernels; past 64 shifts they need a carry array of the same layout).
 struct Outputs {
     int32_t *best = nullptr, *web = nullptr;
     uint16_t *best16 = nullptr, *web16 = nullptr;
     uint16_t *runner_up = nullptr;
+    uint16_t *web_sub = nullptr, *carry = nullptr;
     // pair k of a batch: every array k * stride elements further
     Outputs pair(size_t k, size_t stride) const
     {
         auto at = [&](auto *p) { return p ? p + k * stride : p; };
-        return {at(best), at(web), at(best16), at(web16), at(runner_up)};
+        return {at(best), at(web), at(best16), at(web16), at(runner_up), at(web_sub), at(carry)};
     }
 };
 
@@ -274,8 +283,26 @@ int prepare_ru(sm_ctx *c)
     return SM_OK;
 }
 
-// The main kernel: of the runner-up family with runner_up, of the 16-bit one with out16, else of the int32 one.
-int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cudaStream_t st)
+// Loads the sub-pixel kernels of the context's geometry (once); their resident warps per SM go to c->occ_sub.
+int prepare_sub(sm_ctx *c)
+{
+    if (c->occ_sub > 0) return SM_OK;
+    int occ = c->occ;
+    if (hot_kernel(c) == SM_KERNEL_BITSLICE && bitslice_supports(c->half, c->D)) {
+        occ = prepare_bitslice_sub(hot_args(c, Outputs{}), c->num_sms);
+        if (occ < 0) return occ;
+    }
+    c->occ_sub = occ > 0 ? occ : 1;
+    return SM_OK;
+}
+
+// whether the sub-pixel kernel of the context merges 64-shift chunks (and needs Outputs::carry)
+bool sub_needs_carry(const sm_ctx *c) { return hot_kernel(c) == SM_KERNEL_BITSLICE && c->D > 64; }
+
+// The main kernel: of the runner-up family with runner_up, of the sub-pixel one with web_sub, of the 16-bit one with
+// out16, else of the int32 one.
+int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cudaStream_t st, uint16_t *web_sub = nullptr,
+                uint16_t *carry = nullptr)
 {
     const int k = hot_kernel(c);
     if (k == SM_KERNEL_BITSLICE) {
@@ -283,7 +310,7 @@ int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cu
             set_error("bit-sliced kernel does not cover square_width %d / num_shifts %d", c->sw, c->D);
             return SM_ERR_ARG;
         }
-        if (out16 && !runner_up && !c->prepared16) {  // (sm_create prepared the int32 family)
+        if (out16 && !runner_up && !web_sub && !c->prepared16) {  // (sm_create prepared the int32 family)
             const int rc = prepare_bitslice16(hot_args(c, Outputs{}), c->num_sms);
             if (rc < 0) return rc;
             c->prepared16 = true;
@@ -292,14 +319,19 @@ int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cu
             const int rc = prepare_ru(c);
             if (rc < 0) return rc;
         }
+        if (web_sub) {
+            const int rc = prepare_sub(c);
+            if (rc < 0) return rc;
+        }
         LaunchRecord rec;
         const int rc = runner_up ? launch_bitslice_ru(a, runner_up, c->num_sms, st, &rec)
+                       : web_sub ? launch_bitslice_sub(a, web_sub, carry, c->num_sms, st, &rec)
                        : out16   ? launch_bitslice16(a, c->num_sms, st, &rec)
                                  : launch_bitslice(a, c->num_sms, st, &rec);
         if (rc >= 0) c->last_launch = rec;
         return rc;
     }
-    const int rc = launch_direct(a, st, out16, runner_up);
+    const int rc = launch_direct(a, st, out16, runner_up, web_sub);
     if (rc >= 0) {
         c->last_launch.shape = SM_SHAPE_DIRECT;
         c->last_launch.row_runs = 0;
@@ -331,7 +363,12 @@ int run_hot(sm_ctx *c, const uint8_t *e1, const uint8_t *e2, const Outputs &out)
     // per-kernel profile put an event in between: the main kernel may start as its programmatic dependent.
     // (It waits for every earlier grid of the stream to complete before it reads anything, whatever that grid is.)
     a.after_pack = pe == nullptr && !no_pdl;
-    rc = launch_main(c, a, out.web16 != nullptr, out.runner_up, c->stream);
+    uint16_t *carry = nullptr;
+    if (out.web_sub && sub_needs_carry(c)) {
+        if ((rc = dev_alloc(&c->carry16, c->npix()))) return rc;  // (frame-sized: band contexts write their own rows)
+        carry = c->carry16;
+    }
+    rc = launch_main(c, a, out.web16 != nullptr, out.runner_up, c->stream, out.web_sub, carry);
     if (rc < 0) return rc;
     launches += rc;
     SM_CUDA(cudaEventRecord(c->ev1, c->stream));
@@ -361,7 +398,7 @@ extern "C" const char *sm_last_error(void) { return g_err; }
 
 // 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out;
 // 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS; then, additive, the 16-bit result entries (*16, sm_download_web_u16),
-// the search-range creators (*_range) and the runner-up entries (*_ru16)
+// the search-range creators (*_range), the runner-up entries (*_ru16) and the sub-pixel entries (*_sub16)
 extern "C" int sm_version(void) { return (1 << 16) | 3; }
 
 extern "C" int sm_device_count(void)
@@ -528,7 +565,7 @@ extern "C" int sm_destroy(sm_ctx *c)
         }
     for (int k = 0; k < sm_ctx::NPIPE; k++) {
         void *pp[] = {c->pipe.img[k], c->pipe.edg[k], c->pipe.web[k], c->pipe.best[k], c->pipe.web8[k],
-                      c->pipe.web16[k], c->pipe.best16[k], c->pipe.ru16[k]};
+                      c->pipe.web16[k], c->pipe.best16[k], c->pipe.ru16[k], c->pipe.sub16[k]};
         for (void *p : pp)
             if (p) cudaFree(p);
         for (cudaEvent_t e : {c->pipe.ev_up[k], c->pipe.ev_comp[k], c->pipe.ev_down[k]})
@@ -539,7 +576,7 @@ extern "C" int sm_destroy(sm_ctx *c)
     void *ptrs[] = {c->img_u8[0], nullptr,      c->img_f64[0], c->img_f64[1], c->edges[0], nullptr,  // [1] = [0] + npix
                     c->best,      c->web,       c->web2,       c->tmp,        c->out,      c->minmax,
                     c->LA,        c->LB,        c->RB,         c->scratch_u8, c->scratch_i32,
-                    c->best16,    c->web16,     c->ru16};
+                    c->best16,    c->web16,     c->ru16,       c->sub16,      c->carry16};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     if (c->prof_ev) profile_free(c);
@@ -559,6 +596,7 @@ extern "C" int sm_destroy(sm_ctx *c)
         if (c->ev_packed[k]) cudaEventDestroy(c->ev_packed[k]);
         if (c->ev_used[k]) cudaEventDestroy(c->ev_used[k]);
         if (c->pBest16[k]) cudaFree(c->pBest16[k]);
+        if (c->pCarry16[k]) cudaFree(c->pCarry16[k]);
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -822,6 +860,22 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         }
         if (need > c->pbest16_elems) c->pbest16_elems = need;
     }
+    const bool with_carry = out.web_sub && sub_needs_carry(c);
+    if (with_carry) {
+        // as the scratch best: pair k of a launch k * out_stride elements further, one array per plane set
+        const size_t need = out_stride * (size_t)c->batch_group_cap;
+        if (need > c->pcarry16_elems)
+            for (int k = 0; k < NPB; k++)
+                if (c->pCarry16[k]) {
+                    SM_CUDA(cudaFree(c->pCarry16[k]));  // (waits for the device: no launch still uses it)
+                    c->pCarry16[k] = nullptr;
+                }
+        for (int k = 0; k < NPB; k++) {
+            int rc;
+            if ((rc = dev_alloc(&c->pCarry16[k], need > c->pcarry16_elems ? need : c->pcarry16_elems))) return rc;
+        }
+        if (need > c->pcarry16_elems) c->pcarry16_elems = need;
+    }
     // the kernel may have been switched since the last call (sm_set_kernel): the literal kernel takes one pair
     // per launch, the bit-sliced one a group
     c->batch_group = kk == SM_KERNEL_BITSLICE ? c->batch_group_cap : 1;
@@ -833,6 +887,17 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         if (c->occ_ru != c->occ) {
             HotArgs a = hot_args(c, out);
             a.blocks_per_sm = c->occ_ru;
+            const int g = bitslice_pairs_per_launch(a, c->num_sms, c->batch_group_cap);
+            c->batch_group = g < c->batch_group_cap ? g : c->batch_group_cap;
+        }
+    }
+    if (out.web_sub && kk == SM_KERNEL_BITSLICE) {
+        // the same for the sub-pixel kernels
+        int rc;
+        if ((rc = prepare_sub(c)) < 0) return rc;
+        if (c->occ_sub != c->occ) {
+            HotArgs a = hot_args(c, out);
+            a.blocks_per_sm = c->occ_sub;
             const int g = bitslice_pairs_per_launch(a, c->num_sms, c->batch_group_cap);
             c->batch_group = g < c->batch_group_cap ? g : c->batch_group_cap;
         }
@@ -878,7 +943,7 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
         a.npairs = np;
         a.plane_stride = pw;
         a.out_stride = out_stride;
-        rc = launch_main(c, a, o.web16 != nullptr, o.runner_up, ms);
+        rc = launch_main(c, a, o.web16 != nullptr, o.runner_up, ms, o.web_sub, with_carry ? c->pCarry16[b] : nullptr);
         if (rc < 0) return rc;
         launches += rc;
         if (pe) {
@@ -928,6 +993,24 @@ extern "C" int sm_match_wta_dev_batch_ru16(sm_ctx *c, int n_pairs, const uint8_t
     SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch_ru16: stride below frame size");
     return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride,
                       {nullptr, nullptr, d_best, d_web, d_runner_up}, out_stride);
+}
+
+extern "C" int sm_match_wta_dev_batch_sub16(sm_ctx *c, int n_pairs, const uint8_t *d_first_edges,
+                                            const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best,
+                                            uint16_t *d_web, uint16_t *d_web_sub, size_t out_stride)
+{
+    SM_REQUIRE(n_pairs >= 0 && d_first_edges && d_second_edges && d_web && d_web_sub,
+               "sm_match_wta_dev_batch_sub16: bad arguments");
+    SM_REQUIRE(c, "sm_match_wta_dev_batch_sub16: NULL context");
+    SM_REQUIRE(c->M + c->D <= SUB_MAX_RANGE, "sm_match_wta_dev_batch_sub16: web_sub needs min_shift + num_shifts <= %d",
+               SUB_MAX_RANGE);
+    SM_ENTER(c);
+    SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(), "sm_match_wta_dev_batch_sub16: stride below frame size");
+    Outputs o;
+    o.best16 = d_best;
+    o.web16 = d_web;
+    o.web_sub = d_web_sub;
+    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, o, out_stride);
 }
 
 extern "C" int sm_elapsed_ms(sm_ctx *c, float *ms)
@@ -1181,14 +1264,17 @@ enum WebFormat { WEB_I32, WEB_U8, WEB_U16 };
 static size_t web_bytes(WebFormat f) { return f == WEB_U8 ? 1 : (f == WEB_U16 ? 2 : 4); }
 static size_t best_bytes(WebFormat f) { return f == WEB_U16 ? 2 : 4; }
 
-// sm_run_batch / sm_run_batch16 / sm_run_batch_ru16 (fn: the entry's name, for the messages; ru_out: the runner-up
-// scores, WEB_U16 only)
+// sm_run_batch / sm_run_batch16 / sm_run_batch_ru16 / sm_run_batch_sub16 (fn: the entry's name, for the messages;
+// ru_out: the runner-up scores, sub_out: web_sub, WEB_U16 only, not both)
 static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
-                     double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
+                     double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr,
+                     uint16_t *sub_out = nullptr)
 {
     SM_ENTER(c);
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     SM_REQUIRE(!ru_out || fmt == WEB_U16, "%s: the runner-up needs 16-bit results", fn);
+    SM_REQUIRE(!sub_out || (fmt == WEB_U16 && !ru_out && c->M + c->D <= SUB_MAX_RANGE),
+               "%s: web_sub needs 16-bit results and min_shift + num_shifts <= %d", fn, SUB_MAX_RANGE);
     SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "%s: whole-frame contexts only", fn);
     SM_REQUIRE(fmt != WEB_U8 || c->M + c->D <= 255, "%s: u8 web needs min_shift + num_shifts <= 255", fn);
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "%s: threshold must be between 0 and 1", fn);
@@ -1218,7 +1304,8 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
     for (int k = 0; k < NP; k++) {
         if (fmt == WEB_U16) {
             if ((rc = dev_alloc(&P.web16[k], P.group * n)) || (best_out && (rc = dev_alloc(&P.best16[k], P.group * n))) ||
-                (ru_out && (rc = dev_alloc(&P.ru16[k], P.group * n))))
+                (ru_out && (rc = dev_alloc(&P.ru16[k], P.group * n))) ||
+                (sub_out && (rc = dev_alloc(&P.sub16[k], P.group * n))))
                 return rc;
         } else if ((rc = dev_alloc(&P.web[k], P.group * n)) || (rc = dev_alloc(&P.best[k], P.group * n))) {
             return rc;
@@ -1249,7 +1336,7 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
         // ---- stage 2, the context's stream: edges of all 2*np images, then the batched hot path
         SM_CUDA(cudaStreamWaitEvent(c->stream, P.ev_up[b], 0));
         const Outputs out = fmt == WEB_U16 ? Outputs{nullptr, nullptr, best_out ? P.best16[b] : nullptr, P.web16[b],
-                                                     ru_out ? P.ru16[b] : nullptr}
+                                                     ru_out ? P.ru16[b] : nullptr, sub_out ? P.sub16[b] : nullptr}
                                            : Outputs{P.best[b], P.web[b]};
         if (use_lut) {
             // edges of all 2*np images straight into the packed planes, then the hot path: two kernels per group
@@ -1286,6 +1373,9 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
         if (ru_out)
             SM_CUDA(cudaMemcpyAsync(ru_out + (size_t)k * n, P.ru16[b], (size_t)np * n * sizeof(uint16_t),
                                     cudaMemcpyDeviceToHost, P.down));
+        if (sub_out)
+            SM_CUDA(cudaMemcpyAsync(sub_out + (size_t)k * n, P.sub16[b], (size_t)np * n * sizeof(uint16_t),
+                                    cudaMemcpyDeviceToHost, P.down));
         SM_CUDA(cudaEventRecord(P.ev_down[b], P.down));
     }
     SM_CUDA(cudaStreamSynchronize(P.up));
@@ -1317,6 +1407,18 @@ extern "C" int sm_run_batch_ru16(sm_ctx *c, int n_pairs, const uint8_t *first, c
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out && runner_up_out, "sm_run_batch_ru16: bad arguments");
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch_ru16: threshold must be between 0 and 1");
     return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
+}
+
+extern "C" int sm_run_batch_sub16(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                  double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out)
+{
+    // the checks that need no context first (and no device)
+    SM_REQUIRE(n_pairs >= 0 && first && second && web_out && web_sub_out, "sm_run_batch_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(c, "sm_run_batch_sub16: NULL context");
+    SM_REQUIRE(c->M + c->D <= SUB_MAX_RANGE, "sm_run_batch_sub16: web_sub needs min_shift + num_shifts <= %d",
+               SUB_MAX_RANGE);
+    return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, nullptr, web_sub_out);
 }
 
 // ---- whole pairs over several GPUs of one box ------------------------------------------------
@@ -1456,9 +1558,10 @@ extern "C" int sm_multi_destroy(sm_multi *m)
 
 extern "C" int sm_multi_device_count(const sm_multi *m) { return m ? m->n : SM_ERR_ARG; }
 
-// sm_multi_run_batch / sm_multi_run_batch16 / sm_multi_run_batch_ru16
+// sm_multi_run_batch / sm_multi_run_batch16 / sm_multi_run_batch_ru16 / sm_multi_run_batch_sub16
 static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
-                           double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
+                           double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr,
+                           uint16_t *sub_out = nullptr)
 {
     SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     const int N = m->n;
@@ -1471,8 +1574,9 @@ static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8
         void *wout = (uint8_t *)web_out + (size_t)k0 * n * wb;
         void *bout = best_out ? (void *)((uint8_t *)best_out + (size_t)k0 * n * bb) : nullptr;
         uint16_t *rout = ru_out ? ru_out + (size_t)k0 * n : nullptr;
+        uint16_t *sout = sub_out ? sub_out + (size_t)k0 * n : nullptr;
         rcs[(size_t)d] = run_batch(fn, m->ctx[d], k1 - k0, first + (size_t)k0 * n, second + (size_t)k0 * n, threshold, fmt,
-                                   wout, bout, rout);
+                                   wout, bout, rout, sout);
         if (rcs[(size_t)d]) errs[(size_t)d] = sm_last_error();  // the message is per thread: carry it to the caller's
     };
     if (m->workers)
@@ -1506,6 +1610,18 @@ extern "C" int sm_multi_run_batch_ru16(sm_multi *m, int n_pairs, const uint8_t *
     SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out && runner_up_out, "sm_multi_run_batch_ru16: bad arguments");
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_multi_run_batch_ru16: threshold must be between 0 and 1");
     return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
+}
+
+extern "C" int sm_multi_run_batch_sub16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                        double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out)
+{
+    // the checks that need no handle first (and no device)
+    SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out && web_sub_out, "sm_multi_run_batch_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_multi_run_batch_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(m->ctx[0]->M + m->ctx[0]->D <= SUB_MAX_RANGE,
+               "sm_multi_run_batch_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
+    return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, nullptr,
+                           web_sub_out);
 }
 
 // ---- one pair, row bands over several GPUs of one box ----------------------------------------------
@@ -1573,27 +1689,29 @@ extern "C" int sm_bands_create(sm_bands **out, const int *devices, int n_devices
 
 // One band context's 16-bit run: the hot path writes rows [row0, row1) of the context's frame-sized u16 arrays
 // (best16 when the caller wants best or the kernel stores it anyway; ru16 with ru_out); only those rows are downloaded.
-static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out, uint16_t *ru_out)
+// (sub16 with sub_out)
+static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out, uint16_t *ru_out, uint16_t *sub_out)
 {
     SM_ENTER(c);
     int rc;
     const bool with_best = best_out || stores_best(c);
     if ((rc = dev_alloc(&c->web16, c->npix())) || (with_best && (rc = dev_alloc(&c->best16, c->npix()))) ||
-        (ru_out && (rc = dev_alloc(&c->ru16, c->npix()))))
+        (ru_out && (rc = dev_alloc(&c->ru16, c->npix()))) || (sub_out && (rc = dev_alloc(&c->sub16, c->npix()))))
         return rc;
     if ((rc = run_hot(c, c->edges[0], c->edges[1],
-                      {nullptr, nullptr, with_best ? c->best16 : nullptr, c->web16, ru_out ? c->ru16 : nullptr})))
+                      {nullptr, nullptr, with_best ? c->best16 : nullptr, c->web16, ru_out ? c->ru16 : nullptr,
+                       sub_out ? c->sub16 : nullptr})))
         return rc;
     if ((rc = copy_band_d2h(c, web_out, c->web16)) || (best_out && (rc = copy_band_d2h(c, best_out, c->best16))) ||
-        (ru_out && (rc = copy_band_d2h(c, ru_out, c->ru16))))
+        (ru_out && (rc = copy_band_d2h(c, ru_out, c->ru16))) || (sub_out && (rc = copy_band_d2h(c, sub_out, c->sub16))))
         return rc;
     SM_CUDA(cudaStreamSynchronize(c->stream));
     return SM_OK;
 }
 
-// sm_bands_run / sm_bands_run16 / sm_bands_run_ru16
+// sm_bands_run / sm_bands_run16 / sm_bands_run_ru16 / sm_bands_run_sub16
 static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
-                     WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr)
+                     WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr, uint16_t *sub_out = nullptr)
 {
     SM_REQUIRE(b && first && second && web_out, "%s: bad arguments", fn);
     const int N = b->n;
@@ -1604,7 +1722,7 @@ static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const ui
         int rc = sm_upload_u8(c, first, second);  // a band context copies only the rows it needs
         if (!rc) rc = sm_edges(c, threshold);
         if (fmt == WEB_U16) {
-            if (!rc) rc = band_run16(c, (uint16_t *)web_out, (uint16_t *)best_out, ru_out);
+            if (!rc) rc = band_run16(c, (uint16_t *)web_out, (uint16_t *)best_out, ru_out, sub_out);
         } else {
             if (!rc) rc = sm_match_wta(c);
             if (!rc) rc = sm_download(c, SM_WEB, 0, web_out);  // ... and writes only its own rows
@@ -1643,4 +1761,14 @@ extern "C" int sm_bands_run_ru16(sm_bands *b, const uint8_t *first, const uint8_
     SM_REQUIRE(b && first && second && web_out && runner_up_out, "sm_bands_run_ru16: bad arguments");
     SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_bands_run_ru16: threshold must be between 0 and 1");
     return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out);
+}
+
+extern "C" int sm_bands_run_sub16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                                  uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out)
+{
+    SM_REQUIRE(b && first && second && web_out && web_sub_out, "sm_bands_run_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_bands_run_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(b->ctx[0]->M + b->ctx[0]->D <= SUB_MAX_RANGE,
+               "sm_bands_run_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
+    return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out, nullptr, web_sub_out);
 }
