@@ -79,8 +79,10 @@ typedef enum sm_option {
                               even for 8-bit uploads; 0 (default): the integer table path for 8-bit images */
     SM_OPT_PIPE_GROUP = 2, /* pairs per stage of the sm_run_batch pipeline; 0 (default): chosen by frame size.
                               Only before the first sm_run_batch of the context */
-    SM_OPT_ROW_RUNS = 3    /* row runs per 32-column strip of a one-pair launch of the bit-sliced kernel;
-                              0 (default): the kernel's cost model */
+    SM_OPT_ROW_RUNS = 3    /* row runs per strip of columns of each pair in every launch of the bit-sliced kernel
+                              (one-pair, batch and band entries alike), rounded to whole blocks of rows; a count
+                              above one run per block of the frame or band is clamped to that.  0 (default): the
+                              kernel's cost model */
 } sm_option;
 
 /* What sm_get_info reports about the launch configuration of the bit-sliced kernel on this context. */

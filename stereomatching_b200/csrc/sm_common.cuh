@@ -85,7 +85,8 @@ struct HotArgs {
     // main kernel may then start as its programmatic dependent (griddepcontrol), so that its
     // launch and prologue overlap the pack kernel's tail
     bool after_pack = false;
-    // one pair per launch: number of row runs per strip (0 = one wave of resident warps)
+    // row runs per strip of each pair, one-pair and batch launches alike, clamped to one per block of rows (0 = the
+    // launch shape's cost model)
     int force_segs = 0;
     // resident warps per SM of the bit-sliced kernel this geometry uses (prepare_bitslice; 0 = ask)
     int blocks_per_sm = 0;

@@ -51,7 +51,7 @@ struct sm_ctx {
     cudaEvent_t *prof_ev = nullptr;
     int prof_cap = 0, prof_n = 0;
     int last_launches = 0;
-    int tuned_segs = 0;  // SM_OPT_ROW_RUNS: row runs per strip of a one-pair launch (0: the kernel's cost model)
+    int tuned_segs = 0;  // SM_OPT_ROW_RUNS: row runs per strip of every bit-sliced launch (0: the kernel's cost model)
     int occ = 0;         // resident warps per SM of the bit-sliced kernel of this geometry (prepare_bitslice)
     LaunchRecord last_launch;  // the most recent hot-path launch (SM_INFO_KERNEL_SHAPE, SM_INFO_ROW_RUNS)
 
