@@ -32,7 +32,7 @@ endif
 
 CSRC   := stereomatching_b200/csrc
 LIB    := stereomatching_b200/libstereo_b200.so
-KOBJS  := $(patsubst %,$(CSRC)/build/%.o,stereo_b200 k_edges k_pack k_direct k_bitslice k_bitslice16 k_bitslice_ru k_bitslice_sub k_step3)
+KOBJS  := $(patsubst %,$(CSRC)/build/%.o,stereo_b200 k_edges k_pack k_direct k_bitslice k_bitslice16 k_bitslice_ru k_bitslice_sub k_bitslice_ru_sub k_step3)
 
 all: lib benchlib $(outdir)/stereopar $(outdir)/stereopar-ghost $(outdir)/stereobatch host/libhostimage.so
 
@@ -49,9 +49,9 @@ $(CSRC)/build/%.o: $(CSRC)/%.cu $(CSRC)/sm_common.cuh include/stereo_b200.h
 	@mkdir -p $(CSRC)/build
 	$(NVCC) $(NVFLAGS) -c $< -o $@
 
-# the four output families of the bit-sliced kernel share its source
+# the five output families of the bit-sliced kernel share its source
 $(CSRC)/build/k_bitslice.o $(CSRC)/build/k_bitslice16.o $(CSRC)/build/k_bitslice_ru.o \
-    $(CSRC)/build/k_bitslice_sub.o: $(CSRC)/k_bitslice.cuh
+    $(CSRC)/build/k_bitslice_sub.o $(CSRC)/build/k_bitslice_ru_sub.o: $(CSRC)/k_bitslice.cuh
 
 $(LIB): $(KOBJS)
 	$(NVCC) $(SM_ARCH) -shared $(KOBJS) -o $@
@@ -68,7 +68,7 @@ $(CSRC)/build_dev/%.o: $(CSRC)/%.cu $(CSRC)/sm_common.cuh include/stereo_b200.h
 	$(NVCC) $(NVFLAGS) -DSMB_DEV $(DEVFLAGS) -c $< -o $@
 
 $(CSRC)/build_dev/k_bitslice.o $(CSRC)/build_dev/k_bitslice16.o $(CSRC)/build_dev/k_bitslice_ru.o \
-    $(CSRC)/build_dev/k_bitslice_sub.o: $(CSRC)/k_bitslice.cuh
+    $(CSRC)/build_dev/k_bitslice_sub.o $(CSRC)/build_dev/k_bitslice_ru_sub.o: $(CSRC)/k_bitslice.cuh
 
 $(DEVLIB): $(DEVKOBJS)
 	$(NVCC) $(SM_ARCH) -shared $(DEVKOBJS) -o $@

@@ -121,8 +121,9 @@ const char *sm_last_error(void);
  * sm_multi_run_batch16, sm_bands_run16, sm_download_web_u16), the search-range creators (sm_create_range,
  * sm_create_band_range, sm_multi_create_range, sm_bands_create_range) and the runner-up entries
  * (sm_match_wta_dev_batch_ru16, sm_run_batch_ru16, sm_multi_run_batch_ru16, sm_bands_run_ru16) and the sub-pixel
- * entries (sm_match_wta_dev_batch_sub16, sm_run_batch_sub16, sm_multi_run_batch_sub16, sm_bands_run_sub16) are
- * additions to 1.3 that leave every other entry as it was; clients detect them by symbol. */
+ * entries (sm_match_wta_dev_batch_sub16, sm_run_batch_sub16, sm_multi_run_batch_sub16, sm_bands_run_sub16) and the
+ * entries with both (sm_match_wta_dev_batch_ru_sub16, sm_run_batch_ru_sub16, sm_multi_run_batch_ru_sub16,
+ * sm_bands_run_ru_sub16) are additions to 1.3 that leave every other entry as it was; clients detect them by symbol. */
 int sm_version(void);
 /* Number of CUDA devices visible, or a negative sm_status. */
 int sm_device_count(void);
@@ -263,6 +264,14 @@ int sm_match_wta_dev_batch_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *d_firs
                                  const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best, uint16_t *d_web,
                                  uint16_t *d_web_sub, size_t out_stride);
 
+/* Both extras from ONE launch of the hot kernel: d_best (may be NULL), d_web, d_runner_up and d_web_sub (neither
+ * NULL) each equal, bit for bit, what sm_match_wta_dev_batch_ru16 and sm_match_wta_dev_batch_sub16 write for the
+ * same context and inputs -- the 16.4 fixed-point disparity and the score a uniqueness filter needs, as a block
+ * matcher returns them.  Needs m + D <= 4095, else SM_ERR_ARG before any device call. */
+int sm_match_wta_dev_batch_ru_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *d_first_edges,
+                                    const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best,
+                                    uint16_t *d_web, uint16_t *d_runner_up, uint16_t *d_web_sub, size_t out_stride);
+
 /* Device time of the last sm_match_wta* call on this context, CUDA events on the
  * context's stream (the reference brackets the whole algorithm() with
  * CLOCK_MONOTONIC instead, stereo.cu:308,334-335).  Waits for the call to finish. */
@@ -332,6 +341,10 @@ int sm_run_batch_ru16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint
  * more copy per group.  min_shift + num_shifts <= 4095. */
 int sm_run_batch_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                        uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
+/* Both (see sm_match_wta_dev_batch_ru_sub16): every output equals its sm_run_batch_ru16 / sm_run_batch_sub16
+ * counterpart, from one pass; runner_up_out and web_sub_out not NULL, two more copies per group. */
+int sm_run_batch_ru_sub16(sm_ctx *ctx, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
+                          uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out, uint16_t *web_sub_out);
 
 /* The same over several GPUs of one box (SURVEY 8e, BASELINE config 4: whole pairs sharded across the
  * GPUs, inputs scattered from the host, no cross-device traffic): one context and one host thread per
@@ -353,6 +366,10 @@ int sm_multi_run_batch_ru16(sm_multi *m, int n_pairs, const uint8_t *first, cons
 /* The same through sm_run_batch_sub16 (web_sub_out not NULL). */
 int sm_multi_run_batch_sub16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second, double threshold,
                              uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
+/* The same through sm_run_batch_ru_sub16 (runner_up_out and web_sub_out not NULL). */
+int sm_multi_run_batch_ru_sub16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out,
+                                uint16_t *web_sub_out);
 int sm_multi_device_count(const sm_multi *m);
 int sm_multi_destroy(sm_multi *m);
 
@@ -380,6 +397,10 @@ int sm_bands_run_ru16(sm_bands *b, const uint8_t *first, const uint8_t *second, 
  * web_sub_out (not NULL). */
 int sm_bands_run_sub16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                        uint16_t *web_out, uint16_t *best_out, uint16_t *web_sub_out);
+/* The same with both (see sm_match_wta_dev_batch_ru_sub16): each band writes its own rows of the frame-sized
+ * runner_up_out and web_sub_out (neither NULL), every output equal to its *_ru16 / *_sub16 counterpart. */
+int sm_bands_run_ru_sub16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                          uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out, uint16_t *web_sub_out);
 int sm_bands_destroy(sm_bands *b);
 
 /* ---- geometry helpers (host-side, no GPU) --------------------------------------- */

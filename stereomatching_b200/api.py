@@ -43,6 +43,7 @@ SYMBOLS = [
     "sm_create_range", "sm_create_band_range", "sm_multi_create_range", "sm_bands_create_range",
     "sm_match_wta_dev_batch_ru16", "sm_run_batch_ru16", "sm_multi_run_batch_ru16", "sm_bands_run_ru16",
     "sm_match_wta_dev_batch_sub16", "sm_run_batch_sub16", "sm_multi_run_batch_sub16", "sm_bands_run_sub16",
+    "sm_match_wta_dev_batch_ru_sub16", "sm_run_batch_ru_sub16", "sm_multi_run_batch_ru_sub16", "sm_bands_run_ru_sub16",
 ]
 
 
@@ -86,6 +87,7 @@ def lib() -> C.CDLL:
         L.sm_match_wta_dev_batch16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, C.c_size_t]
         L.sm_match_wta_dev_batch_ru16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t]
         L.sm_match_wta_dev_batch_sub16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, C.c_size_t]
+        L.sm_match_wta_dev_batch_ru_sub16.argtypes = [vp, i, vp, vp, C.c_size_t, vp, vp, vp, vp, C.c_size_t]
         L.sm_elapsed_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.sm_last_launches.argtypes = [vp]
         L.sm_profile_begin.argtypes = [vp, i]
@@ -100,6 +102,7 @@ def lib() -> C.CDLL:
         L.sm_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_run_batch_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
+        L.sm_run_batch_ru_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp, vp]
         L.sm_band_rows.argtypes = [i, i, i, C.POINTER(i), C.POINTER(i)]
         L.sm_multi_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
         L.sm_multi_create_range.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i, i]
@@ -107,6 +110,7 @@ def lib() -> C.CDLL:
         L.sm_multi_run_batch16.argtypes = [vp, i, vp, vp, d, vp, vp]
         L.sm_multi_run_batch_ru16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
         L.sm_multi_run_batch_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp]
+        L.sm_multi_run_batch_ru_sub16.argtypes = [vp, i, vp, vp, d, vp, vp, vp, vp]
         L.sm_multi_device_count.argtypes = [vp]
         L.sm_multi_destroy.argtypes = [vp]
         L.sm_bands_create.argtypes = [C.POINTER(vp), C.POINTER(i), i, i, i, i, i, i]
@@ -115,6 +119,7 @@ def lib() -> C.CDLL:
         L.sm_bands_run16.argtypes = [vp, vp, vp, d, vp, vp]
         L.sm_bands_run_ru16.argtypes = [vp, vp, vp, d, vp, vp, vp]
         L.sm_bands_run_sub16.argtypes = [vp, vp, vp, d, vp, vp, vp]
+        L.sm_bands_run_ru_sub16.argtypes = [vp, vp, vp, d, vp, vp, vp, vp]
         L.sm_bands_destroy.argtypes = [vp]
         _lib = L
     return _lib
@@ -274,6 +279,15 @@ class StereoContext:
                                                   C.c_void_p(d_second_edges), edge_stride, C.c_void_p(d_best or None),
                                                   C.c_void_p(d_web), C.c_void_p(d_web_sub), out_stride))
 
+    def match_wta_dev_batch_ru_sub16(self, n_pairs: int, d_first_edges: int, d_second_edges: int, edge_stride: int,
+                                     d_best, d_web: int, d_runner_up: int, d_web_sub: int, out_stride: int):
+        """match_wta_dev_batch_ru16 and match_wta_dev_batch_sub16 from one launch: the runner-up scores to
+        d_runner_up and web_sub to d_web_sub, each equal to what those two write.  min_shift + num_shifts <= 4095."""
+        _check(lib().sm_match_wta_dev_batch_ru_sub16(self._c, n_pairs, C.c_void_p(d_first_edges),
+                                                     C.c_void_p(d_second_edges), edge_stride,
+                                                     C.c_void_p(d_best or None), C.c_void_p(d_web),
+                                                     C.c_void_p(d_runner_up), C.c_void_p(d_web_sub), out_stride))
+
     def elapsed_ms(self) -> float:
         ms = C.c_float()
         _check(lib().sm_elapsed_ms(self._c, C.byref(ms)))
@@ -339,6 +353,16 @@ class StereoContext:
                           threshold, web_u8, want_best, web_out, web16, want_runner_up, lib().sm_run_batch_sub16,
                           want_subpixel)
 
+    def run_batch_ru_sub16(self, first, second, threshold=0.15, want_best=False):
+        """run_batch(web16=True) with the runner-up and web_sub from one pass: (web, [best], runner_up, web_sub), all
+        uint16, each equal to what want_runner_up / want_subpixel return."""
+        first = np.ascontiguousarray(first, np.uint8)
+        second = np.ascontiguousarray(second, np.uint8)
+        n = first.shape[0]
+        assert first.shape == second.shape == (n, self.H, self.W)
+        return _run_batch(self._c, None, None, None, first, second, threshold, False, want_best, None, True,
+                          run_ru_sub=lib().sm_run_batch_ru_sub16)
+
     # -- convenience: the reference's whole step 2 on host edge maps -----------
     def match_wta_host(self, first_edges, second_edges):
         self.set_edges(first_edges, second_edges)
@@ -352,13 +376,15 @@ def _check_extras(web16, want_runner_up, want_subpixel):
     if want_subpixel and not web16:
         raise ValueError("want_subpixel needs web16=True (web_sub comes with 16-bit results only)")
     if want_subpixel and want_runner_up:
-        raise ValueError("want_subpixel and want_runner_up exclude each other")
+        raise ValueError("want_subpixel and want_runner_up exclude each other (run_batch_ru_sub16 / run_ru_sub16 "
+                         "return both)")
 
 
 def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, want_best, web_out, web16,
-               want_runner_up=False, run_sub=None, want_subpixel=False):
+               want_runner_up=False, run_sub=None, want_subpixel=False, run_ru_sub=None):
     """sm_run_batch / sm_multi_run_batch (run), or with web16 their 16-bit entries (run16), or with want_runner_up
-    their runner-up entries (run_ru), or with want_subpixel their sub-pixel entries (run_sub)."""
+    their runner-up entries (run_ru), or with want_subpixel their sub-pixel entries (run_sub), or (run_ru_sub given,
+    web16) their entries with both, which return (web, [best], runner_up, web_sub)."""
     if web16 and web_u8:
         raise ValueError("web16 and web_u8 exclude each other")
     _check_extras(web16, want_runner_up, want_subpixel)
@@ -368,6 +394,11 @@ def _run_batch(handle, run, run16, run_ru, first, second, threshold, web_u8, wan
         web_out = np.zeros((n, H, W), dt)
     assert web_out.dtype == dt and web_out.shape == (n, H, W) and web_out.flags.c_contiguous
     best = np.zeros((n, H, W), np.uint16 if web16 else np.int32) if want_best else None
+    if run_ru_sub is not None:
+        ru, ws = np.zeros((n, H, W), np.uint16), np.zeros((n, H, W), np.uint16)
+        _check(run_ru_sub(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out),
+                          _ptr(best) if want_best else None, _ptr(ru), _ptr(ws)))
+        return (web_out, best, ru, ws) if want_best else (web_out, ru, ws)
     if want_runner_up:
         ru = np.zeros((n, H, W), np.uint16)
         _check(run_ru(handle, n, _ptr(first), _ptr(second), threshold, _ptr(web_out), _ptr(best) if want_best else None,
@@ -407,6 +438,15 @@ class MultiGpuBatch:
         return _run_batch(self._m, lib().sm_multi_run_batch, lib().sm_multi_run_batch16, lib().sm_multi_run_batch_ru16,
                           first, second, threshold, web_u8, want_best, web_out, web16, want_runner_up,
                           lib().sm_multi_run_batch_sub16, want_subpixel)
+
+    def run_batch_ru_sub16(self, first, second, threshold=0.15, want_best=False):
+        """StereoContext.run_batch_ru_sub16 over the devices: (web, [best], runner_up, web_sub), all uint16."""
+        first = np.ascontiguousarray(first, np.uint8)
+        second = np.ascontiguousarray(second, np.uint8)
+        n = first.shape[0]
+        assert first.shape == second.shape == (n, self.H, self.W)
+        return _run_batch(self._m, None, None, None, first, second, threshold, False, want_best, None, True,
+                          run_ru_sub=lib().sm_multi_run_batch_ru_sub16)
 
     def close(self):
         if self._m:
@@ -456,6 +496,18 @@ class MultiGpuBands:
         run = lib().sm_bands_run16 if web16 else lib().sm_bands_run
         _check(run(self._b, _ptr(first), _ptr(second), threshold, _ptr(web), _ptr(best) if want_best else None))
         return (web, best) if want_best else web
+
+    def run_ru_sub16(self, first, second, threshold=0.15, want_best=False):
+        """run(web16=True) with the runner-up and web_sub from one pass of each band: (web, [best], runner_up,
+        web_sub), all uint16, each equal to what want_runner_up / want_subpixel return."""
+        first = np.ascontiguousarray(first, np.uint8)
+        second = np.ascontiguousarray(second, np.uint8)
+        assert first.shape == second.shape == (self.H, self.W)
+        web, ru, ws = (np.zeros((self.H, self.W), np.uint16) for _ in range(3))
+        best = np.zeros((self.H, self.W), np.uint16) if want_best else None
+        _check(lib().sm_bands_run_ru_sub16(self._b, _ptr(first), _ptr(second), threshold, _ptr(web),
+                                           _ptr(best) if want_best else None, _ptr(ru), _ptr(ws)))
+        return (web, best, ru, ws) if want_best else (web, ru, ws)
 
     def close(self):
         if self._b:

@@ -1,8 +1,8 @@
-// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its four output families:
+// k_bitslice.cuh -- the fast hot-path kernel (SM_KERNEL_BITSLICE), shared by its five output families:
 // k_bitslice (int32 best / web, k_bitslice.cu), k_bitslice16 (uint16_t, k_bitslice16.cu), k_bitslice_ru (uint16_t
-// and the runner-up score, k_bitslice_ru.cu) and k_bitslice_sub (uint16_t and the web in sixteenths of a shift,
-// k_bitslice_sub.cu).  Each translation unit instantiates one family through dispatch, so that the four compile in
-// parallel.
+// and the runner-up score, k_bitslice_ru.cu), k_bitslice_sub (uint16_t and the web in sixteenths of a shift,
+// k_bitslice_sub.cu) and k_bitslice_ru_sub (uint16_t and both, k_bitslice_ru_sub.cu).  Each translation unit
+// instantiates one family through dispatch, so that the five compile in parallel.
 //
 // What it replaces: fillup_matches + 30x{memset, addup_pixels_in_square, record_score} +
 // find_highest_scoring_shifts of the reference (stereo.cu:127-225), i.e. per pixel and per
@@ -760,7 +760,8 @@ __device__ __forceinline__ void store_if(uint16_t *lane_base, int row, int row_b
 // The body of the kernel families; OutT (int32_t or uint16_t) is the type of the stored best and web.  Pair z's
 // outputs are z * best_stride (best) and z * out_stride (web, runner-up, web_sub) elements further.  RU (k_bitslice_ru,
 // 16-bit): the runner-up score goes to out_ru as well.  SUB (k_bitslice_sub, 16-bit): web_sub goes to out_ws, and MULTI
-// carries one u16 per pixel between chunks in out_carry (see put).
+// carries one u16 per pixel between chunks in out_carry (see put).  Both (k_bitslice_ru_sub): the two are independent
+// -- their chains, merges and stores share only best, web and the planes -- so each output is its family's.
 template <typename OutT, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP, bool RU = false, bool SUB = false>
 __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, OutT *out_web, size_t best_stride,
                                               uint16_t *out_ru = nullptr, uint16_t *out_ws = nullptr,
@@ -805,7 +806,7 @@ __device__ __forceinline__ void bitslice_body(BitsliceArgs a, OutT *out_best, Ou
     out_web += blockIdx.z * a.h.out_stride;
     static_assert(!RU || std::is_same<OutT, uint16_t>::value, "runner-up: 16-bit outputs only");
     if constexpr (RU) out_ru += blockIdx.z * a.h.out_stride;
-    static_assert(!SUB || (std::is_same<OutT, uint16_t>::value && !RU), "sub-pixel: 16-bit outputs, no runner-up");
+    static_assert(!SUB || std::is_same<OutT, uint16_t>::value, "sub-pixel: 16-bit outputs only");
     if constexpr (SUB) {
         out_ws += blockIdx.z * a.h.out_stride;
         if (MULTI) out_carry += blockIdx.z * a.h.out_stride;
@@ -1334,16 +1335,56 @@ k_bitslice_sub(BitsliceSubArgs a)
                                                                        a.b.h.out_stride, nullptr, a.web_sub, a.carry);
 }
 
-// which outputs a family stores beyond best / web
-enum Extra { EXTRA_NONE = 0, EXTRA_RU = 1, EXTRA_SUB = 2 };
+// uint16_t best / web, the runner-up score and web_sub from one launch: the 16-bit kernels' argument and the arrays of
+// both families above (each output equals its k_bitslice_ru / k_bitslice_sub counterpart)
+struct BitsliceRuSubArgs {
+    BitsliceArgs b;
+    uint16_t *runner_up;  // [pairs][FH][W], pair z out_stride elements further
+    uint16_t *web_sub;    // the same layout
+    uint16_t *carry;      // the same layout, MULTI only (scratch of the caller's)
+};
 
-// the family: int32 (k_bitslice), 16-bit (k_bitslice16), 16-bit with the runner-up (RU, k_bitslice_ru) or with web_sub
-// (SUB, k_bitslice_sub)
+// CTAs per SM of a kernel with both extras: its 16-bit sibling's, but fewer where that spills and fewer is faster.
+//   - MULTI, windows 7 to 15: 2 (255 registers, no spill).  At 3 CTAs they spill 44 to 136 bytes of stores, at 4 up to
+//     296.  Measured on a B200 (1000 W, tools/ru_sub_time.py's workloads): 128 shifts at window 9 34.7 against 38.7 us
+//     per pair at 3, 129 shifts at window 13 59.3 against 70.0.
+//   - MULTI, window 5: 3 (168 registers, no spill; 144 bytes at 4), as the sub-pixel family.
+//   - C2 + HP, windows 7 to 13: 3 (192 to 632 bytes of spill stores at 4; none at 3 but window 13's 160).  16 shifts at
+//     window 9 19.3 against 22.9 us per pair at 4, window 11 19.4 against 23.1.  Window 5 keeps 4: it spills 80 bytes
+//     there, but runs 15.3 against 15.8 us at 3.
+// Config 2's kernel (<4,2,16,0,0,0>) keeps 4 as well: 4 bytes of spills, and at 3 its steady block grows past the
+// ALU-pipe budget (tests/test_sass_budget_ru_sub.py).
+template <int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+constexpr int ru_sub_ctas_per_sm()
+{
+    constexpr int c = WS<HALF, NW, SEG, true>::CTAS_PER_SM;
+    if (c != 4) return c;
+    if (MULTI && HALF >= 3 && HALF <= 7) return 2;
+    if ((MULTI && HALF == 2) || (C2 && HP && HALF >= 3 && HALF <= 6)) return 3;
+    return c;
+}
+
+template <int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
+__global__ void __launch_bounds__(32 * WS<HALF, NW, SEG, true>::WPC, (ru_sub_ctas_per_sm<HALF, NW, SEG, MULTI, C2, HP>()))
+k_bitslice_ru_sub(BitsliceRuSubArgs a)
+{
+    bitslice_body<uint16_t, HALF, NW, SEG, MULTI, C2, HP, true, true>(a.b, static_cast<uint16_t *>(a.b.h.best),
+                                                                      static_cast<uint16_t *>(a.b.h.web),
+                                                                      a.b.h.out_stride, a.runner_up, a.web_sub, a.carry);
+}
+
+// which outputs a family stores beyond best / web
+enum Extra { EXTRA_NONE = 0, EXTRA_RU = 1, EXTRA_SUB = 2, EXTRA_RU_SUB = 3 };
+
+// the family: int32 (k_bitslice), 16-bit (k_bitslice16), 16-bit with the runner-up (RU, k_bitslice_ru), with web_sub
+// (SUB, k_bitslice_sub) or with both (k_bitslice_ru_sub)
 template <typename OutT, int X, int HALF, int NW, int SEG, bool MULTI, bool C2, bool HP>
 constexpr auto kernel_of()
 {
     static_assert(X == EXTRA_NONE || std::is_same<OutT, uint16_t>::value, "runner-up / sub-pixel: 16-bit outputs only");
-    if constexpr (X == EXTRA_SUB)
+    if constexpr (X == EXTRA_RU_SUB)
+        return k_bitslice_ru_sub<HALF, NW, SEG, MULTI, C2, HP>;
+    else if constexpr (X == EXTRA_SUB)
         return k_bitslice_sub<HALF, NW, SEG, MULTI, C2, HP>;
     else if constexpr (X == EXTRA_RU)
         return k_bitslice_ru<HALF, NW, SEG, MULTI, C2, HP>;
@@ -1353,12 +1394,13 @@ constexpr auto kernel_of()
         return k_bitslice<HALF, NW, SEG, MULTI, C2, HP>;
 }
 
-// extra: the runner-up array (X == EXTRA_RU) or web_sub (EXTRA_SUB); carry: EXTRA_SUB's chunk carry
+// extra: the runner-up array (X == EXTRA_RU or EXTRA_RU_SUB) or web_sub (EXTRA_SUB); carry: the sub-pixel chunk
+// carry (EXTRA_SUB, EXTRA_RU_SUB); web_sub: EXTRA_RU_SUB's web_sub
 template <typename OutT, int X, int HALF, int NW, int SEG, bool C2, bool HP>
 int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec, uint16_t *extra,
-               uint16_t *carry)
+               uint16_t *carry, uint16_t *web_sub)
 {
-    constexpr bool RU = X == EXTRA_RU, SUB = X == EXTRA_SUB;
+    constexpr bool RU = X == EXTRA_RU || X == EXTRA_RU_SUB, SUB = X == EXTRA_SUB || X == EXTRA_RU_SUB;
     using C = WS<HALF, NW, SEG, (RU || SUB) && !C2 && !HP>;  // (bitslice_body's layout: its centre-match ring, its shared memory)
     if (mode == MODE_TMEM_COLUMNS) return C::TCOLS;
     // MULTI: more than one chunk of 32*NW shifts, i.e. (best, web) are merged across passes
@@ -1379,8 +1421,12 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
     // allow, all known at compile time (WS::CTAS_PER_SM is also the kernel's __launch_bounds__).  (The occupancy
     // API is not asked: it answers 1 CTA per SM for these kernels, whatever carve-out is set, while the
     // hardware runs the 4 that ncu's launch__occupancy_limit_* report.)
-    // (the runner-up and sub-pixel families' MULTI kernels may hold fewer: ru_ctas_per_sm, sub_ctas_per_sm)
-    const int ctas_per_sm = RU && multi    ? ru_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>()
+    // (the runner-up and sub-pixel families' MULTI kernels may hold fewer: ru_ctas_per_sm, sub_ctas_per_sm; the
+    // family with both extras others too: ru_sub_ctas_per_sm)
+    const int ctas_per_sm = X == EXTRA_RU_SUB
+                                ? (multi ? ru_sub_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2, false, false>()
+                                         : ru_sub_ctas_per_sm<HALF, NW, SEG, false, C2, HP>())
+                            : RU && multi  ? ru_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>()
                             : SUB && multi ? sub_ctas_per_sm<HALF, NW, SEG, NW == 2 && !HP && !C2>()
                                            : C::CTAS_PER_SM;
     const int warps_per_sm = ctas_per_sm * C::WPC;
@@ -1453,9 +1499,15 @@ int launch_one(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRe
     }
     segs = shape(segs, a.rows_per_seg);
     dim3 grid((strips + C::WPC - 1) / C::WPC, segs, h.npairs);
-    // the kernel's argument: BitsliceArgs, or with RU that and the runner-up array, with SUB web_sub and the carry
-    typename std::conditional<RU, BitsliceRuArgs, typename std::conditional<SUB, BitsliceSubArgs, BitsliceArgs>::type>::type arg;
-    if constexpr (RU)
+    // the kernel's argument: BitsliceArgs, or with RU that and the runner-up array, with SUB web_sub and the carry,
+    // with both all three
+    typename std::conditional<
+        X == EXTRA_RU_SUB, BitsliceRuSubArgs,
+        typename std::conditional<RU, BitsliceRuArgs,
+                                  typename std::conditional<SUB, BitsliceSubArgs, BitsliceArgs>::type>::type>::type arg;
+    if constexpr (X == EXTRA_RU_SUB)
+        arg = BitsliceRuSubArgs{a, extra, web_sub, carry};
+    else if constexpr (RU)
         arg = BitsliceRuArgs{a, extra};
     else if constexpr (SUB)
         arg = BitsliceSubArgs{a, extra, carry};
@@ -1532,10 +1584,10 @@ static Shape pick_shape(const HotArgs &h, int num_sms)
 }
 
 // the kernel of the geometry, from the family that stores OutT (X: and the runner-up or web_sub, to extra; the
-// sub-pixel family's chunk carry to carry)
+// sub-pixel family's chunk carry to carry; EXTRA_RU_SUB: the runner-up to extra, web_sub to web_sub)
 template <typename OutT, int X = EXTRA_NONE>
 int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchRecord *rec = nullptr,
-             uint16_t *extra = nullptr, uint16_t *carry = nullptr)
+             uint16_t *extra = nullptr, uint16_t *carry = nullptr, uint16_t *web_sub = nullptr)
 {
     if (mode == MODE_PREPARE && h.npairs == 1) {
         // a context launches one pair at a time AND batches: prepare the batch flavour too if it is another kernel
@@ -1551,7 +1603,7 @@ int dispatch(const HotArgs &h, int num_sms, cudaStream_t s, int mode, LaunchReco
     const int half = h.g.half;
 #define SM_SHAPE(HF, NW_, SEG_, C2_, HP_) \
     if (half == HF && sh.nw == NW_ && sh.seg == SEG_ && sh.c2 == C2_ && sh.hp == HP_) \
-        return launch_one<OutT, X, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec, extra, carry);
+        return launch_one<OutT, X, HF, NW_, SEG_, C2_, HP_>(h, num_sms, s, mode, rec, extra, carry, web_sub);
 #define SM_HALVES(M, ...) \
     M(0, __VA_ARGS__) M(1, __VA_ARGS__) M(2, __VA_ARGS__) M(3, __VA_ARGS__) M(4, __VA_ARGS__) M(5, __VA_ARGS__) \
     M(6, __VA_ARGS__) M(7, __VA_ARGS__) M(8, __VA_ARGS__) M(9, __VA_ARGS__) M(10, __VA_ARGS__) M(11, __VA_ARGS__) \

@@ -109,11 +109,20 @@ __global__ void __launch_bounds__(256) k_direct16_sub(HotArgs a, uint16_t *web_s
                                         web_sub);
 }
 
+// the 16-bit twin with the runner-up and web_sub (a.best may be NULL; the other two may not)
+__global__ void __launch_bounds__(256) k_direct16_ru_sub(HotArgs a, uint16_t *runner_up, uint16_t *web_sub)
+{
+    direct_pixel<uint16_t, true, true>(a, static_cast<uint16_t *>(a.best), static_cast<uint16_t *>(a.web), runner_up,
+                                       web_sub);
+}
+
 int launch_direct(const HotArgs &a, cudaStream_t s, bool out16, uint16_t *runner_up, uint16_t *web_sub)
 {
     dim3 block(32, 8);
     dim3 grid((a.g.W + block.x - 1) / block.x, (a.g.BH + block.y - 1) / block.y);
-    if (web_sub)
+    if (runner_up && web_sub)
+        k_direct16_ru_sub<<<grid, block, 0, s>>>(a, runner_up, web_sub);
+    else if (web_sub)
         k_direct16_sub<<<grid, block, 0, s>>>(a, web_sub);
     else if (runner_up)
         k_direct16_ru<<<grid, block, 0, s>>>(a, runner_up);
@@ -158,6 +167,7 @@ void warm_direct()
     warm_kernel(k_direct16);
     warm_kernel(k_direct16_ru);
     warm_kernel(k_direct16_sub);
+    warm_kernel(k_direct16_ru_sub);
     warm_kernel(k_planes);
 }
 

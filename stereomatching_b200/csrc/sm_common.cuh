@@ -107,7 +107,8 @@ int launch_pack(const uint8_t *e1, const uint8_t *e2, int FH, int row0, int vari
                 const PackedGeom &g, int M, uint32_t *LA, uint32_t *LB, uint32_t *RB, cudaStream_t s,
                 int npairs = 1, size_t edge_stride = 0, size_t plane_stride = 0);
 // out16: the 16-bit twin; runner_up (16-bit outputs only): the twin that also stores the runner-up score there;
-// web_sub (16-bit outputs only): the twin that also stores the web in sixteenths of a shift there
+// web_sub (16-bit outputs only): the twin that also stores the web in sixteenths of a shift there; both: the twin
+// that stores both
 int launch_direct(const HotArgs &a, cudaStream_t s, bool out16 = false, uint16_t *runner_up = nullptr,
                   uint16_t *web_sub = nullptr);
 int launch_bitslice(const HotArgs &a, int num_sms, cudaStream_t s, LaunchRecord *rec);
@@ -118,11 +119,15 @@ int launch_bitslice_ru(const HotArgs &a, uint16_t *runner_up, int num_sms, cudaS
 // past 64 shifts (the chunk merge's per-pixel state)
 int launch_bitslice_sub(const HotArgs &a, uint16_t *web_sub, uint16_t *carry, int num_sms, cudaStream_t s,
                         LaunchRecord *rec);
+// uint16_t outputs, the runner-up score and web_sub from one launch (the same layouts; carry as for the sub-pixel one)
+int launch_bitslice_ru_sub(const HotArgs &a, uint16_t *runner_up, uint16_t *web_sub, uint16_t *carry, int num_sms,
+                           cudaStream_t s, LaunchRecord *rec);
 bool bitslice_supports(int half, int D);
 int prepare_bitslice(const HotArgs &a, int num_sms);
 int prepare_bitslice16(const HotArgs &a, int num_sms);
 int prepare_bitslice_ru(const HotArgs &a, int num_sms);
 int prepare_bitslice_sub(const HotArgs &a, int num_sms);
+int prepare_bitslice_ru_sub(const HotArgs &a, int num_sms);
 // web_sub = 16 * web + frac must fit 16 bits: min_shift + num_shifts <= SUB_MAX_RANGE for the sub-pixel entries
 constexpr int SUB_MAX_RANGE = 4095;
 int bitslice_tmem_columns(const HotArgs &a);

@@ -76,6 +76,7 @@ struct sm_ctx {
     bool prepared16 = false;  // the 16-bit bit-sliced kernels of this geometry are loaded (prepare_bitslice16)
     int occ_ru = 0;           // ... the runner-up kernels (prepare_bitslice_ru; 0: not yet): their resident warps per SM
     int occ_sub = 0;          // ... the sub-pixel kernels (prepare_bitslice_sub; 0: not yet)
+    int occ_ru_sub = 0;       // ... the kernels with both (prepare_bitslice_ru_sub; 0: not yet)
     int32_t *web2 = nullptr, *tmp = nullptr;  // step 3 ping-pong
     const int32_t *web_filled = nullptr;      // result of fill_web_holes (may alias web)
     bool have_web2 = false;
@@ -270,37 +271,32 @@ int hot_kernel(const sm_ctx *c)
 // its 16-bit family registers): a 16-bit call without a best of the caller's gives it a scratch array.
 bool stores_best(const sm_ctx *c) { return hot_kernel(c) == SM_KERNEL_BITSLICE; }
 
-// Loads the runner-up kernels of the context's geometry (once); their resident warps per SM go to c->occ_ru.
-int prepare_ru(sm_ctx *c)
+// Loads the kernels of the context's geometry that store the extras asked for (ru: the runner-up family, sub: the
+// sub-pixel one, both: the family with both), once per context and family; their resident warps per SM go to
+// c->occ_ru, c->occ_sub or c->occ_ru_sub, and to *occ_out.
+int prepare_extras(sm_ctx *c, bool ru, bool sub, int *occ_out = nullptr)
 {
-    if (c->occ_ru > 0) return SM_OK;
-    int occ = c->occ;
-    if (hot_kernel(c) == SM_KERNEL_BITSLICE && bitslice_supports(c->half, c->D)) {
-        occ = prepare_bitslice_ru(hot_args(c, Outputs{}), c->num_sms);
-        if (occ < 0) return occ;
+    int *slot = ru && sub ? &c->occ_ru_sub : (ru ? &c->occ_ru : &c->occ_sub);
+    if (*slot == 0) {
+        int occ = c->occ;
+        if (hot_kernel(c) == SM_KERNEL_BITSLICE && bitslice_supports(c->half, c->D)) {
+            const HotArgs a = hot_args(c, Outputs{});
+            occ = ru && sub ? prepare_bitslice_ru_sub(a, c->num_sms)
+                  : ru      ? prepare_bitslice_ru(a, c->num_sms)
+                            : prepare_bitslice_sub(a, c->num_sms);
+            if (occ < 0) return occ;
+        }
+        *slot = occ > 0 ? occ : 1;
     }
-    c->occ_ru = occ > 0 ? occ : 1;
-    return SM_OK;
-}
-
-// Loads the sub-pixel kernels of the context's geometry (once); their resident warps per SM go to c->occ_sub.
-int prepare_sub(sm_ctx *c)
-{
-    if (c->occ_sub > 0) return SM_OK;
-    int occ = c->occ;
-    if (hot_kernel(c) == SM_KERNEL_BITSLICE && bitslice_supports(c->half, c->D)) {
-        occ = prepare_bitslice_sub(hot_args(c, Outputs{}), c->num_sms);
-        if (occ < 0) return occ;
-    }
-    c->occ_sub = occ > 0 ? occ : 1;
+    if (occ_out) *occ_out = *slot;
     return SM_OK;
 }
 
 // whether the sub-pixel kernel of the context merges 64-shift chunks (and needs Outputs::carry)
 bool sub_needs_carry(const sm_ctx *c) { return hot_kernel(c) == SM_KERNEL_BITSLICE && c->D > 64; }
 
-// The main kernel: of the runner-up family with runner_up, of the sub-pixel one with web_sub, of the 16-bit one with
-// out16, else of the int32 one.
+// The main kernel: of the family with both extras with runner_up and web_sub, of the runner-up family with runner_up
+// alone, of the sub-pixel one with web_sub alone, of the 16-bit one with out16, else of the int32 one.
 int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cudaStream_t st, uint16_t *web_sub = nullptr,
                 uint16_t *carry = nullptr)
 {
@@ -315,19 +311,16 @@ int launch_main(sm_ctx *c, const HotArgs &a, bool out16, uint16_t *runner_up, cu
             if (rc < 0) return rc;
             c->prepared16 = true;
         }
-        if (runner_up) {
-            const int rc = prepare_ru(c);
-            if (rc < 0) return rc;
-        }
-        if (web_sub) {
-            const int rc = prepare_sub(c);
+        if (runner_up || web_sub) {
+            const int rc = prepare_extras(c, runner_up != nullptr, web_sub != nullptr);
             if (rc < 0) return rc;
         }
         LaunchRecord rec;
-        const int rc = runner_up ? launch_bitslice_ru(a, runner_up, c->num_sms, st, &rec)
-                       : web_sub ? launch_bitslice_sub(a, web_sub, carry, c->num_sms, st, &rec)
-                       : out16   ? launch_bitslice16(a, c->num_sms, st, &rec)
-                                 : launch_bitslice(a, c->num_sms, st, &rec);
+        const int rc = runner_up && web_sub ? launch_bitslice_ru_sub(a, runner_up, web_sub, carry, c->num_sms, st, &rec)
+                       : runner_up          ? launch_bitslice_ru(a, runner_up, c->num_sms, st, &rec)
+                       : web_sub            ? launch_bitslice_sub(a, web_sub, carry, c->num_sms, st, &rec)
+                       : out16              ? launch_bitslice16(a, c->num_sms, st, &rec)
+                                            : launch_bitslice(a, c->num_sms, st, &rec);
         if (rc >= 0) c->last_launch = rec;
         return rc;
     }
@@ -398,7 +391,8 @@ extern "C" const char *sm_last_error(void) { return g_err; }
 
 // 1.1: sm_multi_*, sm_bands_*; 1.2: sm_set_option / sm_get_info, square_width 0, the microbenchmarks moved out;
 // 1.3: SM_INFO_KERNEL_SHAPE / SM_INFO_ROW_RUNS; then, additive, the 16-bit result entries (*16, sm_download_web_u16),
-// the search-range creators (*_range), the runner-up entries (*_ru16) and the sub-pixel entries (*_sub16)
+// the search-range creators (*_range), the runner-up entries (*_ru16), the sub-pixel entries (*_sub16) and the entries
+// with both (*_ru_sub16)
 extern "C" int sm_version(void) { return (1 << 16) | 3; }
 
 extern "C" int sm_device_count(void)
@@ -879,25 +873,14 @@ static int batch_core(sm_ctx *c, int n_pairs, bool from_images, double threshold
     // the kernel may have been switched since the last call (sm_set_kernel): the literal kernel takes one pair
     // per launch, the bit-sliced one a group
     c->batch_group = kk == SM_KERNEL_BITSLICE ? c->batch_group_cap : 1;
-    if (out.runner_up && kk == SM_KERNEL_BITSLICE) {
-        // the runner-up kernels may hold fewer warps per SM than the int32 ones the group was sized for: the pairs
-        // per launch of their own (never more than the plane sets hold)
-        int rc;
-        if ((rc = prepare_ru(c)) < 0) return rc;
-        if (c->occ_ru != c->occ) {
+    if ((out.runner_up || out.web_sub) && kk == SM_KERNEL_BITSLICE) {
+        // the runner-up, sub-pixel and combined kernels may hold fewer warps per SM than the int32 ones the group was
+        // sized for: the pairs per launch of their own (never more than the plane sets hold)
+        int rc, occ;
+        if ((rc = prepare_extras(c, out.runner_up != nullptr, out.web_sub != nullptr, &occ)) < 0) return rc;
+        if (occ != c->occ) {
             HotArgs a = hot_args(c, out);
-            a.blocks_per_sm = c->occ_ru;
-            const int g = bitslice_pairs_per_launch(a, c->num_sms, c->batch_group_cap);
-            c->batch_group = g < c->batch_group_cap ? g : c->batch_group_cap;
-        }
-    }
-    if (out.web_sub && kk == SM_KERNEL_BITSLICE) {
-        // the same for the sub-pixel kernels
-        int rc;
-        if ((rc = prepare_sub(c)) < 0) return rc;
-        if (c->occ_sub != c->occ) {
-            HotArgs a = hot_args(c, out);
-            a.blocks_per_sm = c->occ_sub;
+            a.blocks_per_sm = occ;
             const int g = bitslice_pairs_per_launch(a, c->num_sms, c->batch_group_cap);
             c->batch_group = g < c->batch_group_cap ? g : c->batch_group_cap;
         }
@@ -1009,6 +992,27 @@ extern "C" int sm_match_wta_dev_batch_sub16(sm_ctx *c, int n_pairs, const uint8_
     Outputs o;
     o.best16 = d_best;
     o.web16 = d_web;
+    o.web_sub = d_web_sub;
+    return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, o, out_stride);
+}
+
+extern "C" int sm_match_wta_dev_batch_ru_sub16(sm_ctx *c, int n_pairs, const uint8_t *d_first_edges,
+                                               const uint8_t *d_second_edges, size_t edge_stride, uint16_t *d_best,
+                                               uint16_t *d_web, uint16_t *d_runner_up, uint16_t *d_web_sub,
+                                               size_t out_stride)
+{
+    SM_REQUIRE(n_pairs >= 0 && d_first_edges && d_second_edges && d_web && d_runner_up && d_web_sub,
+               "sm_match_wta_dev_batch_ru_sub16: bad arguments");
+    SM_REQUIRE(c, "sm_match_wta_dev_batch_ru_sub16: NULL context");
+    SM_REQUIRE(c->M + c->D <= SUB_MAX_RANGE,
+               "sm_match_wta_dev_batch_ru_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
+    SM_ENTER(c);
+    SM_REQUIRE(edge_stride >= c->npix() && out_stride >= c->npix(),
+               "sm_match_wta_dev_batch_ru_sub16: stride below frame size");
+    Outputs o;
+    o.best16 = d_best;
+    o.web16 = d_web;
+    o.runner_up = d_runner_up;
     o.web_sub = d_web_sub;
     return batch_core(c, n_pairs, false, 0.0, d_first_edges, d_second_edges, edge_stride, o, out_stride);
 }
@@ -1264,8 +1268,8 @@ enum WebFormat { WEB_I32, WEB_U8, WEB_U16 };
 static size_t web_bytes(WebFormat f) { return f == WEB_U8 ? 1 : (f == WEB_U16 ? 2 : 4); }
 static size_t best_bytes(WebFormat f) { return f == WEB_U16 ? 2 : 4; }
 
-// sm_run_batch / sm_run_batch16 / sm_run_batch_ru16 / sm_run_batch_sub16 (fn: the entry's name, for the messages;
-// ru_out: the runner-up scores, sub_out: web_sub, WEB_U16 only, not both)
+// sm_run_batch / sm_run_batch16 / sm_run_batch_ru16 / sm_run_batch_sub16 / sm_run_batch_ru_sub16 (fn: the entry's
+// name, for the messages; ru_out: the runner-up scores, sub_out: web_sub, WEB_U16 only, either or both)
 static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
                      double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr,
                      uint16_t *sub_out = nullptr)
@@ -1273,7 +1277,7 @@ static int run_batch(const char *fn, sm_ctx *c, int n_pairs, const uint8_t *firs
     SM_ENTER(c);
     SM_REQUIRE(n_pairs >= 0 && first && second && web_out, "%s: bad arguments", fn);
     SM_REQUIRE(!ru_out || fmt == WEB_U16, "%s: the runner-up needs 16-bit results", fn);
-    SM_REQUIRE(!sub_out || (fmt == WEB_U16 && !ru_out && c->M + c->D <= SUB_MAX_RANGE),
+    SM_REQUIRE(!sub_out || (fmt == WEB_U16 && c->M + c->D <= SUB_MAX_RANGE),
                "%s: web_sub needs 16-bit results and min_shift + num_shifts <= %d", fn, SUB_MAX_RANGE);
     SM_REQUIRE(c->row0 == 0 && c->row1 == c->FH, "%s: whole-frame contexts only", fn);
     SM_REQUIRE(fmt != WEB_U8 || c->M + c->D <= 255, "%s: u8 web needs min_shift + num_shifts <= 255", fn);
@@ -1421,6 +1425,21 @@ extern "C" int sm_run_batch_sub16(sm_ctx *c, int n_pairs, const uint8_t *first, 
     return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, nullptr, web_sub_out);
 }
 
+extern "C" int sm_run_batch_ru_sub16(sm_ctx *c, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                     double threshold, uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out,
+                                     uint16_t *web_sub_out)
+{
+    // the checks that need no context first (and no device)
+    SM_REQUIRE(n_pairs >= 0 && first && second && web_out && runner_up_out && web_sub_out,
+               "sm_run_batch_ru_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_run_batch_ru_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(c, "sm_run_batch_ru_sub16: NULL context");
+    SM_REQUIRE(c->M + c->D <= SUB_MAX_RANGE, "sm_run_batch_ru_sub16: web_sub needs min_shift + num_shifts <= %d",
+               SUB_MAX_RANGE);
+    return run_batch(__func__, c, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out,
+                     web_sub_out);
+}
+
 // ---- whole pairs over several GPUs of one box ------------------------------------------------
 //
 // SURVEY 8e: pairs shard with no exchange step.  One context and one host thread per device; device d
@@ -1558,7 +1577,8 @@ extern "C" int sm_multi_destroy(sm_multi *m)
 
 extern "C" int sm_multi_device_count(const sm_multi *m) { return m ? m->n : SM_ERR_ARG; }
 
-// sm_multi_run_batch / sm_multi_run_batch16 / sm_multi_run_batch_ru16 / sm_multi_run_batch_sub16
+// sm_multi_run_batch / sm_multi_run_batch16 / sm_multi_run_batch_ru16 / sm_multi_run_batch_sub16 /
+// sm_multi_run_batch_ru_sub16
 static int multi_run_batch(const char *fn, sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
                            double threshold, WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr,
                            uint16_t *sub_out = nullptr)
@@ -1621,6 +1641,20 @@ extern "C" int sm_multi_run_batch_sub16(sm_multi *m, int n_pairs, const uint8_t 
     SM_REQUIRE(m->ctx[0]->M + m->ctx[0]->D <= SUB_MAX_RANGE,
                "sm_multi_run_batch_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
     return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, nullptr,
+                           web_sub_out);
+}
+
+extern "C" int sm_multi_run_batch_ru_sub16(sm_multi *m, int n_pairs, const uint8_t *first, const uint8_t *second,
+                                           double threshold, uint16_t *web_out, uint16_t *best_out,
+                                           uint16_t *runner_up_out, uint16_t *web_sub_out)
+{
+    // the checks that need no handle first (and no device)
+    SM_REQUIRE(m && n_pairs >= 0 && first && second && web_out && runner_up_out && web_sub_out,
+               "sm_multi_run_batch_ru_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_multi_run_batch_ru_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(m->ctx[0]->M + m->ctx[0]->D <= SUB_MAX_RANGE,
+               "sm_multi_run_batch_ru_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
+    return multi_run_batch(__func__, m, n_pairs, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out,
                            web_sub_out);
 }
 
@@ -1709,7 +1743,7 @@ static int band_run16(sm_ctx *c, uint16_t *web_out, uint16_t *best_out, uint16_t
     return SM_OK;
 }
 
-// sm_bands_run / sm_bands_run16 / sm_bands_run_ru16 / sm_bands_run_sub16
+// sm_bands_run / sm_bands_run16 / sm_bands_run_ru16 / sm_bands_run_sub16 / sm_bands_run_ru_sub16
 static int bands_run(const char *fn, sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
                      WebFormat fmt, void *web_out, void *best_out, uint16_t *ru_out = nullptr, uint16_t *sub_out = nullptr)
 {
@@ -1771,4 +1805,15 @@ extern "C" int sm_bands_run_sub16(sm_bands *b, const uint8_t *first, const uint8
     SM_REQUIRE(b->ctx[0]->M + b->ctx[0]->D <= SUB_MAX_RANGE,
                "sm_bands_run_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
     return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out, nullptr, web_sub_out);
+}
+
+extern "C" int sm_bands_run_ru_sub16(sm_bands *b, const uint8_t *first, const uint8_t *second, double threshold,
+                                     uint16_t *web_out, uint16_t *best_out, uint16_t *runner_up_out,
+                                     uint16_t *web_sub_out)
+{
+    SM_REQUIRE(b && first && second && web_out && runner_up_out && web_sub_out, "sm_bands_run_ru_sub16: bad arguments");
+    SM_REQUIRE(threshold >= 0.0 && threshold <= 1.0, "sm_bands_run_ru_sub16: threshold must be between 0 and 1");
+    SM_REQUIRE(b->ctx[0]->M + b->ctx[0]->D <= SUB_MAX_RANGE,
+               "sm_bands_run_ru_sub16: web_sub needs min_shift + num_shifts <= %d", SUB_MAX_RANGE);
+    return bands_run(__func__, b, first, second, threshold, WEB_U16, web_out, best_out, runner_up_out, web_sub_out);
 }

@@ -3,7 +3,7 @@
 library (no GPU, no profiler).
 
     python tools/sass_budget.py [--lib stereomatching_b200/libstereo_b200.so] [--kernel 4,2,16,0,0,0]
-                                [--family k_bitslice|k_bitslice16|k_bitslice_ru|k_bitslice_sub] [--json]
+                                [--family k_bitslice|k_bitslice16|k_bitslice_ru|k_bitslice_sub|k_bitslice_ru_sub] [--json]
 
 `--kernel` names an instantiation by its template arguments HALF,NW,SEG,MULTI,C2,HP (default: config 2,
 window 9, 64 shifts), `--family` the output family (default: k_bitslice, the int32 one).  The SASS (`cuobjdump -sass`) is cut into basic blocks; of those,
@@ -36,7 +36,7 @@ def bits_for(v):
     return b
 
 
-FAMILIES = ("k_bitslice", "k_bitslice16", "k_bitslice_ru", "k_bitslice_sub")
+FAMILIES = ("k_bitslice", "k_bitslice16", "k_bitslice_ru", "k_bitslice_sub", "k_bitslice_ru_sub")
 
 
 def mangled(half, nw, seg, multi, c2, hp, family="k_bitslice"):
